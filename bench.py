@@ -42,9 +42,11 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the bench writes nothing into the tree (which may be read-only)
 
 METRIC = "NDT scan-matches/sec (1080-pt 2D scans)"
 UNIT = "matches/s"
+DUMP_BUDGET = 64 << 20              # --dump-outputs: bytes in all, over every rank
 FALLBACK_HBM_GBS = 6650.0  # /opt/skills/guides/B200_PROFILING.md fallback
 
 
@@ -82,7 +84,15 @@ def parse_args():
     ap.add_argument("--pinned", default="default", choices=["default", "wc"],
                     help="e2e input buffer: ordinary pinned memory, or write-combined pinned memory (ndt2d_host_alloc_flags)")
     ap.add_argument("--no-numa", action="store_true", help="do not bind the rank to the NUMA node of its GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="scan2map and the reference arm: after the timed steps, write the result records of the last step as "
+                         "DIR/<field>.npy (float64; at most 64 MB, a fixed seeded sample of the scans above that), so that two builds "
+                         "can be compared output for output")
     a = ap.parse_args()
+    if (a.steps is not None and a.steps < 1) or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl == "native" and a.workload != "scan2map":
+        ap.error("--dump-outputs: only the scan2map workload and the reference arm write their outputs")
     dflt = {"scan2map": (65536, [0.25], [0.03, 0.3]), "pyramid": (10000, [2.0, 1.0, 0.5], [0.2, 3.0]), "sweep": (1, [0.25], [0.0, 0.0]),
             "build": (1, [0.25], [0.0, 0.0]), "newton": (1, [0.25], [0.0, 0.0]),
             "odometry": (16384, [0.5], [0.02, 0.2])}[a.workload]
@@ -177,6 +187,25 @@ def to_points(ranges):
     xy = np.stack([ranges * cb[None, :], ranges * sb[None, :]], axis=-1).astype(np.float32)
     offsets = np.arange(ranges.shape[0] + 1, dtype=np.int64) * ranges.shape[1]
     return xy.reshape(-1, 2), offsets
+
+
+def dump_records(out_dir, res, rank=0, world=1):
+    """--dump-outputs: every field of the result records (pose, score, grad, hessian, iterations, status, count) as
+    out_dir/<field>.npy in float64, one row per scan; rank r of a multi-GPU job writes <field>_rank<r>.npy. When the
+    records exceed this rank's share of DUMP_BUDGET, the same seeded sample of scans is written on every run, and
+    index.npy holds the sampled scan indices."""
+    fields = [f for f in res.dtype.names if f != "reserved"]
+    row_bytes = 8 * (1 + sum(int(np.prod(res.dtype[f].shape)) for f in fields))
+    rows = (DUMP_BUDGET // max(1, world) - 4096 * (len(fields) + 1)) // row_bytes
+    arrays = {}
+    if len(res) > rows:
+        arrays["index"] = np.sort(np.random.default_rng(0).choice(len(res), rows, replace=False))
+        res = res[arrays["index"]]
+    arrays.update((f, res[f]) for f in fields)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def ncu_traffic(kernel, args, scans):
@@ -276,6 +305,8 @@ def run_reference(args):
     for _ in range(args.steps):         # the CPU arm gets already converted points: its polar-to-point conversion is not charged
         res = o.align_batch(xy, off, init, nthreads=cores)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_records(args.dump_outputs, res)
     v = nref * args.steps / dt
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": dt / args.steps * 1e3, "higher_is_better": True, "scaling": "weak",
@@ -721,6 +752,8 @@ def run_native(args):
         failed = failed or not leg.get("ok", True)
         if rank == 0:
             line["sweep"] = leg
+    if args.dump_outputs:
+        dump_records(args.dump_outputs, res, rank, world)
     if rank == 0:
         os.sched_setaffinity(0, ctx.affinity0)      # the CPU legs below use every core the process was given
         if "dense" in args.legs:
@@ -881,7 +914,8 @@ def leg_sweep(ctx, args, m):
     hyp = sweep_lattice(args.hyps, poses[0])
     lo, hi = D.shard_range(len(hyp), rank, world)
     d_xy = torch.from_numpy(xy).to(dev)
-    steps, warm = max(50, args.steps), max(5, args.warmup)
+    # as a leg of the default run, at least 50 queries (a step is 0.3-2 ms); as the workload, exactly --steps
+    steps, warm = args.steps if args.workload == "sweep" else max(50, args.steps), max(5, args.warmup)
     # timing rule: a shard's hypotheses (12 B each) and scores (8 B) are far smaller than the 126 MB L2, so the steps
     # rotate through copies totalling more than the L2
     nrot = max(2, int(math.ceil(160e6 / max(1, (hi - lo) * 20))))
@@ -1454,17 +1488,17 @@ def config4_slam_frontend():
     """BASELINE configs[4], the part that exists without GTSAM: examples/slam_frontend.cpp (C++ host code over ndt2d.hpp) drives a
     closed loop through a synthetic room - sequential GPU NDT odometry, the loop-closure search (sweep + refinement), the same
     odometry batched through alignPairs - checks its own factors against the truth and writes the g2o pose graph that
-    gtsam::readG2o + ISAM2 consume. Built with the system g++ on the spot; the figures are the program's own."""
+    gtsam::readG2o + ISAM2 consume. Built with the system g++ on the spot, in a temporary directory (the tree may be
+    read-only); the figures are the program's own."""
     import re
     import tempfile
-    exe = os.path.join(ROOT, "examples", "slam_frontend")
-    src = exe + ".cpp"
+    src = os.path.join(ROOT, "examples", "slam_frontend.cpp")
     libdir = os.path.join(ROOT, "gtsam_ndt_b200")
     try:
-        if not os.path.exists(exe) or os.path.getmtime(exe) < max(os.path.getmtime(src), os.path.getmtime(os.path.join(libdir, "libndt2d.so"))):
-            subprocess.run(["/usr/bin/g++", "-std=c++17", "-O2", "-I", os.path.join(ROOT, "include"), src, "-L", libdir, "-lndt2d",
-                            "-Wl,-rpath," + libdir, "-o", exe], check=True, capture_output=True, timeout=120)
         with tempfile.TemporaryDirectory() as td:
+            exe = os.path.join(td, "slam_frontend")
+            subprocess.run(["g++", "-std=c++17", "-O2", "-I", os.path.join(ROOT, "include"), src, "-L", libdir, "-lndt2d",
+                            "-Wl,-rpath," + libdir, "-o", exe], check=True, capture_output=True, timeout=120)
             r = subprocess.run([exe, os.path.join(td, "graph.g2o")], capture_output=True, text=True, timeout=120)
         out = r.stdout
         num = lambda rx: [float(x) for x in re.search(rx, out).groups()]

@@ -2,7 +2,7 @@
 """Small LaserScan batches (ndt2d_align_batch_ranges[_device]): block-per-scan kernel against the warp-per-scan kernel with helper
 warps, kernel ms per batch, identical records, and the host-API latency of a single scan.  python tools/ranges_small_probe.py  (GPU box)"""
 import os, sys, time, json, numpy as np
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 import gtsam_ndt_b200 as g
 from gtsam_ndt_b200 import synth

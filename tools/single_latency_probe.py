@@ -2,7 +2,7 @@
 """Host-to-host latency of one align through the host API: packed points (ndt2d_align) and one LaserScan (ndt2d_align_batch_ranges).
   [NDT2D_FAST_ZEROCOPY=0] python tools/single_latency_probe.py   (GPU box)"""
 import os, sys, time, json, numpy as np
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import gtsam_ndt_b200 as g
 from gtsam_ndt_b200 import synth
 sc = synth.SCAN_1080

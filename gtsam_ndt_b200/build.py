@@ -43,7 +43,7 @@ def build_cuda(force=False, verbose=False):
     nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
     if not os.path.exists(nvcc):
         raise RuntimeError("nvcc not found; libndt2d.so must be prebuilt")
-    extra = os.environ.get("NDT2D_NVCC_EXTRA", "").split()   # kernel tuning experiments, e.g. -DNDT2D_PIPE=0
+    extra = os.environ.get("NDT2D_NVCC_EXTRA", "").split()   # kernel tuning experiments, e.g. -maxrregcount=96
     cmd = [nvcc, "-ccbin", "/usr/bin/g++"] + NVCC_FLAGS + extra + ["-I", INCLUDE, "-I", CSRC, "-o", LIB_CUDA] + srcs + ["-lcudart"]
     r = subprocess.run(cmd, capture_output=True, text=True)
     log = r.stdout + r.stderr
@@ -57,7 +57,7 @@ def build_cuda(force=False, verbose=False):
 
 
 def build_variant(name, extra_flags):
-    """Kernel tuning experiments: the same sources with extra -D knobs -> build/variants/libndt2d_<name>.so
+    """Kernel tuning experiments: the same sources with extra nvcc flags -> build/variants/libndt2d_<name>.so
     (git-ignored, travels to the GPU box). Select it at run time with NDT2D_LIB=<path>."""
     out_dir = os.path.join(os.path.dirname(HERE), "build", "variants")
     os.makedirs(out_dir, exist_ok=True)

@@ -4,16 +4,6 @@
 #pragma once
 #include "ndt2d_device.cuh"
 
-#ifndef NDT2D_EVAL_INLINE
-#define NDT2D_EVAL_INLINE 1 // 1: k_align inlines the evaluation into the LM loop (r2g: 18.70 vs 18.17 M matches/s - no spills at
-                            // 80 registers and both gathers of a step issue back to back); 0: a separate function, the round-1
-                            // form. The fused pairs kernel always calls it as a function: inlined, its code outgrows the
-                            // instruction cache (r2h: 9.7 vs 10.8 M pairs/s).
-#endif
-#ifndef NDT2D_PIPE
-#define NDT2D_PIPE 0      // align kernel: 1 = register software pipeline (K = 1)
-#endif
-
 namespace ndt2d {
 
 // SPEC 5, one pyramid level. Every lane carries the same f64 state (the butterfly reduction gives
@@ -53,13 +43,8 @@ struct WarpState {
 // never starts another scan, so desks are initialised once per launch. desk.active is 1 from the start of the launch
 // until the warp has seen the empty queue itself (a helper must not mistake a warp between two scans for a finished one).
 // ------------------------------------------------------------------------------------------------
-#ifndef NDT2D_ALIGN_THREADS
-#define NDT2D_ALIGN_THREADS 128
-#endif
-#ifndef NDT2D_HELP_SLEEP
-#define NDT2D_HELP_SLEEP 64   // ns a waiting helper sleeps between two polls of its owner's desk (0: spin)
-#endif
-static constexpr int ALIGN_THREADS = NDT2D_ALIGN_THREADS;
+static constexpr int ALIGN_THREADS = 128;
+static constexpr unsigned kHelpSleepNs = 64;   // a waiting helper sleeps between two polls of its owner's desk
 static constexpr int kAlignWarps = ALIGN_THREADS / 32;
 static constexpr int kMaxHelpers = kAlignWarps - 1 < 7 ? kAlignWarps - 1 : 7;
 static constexpr unsigned kNoHelper = 0xffffffffu;
@@ -177,11 +162,7 @@ __device__ __noinline__ void help_others(const LevelDev *lv)
         unsigned last = 0;
         for (;;) {
             unsigned post;
-            while ((post = lds_volatile(&d->post)) == last && lds_volatile(&d->active)) {
-#if NDT2D_HELP_SLEEP > 0
-                __nanosleep(NDT2D_HELP_SLEEP);
-#endif
-            }
+            while ((post = lds_volatile(&d->post)) == last && lds_volatile(&d->active)) __nanosleep(kHelpSleepNs);
             if (post == last) break;                              // the owner has finished its scan
             last = post;
             const unsigned nh = (post >> 4) & 15u, hs = post & 15u;
@@ -219,12 +200,11 @@ __device__ __forceinline__ void eval_to_smem_body(const LevelDev *L, const float
     const int lane = threadIdx.x & 31;
     const double *pose = ws->pn;
     Eval E;
-    constexpr int PIPE = (STAGED && OV == 0 && TABLE == TABLE_DENSE && !HELP) ? NDT2D_PIPE : 0;
     if (HELP) {
         const HelpPlan hp = post_help(level, n);
-        eval_warp<OV, true, STAGED, PIPE, true, TABLE, false, HelpPlan>(*L, pts, n, pose_for_level(pose[0], pose[1], pose[2], *L), lane, E, hp);
+        eval_warp<OV, true, STAGED, true, TABLE, false, HelpPlan>(*L, pts, n, pose_for_level(pose[0], pose[1], pose[2], *L), lane, E, hp);
     } else {
-        eval_warp<OV, true, STAGED, PIPE, true, TABLE>(*L, pts, n, pose_for_level(pose[0], pose[1], pose[2], *L), lane, E);
+        eval_warp<OV, true, STAGED, true, TABLE>(*L, pts, n, pose_for_level(pose[0], pose[1], pose[2], *L), lane, E);
     }
     __syncwarp();
     ws->t[E.slot] = E.v[0]; // lanes holding the same sum store the same bits
@@ -237,11 +217,14 @@ __device__ __noinline__ void eval_to_smem_call(const LevelDev *L, const float2 *
 {
     eval_to_smem_body<OV, STAGED, TABLE>(L, pts, n, ws);
 }
+// k_align inlines the evaluation into the LM loop (r2g: 18.70 vs 18.17 M matches/s against the call - no spills at 80
+// registers and both gathers of a step issue back to back). The fused pairs kernel calls it as a function: inlined, its
+// code outgrows the instruction cache (r2h: 9.7 vs 10.8 M pairs/s).
 template <int OV, bool STAGED, int TABLE, bool HELP = false>
 __device__ __forceinline__ void eval_to_smem(const LevelDev *L, const float2 *pts, int n, WarpState *ws, int level = 0)
 {
     if (HELP) eval_to_smem_body<OV, STAGED, TABLE, true>(L, pts, n, ws, level);
-    else if (NDT2D_EVAL_INLINE && TABLE != TABLE_SHASH) eval_to_smem_body<OV, STAGED, TABLE>(L, pts, n, ws);
+    else if (TABLE != TABLE_SHASH) eval_to_smem_body<OV, STAGED, TABLE>(L, pts, n, ws);
     else eval_to_smem_call<OV, STAGED, TABLE>(L, pts, n, ws);
 }
 

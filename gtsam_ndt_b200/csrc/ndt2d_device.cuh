@@ -15,26 +15,7 @@
 
 #include "ndt2d_internal.h"
 
-#ifndef NDT2D_UNROLL
-#define NDT2D_UNROLL 1
-#endif
-#ifndef NDT2D_JR1
-#define NDT2D_JR1 1 // 1: K = 1 kernels also take j from r by operand modifiers (see rotate_point)
-#endif
-#ifndef NDT2D_ESEL
-#define NDT2D_ESEL 1 // SPEC 4's pair tests, select and count written in PTX (see select_count)
-#endif
-#ifndef NDT2D_EXP_LEA
-#define NDT2D_EXP_LEA 1 // expneg2: the 2^-n factor from a shift-add on the integer pipe instead of an IMAD (see expneg2)
-#endif
-#ifndef NDT2D_LDMODE
-#define NDT2D_LDMODE 4 // cell gather instruction variant; 4 = ld.global.nc.L1::no_allocate, one 256-bit load (measured best:
-                       // a gathered record is rarely reused before L1 evicts it, and not allocating spares the fill bandwidth)
-#endif
-
 namespace ndt2d {
-
-static constexpr int kUnroll = NDT2D_UNROLL; // point-loop unroll of the non-pipelined evaluation
 
 typedef unsigned long long u64;
 
@@ -219,7 +200,6 @@ __device__ __forceinline__ float expneg(float h)
 __device__ __forceinline__ u64 expneg2(u64 nh)
 {
     const u64 MAGIC = bc(12582912.0f);
-#if NDT2D_EXP_LEA
     // The magic sum taken with the sign of n flipped: t = M - n (fma(-h, L, M); exact mirror of M + n, M's mantissa is even), so
     // that the bits of t are 0x4B400000 - n and 2^-n's bit pattern 0x3F800000 - (n << 23) is 0x3F800000 + (bits(t) << 23)
     // (0x4B400000 << 23 vanishes mod 2^32): one shift-add on the integer pipe per value, where n * -0x800000 + 0x3F800000 was
@@ -240,22 +220,6 @@ __device__ __forceinline__ u64 expneg2(u64 nh)
     p = fma2(p, y, bc(1.0f));
     p = fma2(p, y, bc(1.0f));
     return mul2(p, pk(__int_as_float((int)s0), __int_as_float((int)s1)));
-#else
-    u64 t = fma2(nh, bc(-1.44269502f), MAGIC);
-    u64 nf = sub2(t, MAGIC);
-    float t0, t1;
-    upk(t, t0, t1);
-    int n0 = __float_as_int(t0) - 0x4B400000, n1 = __float_as_int(t1) - 0x4B400000;
-    u64 y = fma2(nf, bc(0.693145752f), nh);
-    y = fma2(nf, bc(1.42860677e-6f), y);
-    u64 p = fma2(bc(1.38888889e-3f), y, bc(8.33333333e-3f));
-    p = fma2(p, y, bc(4.16666667e-2f));
-    p = fma2(p, y, bc(1.66666667e-1f));
-    p = fma2(p, y, bc(0.5f));
-    p = fma2(p, y, bc(1.0f));
-    p = fma2(p, y, bc(1.0f));
-    return mul2(p, pk(__int_as_float(0x3F800000 - n0 * 0x800000), __int_as_float(0x3F800000 - n1 * 0x800000)));
-#endif
 }
 
 // ---- SPEC 4: pose and point -----------------------------------------------------------------------------
@@ -358,7 +322,8 @@ struct PointPk {
 // (round-to-nearest is symmetric under negation), so j is r with its halves swapped and one sign flipped; ptxas folds
 // that into operand modifiers (.HI_LO.NP) and four packed instructions per step disappear. Measured: +2.3 % at K = 4 (v3), where j
 // is used by four cells; at K = 1 it was -2 % under SPEC v3 and is +5 % under v4 (x8: 20.31 vs 19.33 M matches/s - the f64
-// geometry made the loop longer and the four instructions count), so every kernel uses it now.
+// geometry made the loop longer and the four instructions count), so every evaluation uses it now. The diagnostic kernel
+// k_point_terms computes j as SPEC 4 writes it (JR = false), which the parity tests compare against.
 template <bool JR = false>
 __device__ __forceinline__ void rotate_point(const PosePk &P, float x, float y, PointPk &p)
 {
@@ -392,28 +357,10 @@ struct Cell4 {
 __device__ __forceinline__ Cell4 load_cell(const float4 *__restrict__ cells, unsigned idx)
 {
     Cell4 r;
-#ifdef NDT2D_PROBE_IDXMASK
-    idx &= NDT2D_PROBE_IDXMASK; // speed-of-light probe, never shipped: every gather lands in the same few lines (results are garbage)
-#endif
     const float4 *p = cells + 2 * (size_t)idx;
-#if NDT2D_LDMODE == 0
-    asm("ld.global.nc.v4.b64 {%0,%1,%2,%3}, [%4];" : "=l"(r.mu), "=l"(r.B0), "=l"(r.B1), "=l"(r.nv) : "l"(p));
-#elif NDT2D_LDMODE == 1
-    asm("ld.global.v4.b64 {%0,%1,%2,%3}, [%4];" : "=l"(r.mu), "=l"(r.B0), "=l"(r.B1), "=l"(r.nv) : "l"(p));
-#elif NDT2D_LDMODE == 2
-    asm("ld.global.nc.v2.b64 {%0,%1}, [%2];" : "=l"(r.mu), "=l"(r.B0) : "l"(p));
-    asm("ld.global.nc.v2.b64 {%0,%1}, [%2+16];" : "=l"(r.B1), "=l"(r.nv) : "l"(p));
-#elif NDT2D_LDMODE == 3
-    asm("ld.global.nc.L1::evict_last.v4.b64 {%0,%1,%2,%3}, [%4];" : "=l"(r.mu), "=l"(r.B0), "=l"(r.B1), "=l"(r.nv) : "l"(p));
-#elif NDT2D_LDMODE == 4
+    // L1::no_allocate (measured best of the gather forms): a gathered record is rarely reused before L1 evicts it, and not
+    // allocating spares the fill bandwidth
     asm("ld.global.nc.L1::no_allocate.v4.b64 {%0,%1,%2,%3}, [%4];" : "=l"(r.mu), "=l"(r.B0), "=l"(r.B1), "=l"(r.nv) : "l"(p));
-#elif NDT2D_LDMODE == 5
-    asm("ld.global.cg.v4.b64 {%0,%1,%2,%3}, [%4];" : "=l"(r.mu), "=l"(r.B0), "=l"(r.B1), "=l"(r.nv) : "l"(p));
-#elif NDT2D_LDMODE == 6
-    asm("ld.global.nc.L1::no_allocate.L2::256B.v4.b64 {%0,%1,%2,%3}, [%4];" : "=l"(r.mu), "=l"(r.B0), "=l"(r.B1), "=l"(r.nv) : "l"(p));
-#elif NDT2D_LDMODE == 7
-    asm("ld.global.nc.L1::evict_first.v4.b64 {%0,%1,%2,%3}, [%4];" : "=l"(r.mu), "=l"(r.B0), "=l"(r.B1), "=l"(r.nv) : "l"(p));
-#endif
     return r;
 }
 
@@ -535,16 +482,9 @@ __device__ __forceinline__ void cell_factors(const Cell4 &cA, const Cell4 &cB, c
     u64 nh = mul2(bc(-0.5f), pk(hsum(mul2(qA, uA)), hsum(mul2(qB, uB))));
     u64 e = expneg2(nh);
     // skipped pairs get e = 0: fma(0, c, acc) == acc bit for bit (every c is finite, see sanitize())
-#if NDT2D_ESEL
     // the two tests, the select and the count in PTX: one SEL and one predicated add per point (the compiler's own
     // expansion is a zero move plus a predicated move for the select and an add plus a predicated move for the count)
     F.e = pk(select_count<FULL>(hi32(cA.nv), lo32(nh), lo32(e), cnt), select_count<FULL>(hi32(cB.nv), hi32(nh), hi32(e), cnt));
-#else
-    bool okA = (hi32(cA.nv) != 0.0f) && (lo32(nh) > -30.0f);
-    bool okB = (hi32(cB.nv) != 0.0f) && (hi32(nh) > -30.0f);
-    F.e = pk(okA ? lo32(e) : 0.0f, okB ? hi32(e) : 0.0f);
-    if (FULL) cnt += (okA ? 1 : 0) + (okB ? 1 : 0);   // the score-only sweep reports no count
-#endif
     if (FULL) {
         float a2A = hsum(mul2(uA, A.j)), a2B = hsum(mul2(uB, B.j));
         u64 vA = fma2(cA.B0, bc(lo32(A.j)), mul2(cA.B1, bc(hi32(A.j))));
@@ -807,8 +747,8 @@ __device__ __forceinline__ void fetch(const float4 *__restrict__ cells, const La
     } else {
         float2 a, b;
         load_two<SMEM, ADDR>(pts, n, i, a, b);
-        rotate_point<OV != 0 || NDT2D_JR1>(P, a.x, a.y, F.A);
-        rotate_point<OV != 0 || NDT2D_JR1>(P, b.x, b.y, F.B);
+        rotate_point<true>(P, a.x, a.y, F.A);
+        rotate_point<true>(P, b.x, b.y, F.B);
         bA = locate_base(P, a.x, a.y, G, F.A.df);
         bB = locate_base(P, b.x, b.y, G, F.B.df);
     }
@@ -886,8 +826,6 @@ __device__ __forceinline__ void accumulate_step(const LatticePk &G, Fetched<OV> 
 
 // SPEC 4 for one warp. Lane l owns points 64 j + l (A) and 64 j + 32 + l (B), i.e. partials l and l + 32: each of the
 // two gather requests of an iteration then covers 32 consecutive beams (few distinct cache lines per request).
-// PIPE: software pipelining, the records of step j+1 are requested before step j is computed, so the L2 round
-// trip of the gathers overlaps this warp's own arithmetic (costs ~30 registers).
 // TR (FULL only): finish with the transposed reduction; E.v[0] is then sum number E.slot, the other E.v are unset.
 template <bool FULL, bool TR>
 __device__ __forceinline__ void finish_partials(const Partials &S, int cnt, int lane, Eval &E);
@@ -900,10 +838,10 @@ struct NoHelp {
 };
 
 // TABLE: how L's records are stored (TABLE_DENSE / TABLE_GHASH / TABLE_SHASH), resolved in fetch().
-// Help (SMEM, un-pipelined form only): the warp evaluates the first help.own_steps(steps) 64-point steps; help.finish()
+// Help (SMEM only): the warp evaluates the first help.own_steps(steps) 64-point steps; help.finish()
 // then applies the factors of the remaining steps, computed and parked by other warps, in step order (HelpPlan in
 // ndt2d_align.cuh) - SPEC 4's summation order is kept, so the sums are the same bits.
-template <int OV, bool FULL, bool SMEM, int PIPE, bool TR = false, int TABLE = TABLE_DENSE, bool P64 = false, class Help = NoHelp>
+template <int OV, bool FULL, bool SMEM, bool TR = false, int TABLE = TABLE_DENSE, bool P64 = false, class Help = NoHelp>
 __device__ __forceinline__ void eval_warp(const LevelDev &L, const float2 *pts, int n, const Pose32 &q, int lane, Eval &E,
                                           const Help help = Help())
 {
@@ -917,38 +855,13 @@ __device__ __forceinline__ void eval_warp(const LevelDev &L, const float2 *pts, 
     const PosePk P = pose_pack(q);
     const LatticePk G = lattice_pack<OV>(L, TABLE);
     const int npad = (n + 63) & ~63;
-    if (PIPE == 1 && OV == 0) {
-        // Software pipeline over registers, two steps per trip: the records of the next step are requested before
-        // the current step is computed. Inside the loop every fetch and every use is unconditional: ptxas sinks a
-        // load into the branch that uses it and merges conditionally loaded registers with a copy at the join,
-        // and either puts a consumer right behind the load it was meant to overlap. An odd step count is made
-        // even by one un-pipelined step up front; the last trip re-fetches the final step and drops it.
-        int i = lane;
-        if ((npad >> 6) & 1) {
-            Fetched<OV> cur;
-            fetch<OV, SMEM, TABLE, P64>(cells, G, P, pts, n, i, cur);
-            accumulate_step<OV, FULL>(G, cur, S, cnt);
-            i += 64;
-        }
-        if (i < npad) {
-            const int last = npad - 64 + lane;
-            Fetched<OV> F0, F1;
-            fetch<OV, SMEM, TABLE, P64>(cells, G, P, pts, n, i, F0);
-#pragma unroll 1
-            for (; i < npad; i += 128) {
-                fetch<OV, SMEM, TABLE, P64>(cells, G, P, pts, n, i + 64, F1);
-                accumulate_step<OV, FULL>(G, F0, S, cnt);
-                fetch<OV, SMEM, TABLE, P64>(cells, G, P, pts, n, min(i + 128, last), F0);
-                accumulate_step<OV, FULL>(G, F1, S, cnt);
-            }
-        }
-    } else if (SMEM) {
+    if (SMEM) {
         // the staged scan is walked by its shared-window address: one register is loop counter and load address at once (as
         // pts[i] the compiler recomputed slot base + warp * capacity + i with two multiply-adds and a constant load per step)
         constexpr unsigned PB = P64 ? 16u : 8u;     // bytes per staged point
         const unsigned s0 = (unsigned)__cvta_generic_to_shared(pts) + PB * (unsigned)lane;
         const unsigned s1 = s0 + PB * (Help::on ? 64u * help.own_steps((unsigned)npad >> 6) : (unsigned)npad);
-#pragma unroll kUnroll
+#pragma unroll 1
         for (unsigned sa = s0; sa < s1; sa += 64u * PB) {
             Fetched<OV> cur;
             fetch<OV, SMEM, TABLE, P64, true>(cells, G, P, pts, n, (int)sa, cur);
@@ -956,7 +869,7 @@ __device__ __forceinline__ void eval_warp(const LevelDev &L, const float2 *pts, 
         }
         if (Help::on) help.finish(S, cnt, lane);
     } else {
-#pragma unroll kUnroll
+#pragma unroll 1
         for (int i = lane; i < npad; i += 64) {
             Fetched<OV> cur;
             fetch<OV, SMEM, TABLE, P64>(cells, G, P, pts, n, i, cur);

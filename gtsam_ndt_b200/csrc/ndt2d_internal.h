@@ -64,7 +64,7 @@ struct LaunchCfg {
     int max_smem_optin;
     cudaStream_t stream;
     int block_align_max;     // calls with at most this many scans use the block-per-scan align kernel (-1: 8 x SMs)
-    int align_help;          // helper warps in k_align (K = 1, staged scans): 0 never, 1 always, -1 up to NDT2D_HELP_MAX_SCANS scans
+    int align_help;          // helper warps in k_align (K = 1, staged scans): 0 never, 1 always, -1 up to HELP_MAX_SCANS scans
 };
 
 // all launchers return the cudaError_t of the launch; *launches is incremented per kernel launched

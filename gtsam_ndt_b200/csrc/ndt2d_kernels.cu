@@ -5,9 +5,6 @@
 // These are gather-bound kernels over an L2-resident cell table: no tensor cores (north_star).
 // Reference file:line: none (the mount is /root/reference/README.md:1 only); arithmetic follows SPEC.md.
 #include "ndt2d_align.cuh"
-#ifdef NDT2D_PROBE_HALF
-#include "ndt2d_half_probe.cuh"
-#endif
 
 #include <math.h>
 #include <string.h>
@@ -177,30 +174,15 @@ __global__ void k_point_terms(const LevelDev L, const float2 *__restrict__ xy, i
 // ------------------------------------------------------------------------------------------------
 
 static constexpr int EVAL_THREADS = 256;
-#ifndef NDT2D_EVAL_PIPE
-#define NDT2D_EVAL_PIPE 0 // the same for k_eval_poses (evaluate / sweep)
-#endif
-#ifndef NDT2D_SWEEP_P64
-#define NDT2D_SWEEP_P64 1 // the score-only sweep stages the scan as f64 (no input conversions in the loop)
-#endif
-#ifndef NDT2D_EVAL_BLOCKS
-#define NDT2D_EVAL_BLOCKS 4 // resident k_eval_poses blocks per SM for the score-only sweep: 4 (32 warps, 56 registers) and 5 (40 warps, 48
-                            // registers) both reach 446.8 M hypotheses/s, 6 (48 warps, 40 registers: constants re-materialised in the loop) 434 M
-#endif
-#ifndef NDT2D_QUEUE
-#define NDT2D_QUEUE 0 // 0: one global atomic work queue; 1: static per-block ranges (tuning experiment, slower)
-#endif
-static constexpr int EVAL_PIPE = NDT2D_EVAL_PIPE;
-#ifdef NDT2D_PROBE_HALF
-static constexpr int EVAL_BLOCKS_FULL = NDT2D_PROBE_HALF; // probe: resident blocks of the one-point-per-lane evaluation
-#else
+// resident k_eval_poses blocks per SM for the score-only sweep: 4 (32 warps, 56 registers) and 5 (40 warps, 48 registers) both
+// reach 446.8 M hypotheses/s, 6 (48 warps, 40 registers: constants re-materialised in the loop) 434 M
+static constexpr int EVAL_BLOCKS = 4;
 static constexpr int EVAL_BLOCKS_FULL = 3; // the full evaluation needs the align kernel's 80 registers: 24 warps per SM
-#endif
 
 // Block stages the scan in shared memory once (coalesced float2 loads), then each warp takes poses
 // from a grid-stride loop. FULL: ten f64 sums per pose; otherwise the score only (sweep).
 template <int OV, bool FULL, bool F32POSE, bool STAGED>
-__global__ void __launch_bounds__(EVAL_THREADS, FULL ? EVAL_BLOCKS_FULL : NDT2D_EVAL_BLOCKS) k_eval_poses(const LevelDev L, const float2 *__restrict__ xy, int n,
+__global__ void __launch_bounds__(EVAL_THREADS, FULL ? EVAL_BLOCKS_FULL : EVAL_BLOCKS) k_eval_poses(const LevelDev L, const float2 *__restrict__ xy, int n,
                                                                const void *__restrict__ poses, int64_t npose,
                                                                double *__restrict__ out, int out_stride,
                                                                int32_t *__restrict__ count)
@@ -208,7 +190,7 @@ __global__ void __launch_bounds__(EVAL_THREADS, FULL ? EVAL_BLOCKS_FULL : NDT2D_
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int npad = (n + 63) & ~63;
     float2 *sp = reinterpret_cast<float2 *>(smem_raw);
-    constexpr bool P64 = NDT2D_SWEEP_P64 && STAGED && !FULL;   // the score-only sweep needs the points in f64 only: widen them once, here
+    constexpr bool P64 = STAGED && !FULL;   // the score-only sweep needs the points in f64 only: widen them once, here
     if (STAGED) {
         // sanitised points, padded with the far-away point to a multiple of 64 (SPEC 4)
         for (int i = threadIdx.x; i < npad; i += blockDim.x) {
@@ -232,12 +214,8 @@ __global__ void __launch_bounds__(EVAL_THREADS, FULL ? EVAL_BLOCKS_FULL : NDT2D_
         Pose32 q = pose_for_level<!FULL>(tx, ty, th, L);   // the score-only sweep takes the sin/cos coefficients from constant memory
         Eval E;
         // FULL: the transposed reduction leaves sum number E.slot in every lane (lanes with the same slot hold the same bits)
-#ifdef NDT2D_PROBE_HALF
-        if (STAGED && FULL && OV == 0) eval_warp_half_probe<true>(L, sp, n, q, lane, E);
-        else
-#endif
-        if (STAGED) eval_warp<OV, FULL, true, OV == 0 ? EVAL_PIPE : 0, FULL, TABLE_DENSE, P64>(L, sp, n, q, lane, E);
-        else eval_warp<OV, FULL, false, 0, FULL>(L, xy, n, q, lane, E);
+        if (STAGED) eval_warp<OV, FULL, true, FULL, TABLE_DENSE, P64>(L, sp, n, q, lane, E);
+        else eval_warp<OV, FULL, false, FULL>(L, xy, n, q, lane, E);
         if (FULL) out[(size_t)j * out_stride + E.slot] = E.v[0];
         else if (lane == 0) out[(size_t)j * out_stride] = E.v[0];
         if (count && lane == 0) count[j] = E.count;
@@ -252,16 +230,12 @@ __global__ void __launch_bounds__(EVAL_THREADS, FULL ? EVAL_BLOCKS_FULL : NDT2D_
 // on configs[1], all bit-identical): 128 x 6: 20.46, 256 x 3: 20.32, 384 x 2: 20.22 (the same 24 warps in larger blocks: a block
 // holds its shared memory until its last warp has drained the queue), 160 x 4 (20 warps, 96 registers): 19.53, 320 x 2 (20
 // warps): 19.43, 256 x 2 (16 warps, 104 registers, the only point whose loop has no register copies): 19.17.
-// ALIGN_THREADS (k_align's block size, NDT2D_ALIGN_THREADS) lives in ndt2d_align.cuh with the helper-warp machinery
-#ifndef NDT2D_HELP_MAX_SCANS
-#define NDT2D_HELP_MAX_SCANS 8192 // batches of at most this many scans run k_align with helper warps, when the handle leaves the choice open
-                                  // (tools/midsize_probe.py: -12 % at 1250-2500 scans, -5 % at 5000, +-0 at 10 000, +2 % at 20 000,
-                                  // +8 % at 65 536 - the helper form's point loop is 134 instructions against 129)
-#endif
-#ifndef NDT2D_ALIGN_MIN_BLOCKS
-#define NDT2D_ALIGN_MIN_BLOCKS 6
-#endif
-static constexpr int ALIGN_MIN_BLOCKS = NDT2D_ALIGN_MIN_BLOCKS;
+// ALIGN_THREADS (k_align's block size) lives in ndt2d_align.cuh with the helper-warp machinery
+static constexpr int ALIGN_MIN_BLOCKS = 6;
+// batches of at most this many scans run k_align with helper warps, when the handle leaves the choice open
+// (tools/midsize_probe.py: -12 % at 1250-2500 scans, -5 % at 5000, +-0 at 10 000, +2 % at 20 000,
+// +8 % at 65 536 - the helper form's point loop is 134 instructions against 129)
+static constexpr int HELP_MAX_SCANS = 8192;
 
 // ------------------------------------------------------------------------------------------------
 // (2d) low-latency align: one BLOCK per scan, for calls with few scans (a single align above all)
@@ -273,10 +247,7 @@ static constexpr int ALIGN_MIN_BLOCKS = NDT2D_ALIGN_MIN_BLOCKS;
 // sums, and everything after, are the bits of the one-warp kernel. The LM logic is executed by every thread on the same
 // shared-memory state (uniform).
 
-#ifndef NDT2D_BLOCK_ALIGN_THREADS
-#define NDT2D_BLOCK_ALIGN_THREADS 256
-#endif
-static constexpr int BLOCK_ALIGN_THREADS = NDT2D_BLOCK_ALIGN_THREADS; // at least 5 warps (the second half of eval_block)
+static constexpr int BLOCK_ALIGN_THREADS = 256; // at least 5 warps (the second half of eval_block)
 static_assert(BLOCK_ALIGN_THREADS >= 160 && BLOCK_ALIGN_THREADS % 32 == 0, "eval_block applies the factors with five warps");
 
 template <int OV>
@@ -459,22 +430,9 @@ __global__ void __launch_bounds__(ALIGN_THREADS, (STAGED || RANGES) ? ALIGN_MIN_
         __syncthreads();
     }
 
-#if NDT2D_QUEUE == 1
-    // static ranges (tuning experiment): each block owns a contiguous range of scans
-    __shared__ unsigned s_next;
-    const unsigned q_lo = (unsigned)(((unsigned long long)blockIdx.x * (unsigned)a.nscans) / gridDim.x);
-    const unsigned q_hi = (unsigned)(((unsigned long long)(blockIdx.x + 1) * (unsigned)a.nscans) / gridDim.x);
-    if (threadIdx.x == 0) s_next = q_lo;
-    __syncthreads();
-#endif
     bool first_job = true;
     for (;;) {
         unsigned job = 0;
-#if NDT2D_QUEUE == 1
-        if (lane == 0) job = atomicAdd(&s_next, 1u);
-        job = __shfl_sync(FULL_MASK, job, 0);
-        const bool drained = job >= q_hi;
-#else
         if (HELP && first_job) {
             // a warp's first scan is assigned statically, warp w of every block before warp w + 1 of any: a batch that does
             // not fill the GPU is spread over the blocks, and the warps left without a scan are helpers next to an owner
@@ -486,7 +444,6 @@ __global__ void __launch_bounds__(ALIGN_THREADS, (STAGED || RANGES) ? ALIGN_MIN_
             if (HELP) job += gridDim.x * (unsigned)kAlignWarps;
         }
         const bool drained = job >= (unsigned)a.nscans;
-#endif
         if (drained) {
             if (HELP) {
                 if (lane == 0) sts_volatile(&help_desk(warp)->active, 0u);   // releases this warp's helpers
@@ -690,8 +647,8 @@ template <int OV, bool FULL, bool F32POSE>
 static cudaError_t launch_eval_t(const LaunchCfg &c, const LevelDev &L, const float2 *d_xy, int n, const void *d_poses,
                                  int64_t npose, double *d_out, int out_stride, int32_t *d_count)
 {
-    size_t smem = (size_t)((n + 63) & ~63) * ((FULL || !NDT2D_SWEEP_P64) ? sizeof(float2) : sizeof(double2));   // score only: points staged as f64
-    int grid = grid_for(npose, EVAL_THREADS / 32, c.sm_count, FULL ? EVAL_BLOCKS_FULL : NDT2D_EVAL_BLOCKS);
+    size_t smem = (size_t)((n + 63) & ~63) * (FULL ? sizeof(float2) : sizeof(double2));   // score only: points staged as f64
+    int grid = grid_for(npose, EVAL_THREADS / 32, c.sm_count, FULL ? EVAL_BLOCKS_FULL : EVAL_BLOCKS);
     if (smem <= (size_t)c.max_smem_optin - 1024) {
         auto kern = k_eval_poses<OV, FULL, F32POSE, true>;
         if (smem > 48 * 1024) {
@@ -748,12 +705,6 @@ static cudaError_t launch_align_t(const LaunchCfg &c, const AlignArgs &a)
     cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, ALIGN_THREADS, smem);
     if (e != cudaSuccess) return e;
     if (per_sm < 1) per_sm = 1;
-#ifdef NDT2D_MAX_BLOCKS_PER_SM
-    if (per_sm > NDT2D_MAX_BLOCKS_PER_SM) per_sm = NDT2D_MAX_BLOCKS_PER_SM;
-#endif
-#ifdef NDT2D_PAIRS_BLOCKS_PER_SM
-    if (PAIRS && per_sm > NDT2D_PAIRS_BLOCKS_PER_SM) per_sm = NDT2D_PAIRS_BLOCKS_PER_SM; // fewer tables in flight: L2 residency experiment
-#endif
     // HELP: one block per scan while blocks are free (its other warps start as helpers); the first scans are dealt out
     // warp 0 of every block first
     int grid = grid_for(a.nscans, HELP ? 1 : ALIGN_THREADS / 32, c.sm_count, per_sm);
@@ -796,7 +747,7 @@ cudaError_t launch_align(const LaunchCfg &c, const AlignArgs &a, int64_t *launch
         return staged ? launch_align_t<1, true, false>(c, a) : launch_align_t<1, false, false>(c, a);
     }
     // K = 1, scans in shared memory: the helper-warp form (c.align_help: 0 never, 1 always, -1 = batches whose tail matters)
-    const bool help = c.align_help > 0 || (c.align_help < 0 && (a.batch_scans > 0 ? a.batch_scans : a.nscans) <= NDT2D_HELP_MAX_SCANS);
+    const bool help = c.align_help > 0 || (c.align_help < 0 && (a.batch_scans > 0 ? a.batch_scans : a.nscans) <= HELP_MAX_SCANS);
     if (ranges) return help ? launch_align_t<0, true, true, false, true>(c, a) : launch_align_t<0, true, true>(c, a);
     if (staged) return help ? launch_align_t<0, true, false, false, true>(c, a) : launch_align_t<0, true, false>(c, a);
     return launch_align_t<0, false, false>(c, a);

@@ -126,7 +126,7 @@ int upload(ndt2d_matcher *m, DevBuf &b, const void *src, size_t bytes)
 }
 
 // shared-memory slot capacity (points per warp) for the align kernel; 0 = read scans from global memory
-int align_cap_points(const ndt2d_matcher *m, int max_points)
+static int align_cap_points(const ndt2d_matcher *m, int max_points)
 {
     int cap = (max_points + 63) & ~63; // two NaN-padded planes per warp, 64 points per warp iteration
     if (cap < 64) cap = 64;
@@ -151,13 +151,21 @@ int ensure_beams(ndt2d_matcher *m, int nbeams, double angle_min, double angle_in
     return NDT2D_OK;
 }
 
-void fill_align_args(ndt2d_matcher *m, AlignArgs &a)
+int align_device(ndt2d_matcher *m, AlignArgs a, int max_points, double angle_min, double angle_inc)
 {
-    memset(&a, 0, sizeof(a));
+    a.cap_points = align_cap_points(m, max_points);
+    if (a.ranges) {     // LaserScan ranges are converted in the staging step, so they need the shared-memory slot
+        if (a.cap_points == 0) return fail(m, NDT2D_EINVAL, "nbeams %d exceeds the shared-memory staging limit", a.nbeams);
+        int rc = ensure_beams(m, a.nbeams, angle_min, angle_inc);
+        if (rc) return rc;
+        a.beams = m->b_beams.as<float2>();
+    }
     for (int l = 0; l < m->nlevels; ++l) a.lv[l] = m->lv[l];
     a.nlevels = m->nlevels;
     a.prm = m->prm;
-    a.counter = m->b_counter.as<unsigned int>();
+    if (!a.counter) a.counter = m->b_counter.as<unsigned int>();
+    CK(m, launch_align(m->cfg, a, &m->launches));
+    return NDT2D_OK;
 }
 
 // Host-buffer batch driver shared by the xy and ranges entry points. The input is cut into chunks; chunk
@@ -172,11 +180,10 @@ struct ChunkPlan {
 // copy and last kernel (measured on PCIe 5 x16, 65 536 scans: 8192-scan chunks 10.1 M matches/s, 4096-scan chunks
 // 10.7-11.5 M); a kernel-bound call (u16 ranges) wants large ones, since every chunk is a launch with its own partial
 // last wave (15.9 M vs 15.1 M). About 18 MB per chunk gives 16 chunks for the former and 8 for the latter.
-ChunkPlan plan_chunks(const ndt2d_matcher *m, int nscans, size_t total_bytes)
+ChunkPlan plan_chunks(int nscans, size_t total_bytes)
 {
     ChunkPlan p;
-    if (m->chunk_scans > 0) p.nchunks = (nscans + m->chunk_scans - 1) / m->chunk_scans;
-    else p.nchunks = (int)((total_bytes + (18u << 20) - 1) / (18u << 20));
+    p.nchunks = (int)((total_bytes + (18u << 20) - 1) / (18u << 20));
     if (p.nchunks > ndt2d_matcher::MAX_CHUNKS) p.nchunks = ndt2d_matcher::MAX_CHUNKS;
     if (p.nchunks < 1) p.nchunks = 1;
     p.per = (nscans + p.nchunks - 1) / p.nchunks;
@@ -210,7 +217,7 @@ static void release_relay(ndt2d_matcher *m)
 template <typename DescFn, typename LaunchFn>
 int run_pipeline(ndt2d_matcher *m, int nscans, size_t total_bytes, ndt2d_result *res, DescFn chunk_desc, LaunchFn launch_chunk)
 {
-    const ChunkPlan pl = plan_chunks(m, nscans, total_bytes);
+    const ChunkPlan pl = plan_chunks(nscans, total_bytes);
     const bool relay = m->relay_dev >= 0 && pl.nchunks > 1;
     if (relay && m->relay_cap < total_bytes) {          // the relay GPU mirrors the call's input buffer
         DeviceGuard g(m->relay_dev);
@@ -339,10 +346,6 @@ int ndt2d_create_on_stream(int device, void *cuda_stream, ndt2d_matcher **out)
         if (const char *e = getenv("NDT2D_BLOCK_ALIGN_MAX")) m->cfg.block_align_max = atoi(e); // 0: always one warp per scan
         m->cfg.align_help = -1;
         if (const char *e = getenv("NDT2D_ALIGN_HELP")) m->cfg.align_help = atoi(e);             // 0: never, 1: always
-        if (const char *e = getenv("NDT2D_CHUNK_SCANS")) {
-            int v = atoi(e);
-            if (v > 0) m->chunk_scans = v;
-        }
     }
     if (m->b_counter.ensure(4 * (ndt2d_matcher::MAX_CHUNKS + 1)) != cudaSuccess || m->b_box.ensure(16) != cudaSuccess ||
         m->b_scratch.ensure(sizeof(unsigned long long) * (size_t)topk_scratch_words(m->cfg.sm_count)) != cudaSuccess) {
@@ -800,18 +803,8 @@ int ndt2d_point_terms(ndt2d_matcher *m, int level, const float *xy, int n, const
     return ndt2d_synchronize(m);
 }
 
-static int align_batch_device_impl(ndt2d_matcher *m, const float *d_xy, const int64_t *d_offsets, int nscans, int max_points,
-                                   const double *d_init, ndt2d_result *d_res, unsigned int *counter, int batch_scans = 0);
-
 int ndt2d_align_batch_device(ndt2d_matcher *m, const float *d_xy, const int64_t *d_offsets, int nscans, int max_points,
                              const double *d_init, ndt2d_result *d_res)
-{
-    return align_batch_device_impl(m, d_xy, d_offsets, nscans, max_points, d_init, d_res, nullptr);
-}
-
-// counter / batch_scans: set when this launch is one chunk of a pipelined host-buffer call of batch_scans scans
-static int align_batch_device_impl(ndt2d_matcher *m, const float *d_xy, const int64_t *d_offsets, int nscans, int max_points,
-                                   const double *d_init, ndt2d_result *d_res, unsigned int *counter, int batch_scans)
 {
     if (!m) return NDT2D_EINVAL;
     if (!m->has_target) return fail(m, NDT2D_ENOTARGET, "no target set");
@@ -819,35 +812,24 @@ static int align_batch_device_impl(ndt2d_matcher *m, const float *d_xy, const in
         return fail(m, NDT2D_EINVAL, "bad arguments");
     if (nscans == 0) return NDT2D_OK;
     DeviceGuard g(m->device);
-    AlignArgs a;
-    fill_align_args(m, a);
+    AlignArgs a{};
     a.xy = reinterpret_cast<const float2 *>(d_xy);
-    if (!a.xy) a.xy = m->b_counter.as<float2>(); // all scans empty: any non-null pointer selects the xy path
     a.offsets = d_offsets;
     a.init = d_init;
     a.res = d_res;
     a.nscans = nscans;
-    a.cap_points = align_cap_points(m, max_points);
-    if (counter) a.counter = counter;
-    a.batch_scans = batch_scans;
-    CK(m, launch_align(m->cfg, a, &m->launches));
-    return NDT2D_OK;
+    return align_device(m, a, max_points);
 }
 
-// Small host-buffer batches (a single align above all): offsets, initial poses and points are packed into one pinned
-// buffer and go up in ONE copy, the kernel writes its results into mapped pinned memory, the queue counter comes from a
-// pre-zeroed ring: copy, launch, synchronise - instead of the ~15 calls of the chunked pipeline.
-// the buffers of the small-call path (align_batch_fast, align_ranges_fast), and a zeroed work-queue counter from the ring
+// Small host-buffer batches (a single align above all): offsets, initial poses and scans are packed into one pinned
+// buffer and go up in ONE upload, the kernel writes its results into mapped pinned memory, the queue counter comes from a
+// pre-zeroed ring: upload, launch, synchronise - instead of the ~15 calls of the chunked pipeline.
+// the buffers of the small-call path (align_small), and a zeroed work-queue counter from the ring
 static int fast_prepare(ndt2d_matcher *m)
 {
     if (!m->fast_ready) {   // set only after every allocation below has succeeded: a failed attempt is simply repeated
         if (!m->fast_host) CK(m, cudaHostAlloc(reinterpret_cast<void **>(&m->fast_host), ndt2d_matcher::FAST_BYTES, cudaHostAllocMapped));
         CK(m, cudaHostGetDevicePointer(reinterpret_cast<void **>(&m->fast_host_dev), m->fast_host, 0));
-        // small xy calls: the block kernel stages its input straight from the mapped staging buffer (8.6 KB over PCIe, every
-        // thread with a load in flight) - one copy operation fewer per call, 66.7 -> 62.3 us for a 1080-point align; the ranges
-        // form keeps the copy (one warp converts the beams: 34 dependent PCIe round trips measured 102 us against 83 us)
-        m->fast_zerocopy = true;
-        if (const char *e = getenv("NDT2D_FAST_ZEROCOPY")) m->fast_zerocopy = atoi(e) != 0;
         if (!m->fast_res) CK(m, cudaHostAlloc(reinterpret_cast<void **>(&m->fast_res), ndt2d_matcher::FAST_SCANS * sizeof(ndt2d_result), cudaHostAllocMapped));
         CK(m, cudaHostGetDevicePointer(reinterpret_cast<void **>(&m->fast_res_dev), m->fast_res, 0));
         CK(m, m->b_fast.ensure(ndt2d_matcher::FAST_BYTES));
@@ -863,33 +845,86 @@ static int fast_prepare(ndt2d_matcher *m)
     return NDT2D_OK;
 }
 
-static int align_batch_fast(ndt2d_matcher *m, const float *xy, const int64_t *offsets, int nscans, int64_t total, int64_t maxn,
-                            const double *init, ndt2d_result *res)
+// `a`: the call's input in host memory, as align_host takes it; scan_bytes: its scans. Packed layout: offsets (points
+// only) | init | scans, every section at a multiple of 8 bytes.
+static int align_small(ndt2d_matcher *m, AlignArgs a, size_t scan_bytes, int max_points, const double *init, ndt2d_result *res,
+                       double angle_min, double angle_inc)
 {
-    int rcp = fast_prepare(m);
-    if (rcp) return rcp;
-    const size_t off_bytes = (size_t)(nscans + 1) * 8, init_bytes = (size_t)nscans * 24, xy_bytes = (size_t)total * 8;
+    int rc = fast_prepare(m);
+    if (rc) return rc;
+    const bool ranges = a.ranges != nullptr;
+    const size_t off_bytes = ranges ? 0 : (size_t)(a.nscans + 1) * 8, init_bytes = (size_t)a.nscans * 24;
     unsigned char *h = m->fast_host;
-    memcpy(h, offsets, off_bytes);
+    if (off_bytes) memcpy(h, a.offsets, off_bytes);
     memcpy(h + off_bytes, init, init_bytes);
-    if (xy_bytes) memcpy(h + off_bytes + init_bytes, xy, xy_bytes);
-    unsigned char *d = m->fast_zerocopy ? m->fast_host_dev : m->b_fast.as<unsigned char>();
-    if (!m->fast_zerocopy) CK(m, cudaMemcpyAsync(d, h, off_bytes + init_bytes + xy_bytes, cudaMemcpyHostToDevice, m->cfg.stream));
-    AlignArgs a;
-    fill_align_args(m, a);
-    a.offsets = reinterpret_cast<const int64_t *>(d);
+    if (scan_bytes) memcpy(h + off_bytes + init_bytes, ranges ? a.ranges : static_cast<const void *>(a.xy), scan_bytes);
+    // Point scans are staged by the block kernel straight from the mapped staging buffer (8.6 KB over PCIe, every thread
+    // with a load in flight): one copy operation fewer per call, 66.7 -> 62.3 us for a 1080-point align. LaserScan ranges
+    // are copied first: one warp converts the beams, and from mapped memory its 34 dependent PCIe round trips measured
+    // 102 us against 83 us.
+    unsigned char *d = ranges ? m->b_fast.as<unsigned char>() : m->fast_host_dev;
+    if (ranges) CK(m, cudaMemcpyAsync(d, h, init_bytes + scan_bytes, cudaMemcpyHostToDevice, m->cfg.stream));
+    const unsigned char *scans = d + off_bytes + init_bytes;
+    if (ranges) {
+        a.ranges = scans;
+    } else {
+        a.offsets = reinterpret_cast<const int64_t *>(d);
+        a.xy = reinterpret_cast<const float2 *>(scans);
+    }
     a.init = reinterpret_cast<const double *>(d + off_bytes);
-    a.xy = reinterpret_cast<const float2 *>(d + off_bytes + init_bytes);
     a.res = m->fast_res_dev;
-    a.nscans = nscans;
-    a.cap_points = align_cap_points(m, (int)maxn);
     a.counter = m->b_ring.as<unsigned int>() + m->ring_pos++;
     a.counter_is_zero = 1;
-    CK(m, launch_align(m->cfg, a, &m->launches));
-    int rc = ndt2d_synchronize(m);
-    if (rc) return rc;
-    memcpy(res, m->fast_res, (size_t)nscans * sizeof(ndt2d_result));
+    if ((rc = align_device(m, a, max_points, angle_min, angle_inc))) return rc;
+    if ((rc = ndt2d_synchronize(m))) return rc;
+    memcpy(res, m->fast_res, (size_t)a.nscans * sizeof(ndt2d_result));
     return NDT2D_OK;
+}
+
+// The host-buffer batch of ndt2d_align_batch and ndt2d_align_batch_ranges, after their argument checks. `in` is the call's
+// input as the caller passed it, in host memory: in.nscans scans of at most max_points points each, as xy and offsets or as
+// ranges with their beam fields. Small calls take align_small, the others the chunked pipeline.
+static int align_host(ndt2d_matcher *m, const AlignArgs &in, int max_points, const double *init, ndt2d_result *res,
+                      double angle_min = 0.0, double angle_inc = 0.0)
+{
+    const int nscans = in.nscans;
+    const bool ranges = in.ranges != nullptr;
+    const unsigned char *src = static_cast<const unsigned char *>(ranges ? in.ranges : static_cast<const void *>(in.xy));
+    const size_t row = (size_t)in.nbeams * (in.ranges_u16 ? 2 : 4);
+    auto pos = [&](int s) { return ranges ? (size_t)s * row : (size_t)in.offsets[s] * 8; };  // first byte of scan s in src
+    const size_t off_bytes = ranges ? 0 : (size_t)(nscans + 1) * 8, init_bytes = (size_t)nscans * 24;
+    if (nscans <= ndt2d_matcher::FAST_SCANS && pos(0) == 0 && off_bytes + init_bytes + pos(nscans) <= ndt2d_matcher::FAST_BYTES)
+        return align_small(m, in, pos(nscans), max_points, init, res, angle_min, angle_inc);
+    DevBuf &buf = ranges ? m->b_ranges : m->b_xy;
+    int rc;
+    CK(m, buf.ensure(std::max<size_t>(pos(nscans), 8)));
+    CK(m, m->b_res.ensure((size_t)nscans * sizeof(ndt2d_result)));
+    if (!ranges && (rc = upload(m, m->b_off, in.offsets, off_bytes))) return rc;
+    if ((rc = upload(m, m->b_init, init, init_bytes))) return rc;
+    if (ranges && (rc = ensure_beams(m, in.nbeams, angle_min, angle_inc))) return rc; // on the main stream, before the work streams fork
+    unsigned char *dev = buf.as<unsigned char>();
+    return run_pipeline(
+        m, nscans, pos(nscans), res,
+        [&](int s0, int s1, void **dst, const void **from, size_t *bytes) {
+            *dst = dev + pos(s0);
+            *from = src + pos(s0);
+            *bytes = pos(s1) - pos(s0);
+        },
+        [&](int s0, int s1, unsigned int *counter) -> int {
+            AlignArgs a = in;
+            if (ranges) {
+                a.ranges = dev + pos(s0);
+            } else {            // the points keep their place in the batch: the offsets index them
+                a.xy = reinterpret_cast<const float2 *>(dev);
+                a.offsets = m->b_off.as<int64_t>() + s0;
+            }
+            a.init = m->b_init.as<double>() + 3 * (size_t)s0;
+            a.res = m->b_res.as<ndt2d_result>() + s0;
+            a.nscans = s1 - s0;
+            a.counter = counter;
+            a.batch_scans = nscans;
+            return align_device(m, a, max_points, angle_min, angle_inc);
+        });
 }
 
 int ndt2d_align_batch(ndt2d_matcher *m, const float *xy, const int64_t *offsets, int nscans, const double *init,
@@ -908,26 +943,11 @@ int ndt2d_align_batch(ndt2d_matcher *m, const float *xy, const int64_t *offsets,
     int64_t total = offsets[nscans];
     if (offsets[0] < 0 || (total > 0 && !xy)) return fail(m, NDT2D_EINVAL, "bad offsets / xy");
     DeviceGuard g(m->device);
-    if (nscans <= ndt2d_matcher::FAST_SCANS && offsets[0] == 0 &&
-        (size_t)(nscans + 1) * 8 + (size_t)nscans * 24 + (size_t)total * 8 <= ndt2d_matcher::FAST_BYTES)
-        return align_batch_fast(m, xy, offsets, nscans, total, maxn, init, res);
-    int rc;
-    CK(m, m->b_xy.ensure((size_t)(total ? total : 1) * 8));
-    CK(m, m->b_res.ensure((size_t)nscans * sizeof(ndt2d_result)));
-    if ((rc = upload(m, m->b_off, offsets, (size_t)(nscans + 1) * 8))) return rc;
-    if ((rc = upload(m, m->b_init, init, (size_t)nscans * 24))) return rc;
-    return run_pipeline(
-        m, nscans, (size_t)total * 8, res,
-        [&](int s0, int s1, void **dst, const void **src, size_t *bytes) {
-            int64_t p0 = offsets[s0], p1 = offsets[s1];
-            *dst = m->b_xy.as<float>() + 2 * p0;
-            *src = xy + 2 * p0;
-            *bytes = (size_t)(p1 - p0) * 8;
-        },
-        [&](int s0, int s1, unsigned int *counter) -> int {
-            return align_batch_device_impl(m, m->b_xy.as<float>(), m->b_off.as<int64_t>() + s0, s1 - s0, (int)maxn,
-                                           m->b_init.as<double>() + 3 * (size_t)s0, m->b_res.as<ndt2d_result>() + s0, counter, nscans);
-        });
+    AlignArgs in{};
+    in.xy = reinterpret_cast<const float2 *>(xy);
+    in.offsets = offsets;
+    in.nscans = nscans;
+    return align_host(m, in, (int)maxn, init, res);
 }
 
 int ndt2d_align(ndt2d_matcher *m, const float *xy, int n, const double init[3], ndt2d_result *res)
@@ -937,21 +957,22 @@ int ndt2d_align(ndt2d_matcher *m, const float *xy, int n, const double init[3], 
     return ndt2d_align_batch(m, xy, off, 1, init, res);
 }
 
-static int align_ranges_device_impl(ndt2d_matcher *m, const void *d_ranges, int ranges_are_u16, int nscans, int nbeams,
-                                    double angle_min, double angle_inc, float range_scale, float range_min, float range_max,
-                                    const double *d_init, ndt2d_result *d_res, unsigned int *counter, int batch_scans = 0);
+// the LaserScan input of an align (SPEC 8); align_device adds the beam table
+static AlignArgs ranges_input(const void *ranges, int ranges_are_u16, int nscans, int nbeams, float range_scale, float range_min,
+                              float range_max)
+{
+    AlignArgs a{};
+    a.ranges = ranges;
+    a.ranges_u16 = ranges_are_u16 ? 1 : 0;
+    a.nbeams = nbeams;
+    a.range_scale = range_scale; a.range_min = range_min; a.range_max = range_max;
+    a.nscans = nscans;
+    return a;
+}
 
 int ndt2d_align_batch_ranges_device(ndt2d_matcher *m, const void *d_ranges, int ranges_are_u16, int nscans, int nbeams,
                                     double angle_min, double angle_inc, float range_scale, float range_min, float range_max,
                                     const double *d_init, ndt2d_result *d_res)
-{
-    return align_ranges_device_impl(m, d_ranges, ranges_are_u16, nscans, nbeams, angle_min, angle_inc, range_scale, range_min,
-                                    range_max, d_init, d_res, nullptr);
-}
-
-static int align_ranges_device_impl(ndt2d_matcher *m, const void *d_ranges, int ranges_are_u16, int nscans, int nbeams,
-                                    double angle_min, double angle_inc, float range_scale, float range_min, float range_max,
-                                    const double *d_init, ndt2d_result *d_res, unsigned int *counter, int batch_scans)
 {
     if (!m) return NDT2D_EINVAL;
     if (!m->has_target) return fail(m, NDT2D_ENOTARGET, "no target set");
@@ -959,65 +980,10 @@ static int align_ranges_device_impl(ndt2d_matcher *m, const void *d_ranges, int 
         return fail(m, NDT2D_EINVAL, "bad arguments");
     if (nscans == 0) return NDT2D_OK;
     DeviceGuard g(m->device);
-    int cap = align_cap_points(m, nbeams);
-    if (cap == 0) return fail(m, NDT2D_EINVAL, "nbeams %d exceeds the shared-memory staging limit", nbeams);
-    {
-        int rcb = ensure_beams(m, nbeams, angle_min, angle_inc);
-        if (rcb) return rcb;
-    }
-    AlignArgs a;
-    fill_align_args(m, a);
-    a.xy = nullptr;
-    a.ranges = d_ranges;
-    a.beams = m->b_beams.as<float2>();
-    a.ranges_u16 = ranges_are_u16 ? 1 : 0;
-    a.nbeams = nbeams;
-    a.range_scale = range_scale; a.range_min = range_min; a.range_max = range_max;
+    AlignArgs a = ranges_input(d_ranges, ranges_are_u16, nscans, nbeams, range_scale, range_min, range_max);
     a.init = d_init;
     a.res = d_res;
-    a.nscans = nscans;
-    a.cap_points = cap;
-    if (counter) a.counter = counter;
-    a.batch_scans = batch_scans;
-    CK(m, launch_align(m->cfg, a, &m->launches));
-    return NDT2D_OK;
-}
-
-// Small LaserScan calls (one scan above all), the ranges form of align_batch_fast: initial poses and ranges in one pinned
-// upload, results written by the kernel into mapped pinned memory - three CUDA calls instead of a pipeline.
-static int align_ranges_fast(ndt2d_matcher *m, const void *ranges, int ranges_are_u16, int nscans, int nbeams, double angle_min,
-                             double angle_inc, float range_scale, float range_min, float range_max, const double *init, ndt2d_result *res)
-{
-    int rc = fast_prepare(m);
-    if (rc) return rc;
-    int cap = align_cap_points(m, nbeams);
-    if (cap == 0) return fail(m, NDT2D_EINVAL, "nbeams %d exceeds the shared-memory staging limit", nbeams);
-    if ((rc = ensure_beams(m, nbeams, angle_min, angle_inc))) return rc;
-    const size_t init_bytes = (size_t)nscans * 24, r_bytes = (size_t)nscans * nbeams * (ranges_are_u16 ? 2 : 4);
-    unsigned char *h = m->fast_host;
-    memcpy(h, init, init_bytes);
-    memcpy(h + init_bytes, ranges, r_bytes);
-    unsigned char *d = m->b_fast.as<unsigned char>();
-    CK(m, cudaMemcpyAsync(d, h, init_bytes + r_bytes, cudaMemcpyHostToDevice, m->cfg.stream));
-    AlignArgs a;
-    fill_align_args(m, a);
-    a.xy = nullptr;
-    a.ranges = d + init_bytes;
-    a.beams = m->b_beams.as<float2>();
-    a.ranges_u16 = ranges_are_u16 ? 1 : 0;
-    a.nbeams = nbeams;
-    a.range_scale = range_scale; a.range_min = range_min; a.range_max = range_max;
-    a.init = reinterpret_cast<const double *>(d);
-    a.res = m->fast_res_dev;
-    a.nscans = nscans;
-    a.cap_points = cap;
-    a.counter = m->b_ring.as<unsigned int>() + m->ring_pos++;
-    a.counter_is_zero = 1;
-    CK(m, launch_align(m->cfg, a, &m->launches));
-    rc = ndt2d_synchronize(m);
-    if (rc) return rc;
-    memcpy(res, m->fast_res, (size_t)nscans * sizeof(ndt2d_result));
-    return NDT2D_OK;
+    return align_device(m, a, nbeams, angle_min, angle_inc);
 }
 
 int ndt2d_align_batch_ranges(ndt2d_matcher *m, const void *ranges, int ranges_are_u16, int nscans, int nbeams,
@@ -1029,27 +995,8 @@ int ndt2d_align_batch_ranges(ndt2d_matcher *m, const void *ranges, int ranges_ar
     if (nscans < 0 || nbeams < 1 || (nscans > 0 && (!ranges || !init || !res))) return fail(m, NDT2D_EINVAL, "bad arguments");
     if (nscans == 0) return NDT2D_OK;
     DeviceGuard g(m->device);
-    int rc;
-    const size_t esz = ranges_are_u16 ? 2 : 4;
-    // init at offset 0 (8-byte aligned) and the ranges behind it: nscans * 24 is a multiple of 4, enough for f32 and u16
-    if (nscans <= ndt2d_matcher::FAST_SCANS && (size_t)nscans * 24 + (size_t)nscans * nbeams * esz <= ndt2d_matcher::FAST_BYTES)
-        return align_ranges_fast(m, ranges, ranges_are_u16, nscans, nbeams, angle_min, angle_inc, range_scale, range_min, range_max, init, res);
-    CK(m, m->b_ranges.ensure((size_t)nscans * nbeams * esz));
-    CK(m, m->b_res.ensure((size_t)nscans * sizeof(ndt2d_result)));
-    if ((rc = upload(m, m->b_init, init, (size_t)nscans * 24))) return rc;
-    if ((rc = ensure_beams(m, nbeams, angle_min, angle_inc))) return rc; // on the main stream, before the work streams fork
-    return run_pipeline(
-        m, nscans, (size_t)nscans * nbeams * esz, res,
-        [&](int s0, int s1, void **dst, const void **src, size_t *bytes) {
-            *dst = m->b_ranges.as<unsigned char>() + (size_t)s0 * nbeams * esz;
-            *src = reinterpret_cast<const unsigned char *>(ranges) + (size_t)s0 * nbeams * esz;
-            *bytes = (size_t)(s1 - s0) * nbeams * esz;
-        },
-        [&](int s0, int s1, unsigned int *counter) -> int {
-            return align_ranges_device_impl(m, m->b_ranges.as<unsigned char>() + (size_t)s0 * nbeams * esz, ranges_are_u16,
-                                            s1 - s0, nbeams, angle_min, angle_inc, range_scale, range_min, range_max,
-                                            m->b_init.as<double>() + 3 * (size_t)s0, m->b_res.as<ndt2d_result>() + s0, counter, nscans);
-        });
+    return align_host(m, ranges_input(ranges, ranges_are_u16, nscans, nbeams, range_scale, range_min, range_max), nbeams, init,
+                      res, angle_min, angle_inc);
 }
 
 int ndt2d_sweep_device(ndt2d_matcher *m, int level, const float *d_xy, int n, const float *d_hyp, int64_t nhyp,
@@ -1116,18 +1063,14 @@ int ndt2d_relocalize_device(ndt2d_matcher *m, int level, const float *d_xy, int 
     m->reloc_off[1] = n;
     CK(m, cudaMemcpyAsync(d_off, m->reloc_off, 16, cudaMemcpyHostToDevice, m->cfg.stream));
     CK(m, launch_topk_to_jobs(m->cfg, d_hyp, d_best_idx, k, d_init, d_jobs, &m->launches));
-    AlignArgs a;
-    fill_align_args(m, a);
+    AlignArgs a{};
     a.xy = reinterpret_cast<const float2 *>(d_xy);
-    if (!a.xy) a.xy = m->b_counter.as<float2>();
     a.offsets = d_off;
     a.job_scan = d_jobs;
     a.init = d_init;
     a.res = d_res;
     a.nscans = k;
-    a.cap_points = align_cap_points(m, n);
-    CK(m, launch_align(m->cfg, a, &m->launches));
-    return NDT2D_OK;
+    return align_device(m, a, n);
 }
 
 int ndt2d_relocalize(ndt2d_matcher *m, int level, const float *xy, int n, const float *hyp, int64_t nhyp, int k,

@@ -119,7 +119,6 @@ struct ndt2d_matcher {
     // candidates of a sharded relocalisation (ndt2d_reloc_*)
     ndt2d::PeerTable ex, rx;
     int rx_k = 0;                   // candidates per rank and query in `rx`
-    int chunk_scans = 0; // NDT2D_CHUNK_SCANS override; 0 = choose by bytes (plan_chunks)
     // upload relay (ndt2d_set_upload_relay): a share of the chunks of a host-buffer call travels host -> relay GPU over that
     // GPU's PCIe link, then relay GPU -> this GPU over NVLink
     int relay_dev = -1;
@@ -135,8 +134,7 @@ struct ndt2d_matcher {
     static constexpr int FAST_SCANS = 256, RING = 4096;
     bool fast_ready = false;                 // every allocation of the fast path exists and the ring is zeroed
     unsigned char *fast_host = nullptr;      // pinned + mapped, FAST_BYTES
-    unsigned char *fast_host_dev = nullptr;  // its device address: small xy calls are staged by the kernel from there (NDT2D_FAST_ZEROCOPY=0: copied first)
-    bool fast_zerocopy = true;
+    unsigned char *fast_host_dev = nullptr;  // its device address: small xy calls are staged by the kernel from there
     ndt2d_result *fast_res = nullptr;        // pinned + mapped, FAST_SCANS records
     ndt2d_result *fast_res_dev = nullptr;    // its device address
     ndt2d::DevBuf b_fast, b_ring;
@@ -174,7 +172,11 @@ struct DeviceGuard {
 
 int check_level(ndt2d_matcher *m, int level);
 int upload(ndt2d_matcher *m, DevBuf &b, const void *src, size_t bytes);
-int align_cap_points(const ndt2d_matcher *m, int max_points);
-void fill_align_args(ndt2d_matcher *m, AlignArgs &a);
+// Launches one align. The caller sets the scans' input in `a` and leaves the fields it does not use zero: xy and offsets
+// (points; also job_scan, or pairs and geo), or ranges, ranges_u16, nbeams and the range limits (LaserScan ranges, whose
+// beam table is made from angle_min / angle_inc); then init, res and nscans, and its own work-queue counter and batch_scans
+// where it has them. This fills in the target's levels, the parameters, the shared-memory capacity for scans of up to
+// max_points points and, when counter is unset, the handle's work-queue counter.
+int align_device(ndt2d_matcher *m, AlignArgs a, int max_points, double angle_min = 0.0, double angle_inc = 0.0);
 
 } // namespace ndt2d

@@ -38,7 +38,7 @@ struct AlignArgs {
     ndt2d_params prm;
     const float2 *xy;        // packed scans (xy mode)
     const int64_t *offsets;  // nscans+1 (xy mode)
-    // ranges mode (SPEC 8): xy == nullptr
+    // ranges mode (SPEC 8): ranges != nullptr
     const void *ranges;
     const float2 *beams;     // (cb, sb) per beam
     int ranges_u16, nbeams;

@@ -364,7 +364,7 @@ __device__ __forceinline__ int stage_ranges(const AlignArgs &a, unsigned job, fl
     return kept;
 }
 
-// RANGES: LaserScan input (a.xy == nullptr); warp 0 converts and compacts the beams, the other warps wait at the barrier
+// RANGES: LaserScan input (a.ranges != nullptr); warp 0 converts and compacts the beams, the other warps wait at the barrier
 template <int OV, bool RANGES = false>
 __global__ void __launch_bounds__(BLOCK_ALIGN_THREADS) k_align_block(const __grid_constant__ AlignArgs a)
 {
@@ -720,7 +720,7 @@ cudaError_t launch_align(const LaunchCfg &c, const AlignArgs &a, int64_t *launch
         if (e != cudaSuccess) return e;
     }
     ++*launches;
-    const bool ranges = (a.xy == nullptr);
+    const bool ranges = (a.ranges != nullptr);
     const bool staged = a.cap_points > 0;
     // few scans: latency matters, not throughput - one block per scan (k_align_block) if its factor buffer fits
     // (tools/midsize_probe.py: the block form wins up to ~1250 scans on a 148-SM part, four resident blocks per SM)

@@ -567,7 +567,6 @@ static int align_pairs_impl(ndt2d_matcher *m, const float *d_xy, const int64_t *
             if ((rcu = upload(m, m->b_ppairs, pairs, (size_t)npairs * 8))) return rcu;
             CK(m, cudaStreamSynchronize(m->cfg.stream));     // `pairs` is the caller's buffer
             f.xy = reinterpret_cast<const float2 *>(d_xy);
-            if (!f.xy) f.xy = m->b_counter.as<float2>();
             f.offsets = d_offsets;
             f.pairs = m->b_ppairs.as<int32_t>();
             f.init = d_init;
@@ -637,18 +636,15 @@ static int align_pairs_impl(ndt2d_matcher *m, const float *d_xy, const int64_t *
         b.geo = m->b_pgeo.as<LevelDev>();
         b.error = m->b_perr.as<int>();
         CK(m, launch_pairs_build(m->cfg, b, &m->launches));
-        AlignArgs a;
-        fill_align_args(m, a);
+        AlignArgs a{};
         a.xy = reinterpret_cast<const float2 *>(d_xy);
-        if (!a.xy) a.xy = m->b_counter.as<float2>();
         a.offsets = d_offsets;
         a.pairs = m->b_ppairs.as<int32_t>();
         a.geo = m->b_pgeo.as<LevelDev>();
         a.init = d_init + 3 * (size_t)p0;
         a.res = d_res + p0;
         a.nscans = p1 - p0;
-        a.cap_points = align_cap_points(m, (int)max_src);
-        CK(m, launch_align(m->cfg, a, &m->launches));
+        if ((rc = align_device(m, a, (int)max_src))) return rc;
         for (int32_t t : targets) slot[t] = -1;
         p0 = p1;
     }

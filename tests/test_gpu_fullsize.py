@@ -61,6 +61,22 @@ def test_config2_laserscan_input_equals_point_input(world):
     assert rr.tobytes() == r.tobytes()
 
 
+def test_config2_laserscan_pipeline_over_several_chunks(world):
+    """The batch tiled four times (16 384 scans) crosses the host-buffer pipeline's ~18 MB chunk size: four chunks of f32
+    ranges, two of u16. A result does not depend on its place in the batch, so the results tile too."""
+    m, sc, init = world["m"], world["sc"], world["init"]
+    r = world.get("res")
+    if r is None:
+        r = m.align_batch(world["xy"], world["off"], init)
+    init4 = np.tile(init, (4, 1))
+    rr = m.align_batch_ranges(np.tile(world["ranges"], (4, 1)), sc["angle_min"], sc["angle_inc"], init4, range_scale=1.0)
+    assert rr.tobytes() == np.tile(r, 4).tobytes()
+    u16 = np.round(world["ranges"] / 0.004).clip(0, 65535).astype(np.uint16)
+    one = m.align_batch_ranges(u16, sc["angle_min"], sc["angle_inc"], init, range_scale=0.004)      # a single chunk
+    r4 = m.align_batch_ranges(np.tile(u16, (4, 1)), sc["angle_min"], sc["angle_inc"], init4, range_scale=0.004)
+    assert r4.tobytes() == np.tile(one, 4).tobytes()
+
+
 def test_config2_device_api_equals_host_api(world):
     import torch
     m, B, g = world["m"], world["B"], world["g"]

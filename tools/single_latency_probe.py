@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Host-to-host latency of one align through the host API: packed points (ndt2d_align) and one LaserScan (ndt2d_align_batch_ranges).
-  [NDT2D_FAST_ZEROCOPY=0] python tools/single_latency_probe.py   (GPU box)"""
+  python tools/single_latency_probe.py   (GPU box)"""
 import os, sys, time, json, numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import gtsam_ndt_b200 as g
@@ -20,4 +20,4 @@ for name, fn in (("align_xy", lambda: m.align(one, init[0])), ("align_ranges", l
     for _ in range(200):
         t0 = time.perf_counter(); r = fn(); lat.append((time.perf_counter() - t0) * 1e6)
     out[name] = {"median_us": round(float(np.median(lat)), 1), "min_us": round(min(lat), 1), "iters": int(np.atleast_1d(r)["iterations"][0])}
-print(json.dumps({"NDT2D_FAST_ZEROCOPY": os.environ.get("NDT2D_FAST_ZEROCOPY", "default (1)"), **out}))
+print(json.dumps(out))

@@ -18,6 +18,11 @@ class Params(C.Structure):
                [(n, C.c_int32) for n in ("min_points", "max_iterations", "overlap", "reserved")]
 
 
+class Window(C.Structure):
+    """ndt2d_window (include/ndt2d.h, SPEC.md section 6.1): half-widths and steps of a search window."""
+    _fields_ = [(n, C.c_int32) for n in ("nx", "ny", "nth", "reserved")] + [(n, C.c_double) for n in ("step_x", "step_y", "step_th")]
+
+
 # every symbol include/ndt2d.h declares: name -> (restype, argtypes)
 _V = C.c_void_p
 SIGNATURES = {
@@ -59,6 +64,9 @@ SIGNATURES = {
                                                   C.c_float, C.c_float, _V, _V]),
     "ndt2d_align_pairs": (C.c_int, [_V, _V, _V, C.c_int, _V, C.c_int, _V, _V]),
     "ndt2d_align_pairs_device": (C.c_int, [_V, _V, _V, _V, C.c_int, _V, C.c_int, _V, _V]),
+    "ndt2d_relocalize_pairs": (C.c_int, [_V, C.c_int, _V, _V, C.c_int, _V, C.c_int, _V, C.POINTER(Window), C.c_int, _V, _V, _V]),
+    "ndt2d_relocalize_pairs_device": (C.c_int, [_V, C.c_int, _V, _V, _V, C.c_int, _V, C.c_int, _V, C.POINTER(Window), C.c_int,
+                                                _V, _V, _V]),
     "ndt2d_sweep": (C.c_int, [_V, C.c_int, _V, C.c_int, _V, C.c_int64, _V, C.c_int, _V, _V]),
     "ndt2d_sweep_device": (C.c_int, [_V, C.c_int, _V, C.c_int, _V, C.c_int64, _V, C.c_int, _V, _V]),
     "ndt2d_relocalize": (C.c_int, [_V, C.c_int, _V, C.c_int, _V, C.c_int64, C.c_int, _V, _V]),

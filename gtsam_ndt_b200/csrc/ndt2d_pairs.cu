@@ -391,6 +391,34 @@ __device__ __noinline__ int build_table_shared(const LevelDev *Lp, const float2 
     return nrec;
 }
 
+// SPEC 2 auto-fit: bounding box of the target's finite points, by one warp (every lane gets the result; min and max are
+// order independent). k_pairs_fused keeps its own copy of this loop inline: called from there, the helper changes its code.
+__device__ __forceinline__ void target_bbox(const float2 *__restrict__ tsrc, int tn, int lane, float &xmin, float &ymin, float &xmax,
+                                            float &ymax)
+{
+    for (int base = 0; base < tn; base += 128) {
+        float2 pw[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const int i = base + 32 * u + lane;
+            pw[u] = i < tn ? __ldg(tsrc + i) : make_float2(NAN, NAN);
+        }
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            if (!isfinite(pw[u].x) || !isfinite(pw[u].y)) continue;
+            xmin = fminf(xmin, pw[u].x); xmax = fmaxf(xmax, pw[u].x);
+            ymin = fminf(ymin, pw[u].y); ymax = fmaxf(ymax, pw[u].y);
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        xmin = fminf(xmin, __shfl_xor_sync(FULL_MASK, xmin, o));
+        ymin = fminf(ymin, __shfl_xor_sync(FULL_MASK, ymin, o));
+        xmax = fmaxf(xmax, __shfl_xor_sync(FULL_MASK, xmax, o));
+        ymax = fmaxf(ymax, __shfl_xor_sync(FULL_MASK, ymax, o));
+    }
+}
+
 __global__ void __launch_bounds__(FUSED_WARPS_MAX * 32) k_pairs_fused(const __grid_constant__ PairFusedArgs a)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -525,11 +553,298 @@ cudaError_t launch_pairs_build(const LaunchCfg &c, const PairBuildArgs &a, int64
     return cudaGetLastError();
 }
 
+// ------------------------------------------------------------------------------------------------
+// windowed search over pairs (ndt2d_relocalize_pairs, SPEC 6.1): k_search_sweep scores every window hypothesis of every pair
+// and keeps the k best per (pair, hypothesis chunk); k_search_topk merges a pair's chunks into its exact top-k and turns it
+// into refinement jobs, which k_pairs_fused (shared-memory tables) or k_align in pairs mode (per-target hash tables) align
+// ------------------------------------------------------------------------------------------------
+
+static constexpr int SEARCH_WARPS = 8;
+static constexpr unsigned SEARCH_HEAD_BYTES = 128 + SEARCH_WARPS * 32 * 16;   // LevelDev, then the warps' top-k lists
+static_assert(sizeof(LevelDev) <= 128, "k_search_sweep's head");
+
+struct SearchCand {
+    double score;
+    long long idx;      // -1: no candidate
+};
+
+struct SearchArgs {
+    const float2 *xy;
+    const int64_t *offsets;
+    const int32_t *pairs;    // (target scan, source scan) per pair; with geo: (target slot, source scan)
+    const LevelDev *geo;     // per-target tables (TABLE_GHASH): geo[slot * nlevels + level]
+    const double *centres;   // 3 per pair
+    ndt2d_window win;
+    long long nhyp;          // hypotheses per pair (< 2^31)
+    int npairs, chunks, k, level, nlevels;
+    // TABLE_SHASH: the sweep level's lattice and the layout of the table areas (from pairs_fused_layout)
+    int explicit_grid;
+    float res_m, gox, goy, gex, gey;
+    int min_points;
+    double eig_ratio;
+    unsigned cap_t, hslots, off_r, off_h, off_s;   // byte offsets behind the head: records, bucket index, staged source
+    SearchCand *cand;        // [npairs * chunks * k]
+    unsigned int *counter;   // work queue head, zero on entry
+    int *error;              // set to 1 + pair when a target's lattice would exceed 2^31 cells
+};
+
+// k_argmax_pass's order: (-score, index); an empty candidate (index -1) comes last
+__device__ __forceinline__ bool search_better(double s1, long long i1, double s2, long long i2)
+{
+    if (i2 < 0) return i1 >= 0;
+    if (i1 < 0) return false;
+    return (s1 > s2) || (s1 == s2 && i1 < i2);
+}
+
+// hypothesis j of the window around c (SPEC 6.1): one f64 multiply, one f64 add, one rounding to f32 per coordinate; widened
+// back to f64 as the sweep and the refinement read f32 hypotheses
+__device__ __forceinline__ void window_pose(const double *__restrict__ c, const ndt2d_window &w, long long j, double p[3])
+{
+    const long long nt = 2 * (long long)w.nth + 1, ny = 2 * (long long)w.ny + 1;
+    const long long it = j % nt - w.nth, iy = (j / nt) % ny - w.ny, ix = j / (nt * ny) - w.nx;
+    p[0] = (double)__double2float_rn(__dadd_rn(__ldg(c), __dmul_rn((double)ix, w.step_x)));
+    p[1] = (double)__double2float_rn(__dadd_rn(__ldg(c + 1), __dmul_rn((double)iy, w.step_y)));
+    p[2] = (double)__double2float_rn(__dadd_rn(__ldg(c + 2), __dmul_rn((double)it, w.step_th)));
+}
+
+// running top-k of a warp: lane r < k holds the r-th best candidate so far (sorted, empty entries last)
+__device__ __forceinline__ void topk_insert(double &ms, long long &mi, double s, long long i, int k, int lane)
+{
+    if (s != s || i < 0) return;        // NaN scores are skipped, as by k_argmax_pass
+    const int pos = __popc(__ballot_sync(FULL_MASK, lane < k && search_better(ms, mi, s, i)));
+    const double us = __shfl_up_sync(FULL_MASK, ms, 1);
+    const long long ui = __shfl_up_sync(FULL_MASK, mi, 1);
+    if (pos >= k) return;
+    if (lane > pos) { ms = us; mi = ui; }
+    else if (lane == pos) { ms = s; mi = i; }
+}
+
+// One work item = (pair, chunk of its hypotheses) from the queue. TABLE_SHASH: warp 0 builds the target's grid of the sweep
+// level in shared memory (build_table_shared, as k_pairs_fused) while the other warps stage the source as f64; TABLE_GHASH:
+// the prebuilt per-target table. Each warp then scores its hypotheses with the dense sweep's evaluation (the same bits as
+// ndt2d_sweep on ndt2d_set_target(target scan)), keeps a running top-k, and warp 0 merges the warps' lists into the item's k
+// candidates. STAGED = false: sources too long for shared memory are read from global memory, as by k_eval_poses.
+template <int OV, int TABLE, bool STAGED>
+__global__ void __launch_bounds__(SEARCH_WARPS * 32, 3) k_search_sweep(const __grid_constant__ SearchArgs a)
+{
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    __shared__ unsigned s_item;
+    LevelDev *Ls = reinterpret_cast<LevelDev *>(smem_raw);
+    SearchCand *lists = reinterpret_cast<SearchCand *>(smem_raw + 128);
+    unsigned char *area = smem_raw + SEARCH_HEAD_BYTES;
+    double2 *sp = reinterpret_cast<double2 *>(area + a.off_s);
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const unsigned nitems = (unsigned)a.npairs * (unsigned)a.chunks;
+    for (;;) {
+        __syncthreads();                // the previous item is done with the shared memory
+        if (threadIdx.x == 0) s_item = atomicAdd(a.counter, 1u);
+        __syncthreads();
+        const unsigned item = s_item;
+        if (item >= nitems) break;
+        const int p = (int)(item / (unsigned)a.chunks), c = (int)(item % (unsigned)a.chunks);
+        const int tsel = __ldg(a.pairs + 2 * (size_t)p), sscan = __ldg(a.pairs + 2 * (size_t)p + 1);
+        const int64_t s0 = __ldg(a.offsets + sscan), s1 = __ldg(a.offsets + sscan + 1);
+        const int sn = (int)(s1 - s0);
+        const float2 *__restrict__ ssrc = a.xy + s0;
+        int stager = (int)threadIdx.x, nstagers = (int)blockDim.x;
+        if (TABLE == TABLE_SHASH) {
+            stager -= 32; nstagers -= 32;
+            if (warp == 0) {
+                const int64_t t0 = __ldg(a.offsets + tsel), t1 = __ldg(a.offsets + tsel + 1);
+                const int tn = (int)(t1 - t0);
+                const float2 *__restrict__ tsrc = a.xy + t0;
+                float xmin = INFINITY, ymin = INFINITY, xmax = -INFINITY, ymax = -INFINITY;
+                if (!a.explicit_grid) target_bbox(tsrc, tn, lane, xmin, ymin, xmax, ymax);
+                LevelDev L;
+                const bool usable = pair_level_geometry(L, a.res_m, 0, a.explicit_grid != 0, a.gox, a.goy, a.gex, a.gey, xmin, ymin, xmax, ymax);
+                float *rec = reinterpret_cast<float *>(area + a.off_r);
+                unsigned *hidx = reinterpret_cast<unsigned *>(area + a.off_h);
+                L.cells = reinterpret_cast<const float4 *>(rec);
+                L.cnt = hidx;
+                L.sums = nullptr;
+                L.hash_mask = a.hslots / 4u - 1u;
+                L.zero_rec = 0u;
+                if (!usable && lane == 0) atomicMax(a.error, p + 1);
+                if (lane == 0) *Ls = L;
+                __syncwarp();
+                const int nrec = build_table_shared(Ls, tsrc, tn, a.min_points, a.eig_ratio, reinterpret_cast<unsigned *>(area), a.cap_t,
+                                                    rec, hidx, a.hslots);
+                if (lane == 0) Ls->zero_rec = (unsigned)nrec;
+            }
+        } else if (threadIdx.x == 0) {
+            *Ls = a.geo[(size_t)tsel * a.nlevels + a.level];
+        }
+        if (STAGED && stager >= 0) {    // sanitised points as f64, padded with the far-away point (SPEC 4), as the dense sweep
+            const int npad = (sn + 63) & ~63;
+            for (int i = stager; i < npad; i += nstagers) {
+                const float2 q = i < sn ? sanitize(__ldg(ssrc + i)) : make_float2(1e18f, 1e18f);
+                sp[i] = make_double2((double)q.x, (double)q.y);
+            }
+        }
+        __syncthreads();
+        const long long h0 = (long long)c * a.nhyp / a.chunks, h1 = (long long)(c + 1) * a.nhyp / a.chunks;
+        const double *cp = a.centres + 3 * (size_t)p;
+        double ms = 0.0;
+        long long mi = -1;
+#pragma unroll 1
+        for (long long j = h0 + warp; j < h1; j += SEARCH_WARPS) {
+            double h[3];
+            window_pose(cp, a.win, j, h);
+            const Pose32 q = pose_for_level<true>(h[0], h[1], h[2], *Ls);
+            Eval E;
+            if (STAGED) eval_warp<OV, false, true, false, TABLE, true>(*Ls, reinterpret_cast<const float2 *>(sp), sn, q, lane, E);
+            else eval_warp<OV, false, false, false, TABLE>(*Ls, ssrc, sn, q, lane, E);
+            topk_insert(ms, mi, __shfl_sync(FULL_MASK, E.v[0], 0), j, a.k, lane);
+        }
+        if (lane < a.k) lists[warp * 32 + lane] = SearchCand{ms, mi};
+        __syncthreads();
+        if (warp == 0) {
+#pragma unroll 1
+            for (int w = 1; w < SEARCH_WARPS; ++w)
+#pragma unroll 1
+                for (int r = 0; r < a.k; ++r) {
+                    const SearchCand e = lists[w * 32 + r];
+                    if (e.idx < 0) break;
+                    topk_insert(ms, mi, e.score, e.idx, a.k, lane);
+                }
+            if (lane < a.k) a.cand[(size_t)item * a.k + lane] = SearchCand{ms, mi};
+        }
+    }
+}
+
+// One block per pair: its exact top-k by (-score, index) in k passes of a block-wide arg-max over its chunks' candidates (every
+// member of the pair's top-k is among its own chunk's k best), written to best_idx / best_score as by ndt2d_sweep, and the
+// refinement job of each: the pair's (target, source) and the hypothesis widened to f64, as k_topk_to_jobs does.
+__global__ void __launch_bounds__(256) k_search_topk(const __grid_constant__ SearchArgs a, int64_t *__restrict__ best_idx,
+                                                     double *__restrict__ best_score, int32_t *__restrict__ jobs, double *__restrict__ init)
+{
+    __shared__ double s_val[8];
+    __shared__ long long s_idx[8];
+    const int p = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const SearchCand *__restrict__ cand = a.cand + (size_t)p * a.chunks * a.k;
+    const int n = a.chunks * a.k;
+    double pv = 0.0;
+    long long pi = -1;                  // the previous pass's pick
+    for (int r = 0; r < a.k; ++r) {
+        double bv = 0.0;
+        long long bi = -1;
+        for (int i = threadIdx.x; i < n; i += blockDim.x) {
+            const SearchCand e = cand[i];
+            if ((r == 0 || search_better(pv, pi, e.score, e.idx)) && search_better(e.score, e.idx, bv, bi)) { bv = e.score; bi = e.idx; }
+        }
+        auto warp_best = [&]() {
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+                const double v2 = __shfl_xor_sync(FULL_MASK, bv, o);
+                const long long i2 = __shfl_xor_sync(FULL_MASK, bi, o);
+                if (search_better(v2, i2, bv, bi)) { bv = v2; bi = i2; }
+            }
+        };
+        warp_best();
+        if (lane == 0) { s_val[warp] = bv; s_idx[warp] = bi; }
+        __syncthreads();
+        bv = lane < (int)(blockDim.x >> 5) ? s_val[lane] : 0.0;
+        bi = lane < (int)(blockDim.x >> 5) ? s_idx[lane] : -1;
+        warp_best();                    // every warp reduces the same eight entries: every thread has the pick
+        __syncthreads();
+        const size_t j = (size_t)p * a.k + r;
+        if (threadIdx.x == 0) {
+            best_idx[j] = bi;
+            if (best_score) best_score[j] = bi >= 0 ? bv : 0.0;
+            jobs[2 * j] = __ldg(a.pairs + 2 * (size_t)p);
+            jobs[2 * j + 1] = __ldg(a.pairs + 2 * (size_t)p + 1);
+            double h[3] = {0.0, 0.0, 0.0};
+            if (bi >= 0) window_pose(a.centres + 3 * (size_t)p, a.win, bi, h);
+            init[3 * j] = h[0]; init[3 * j + 1] = h[1]; init[3 * j + 2] = h[2];
+        }
+        pv = bv;
+        pi = bi;
+    }
+}
+
+// the slots without a candidate: the all-zero NO_OVERLAP record ndt2d_relocalize returns for them
+__global__ void k_search_clear(const int64_t *__restrict__ best_idx, int n, ndt2d_result *__restrict__ res)
+{
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n || best_idx[j] >= 0) return;
+    ndt2d_result z;
+    memset(&z, 0, sizeof(z));
+    z.status = NDT2D_NO_OVERLAP;
+    res[j] = z;
+}
+
+// Shared-memory layout of k_search_sweep behind its head: TABLE_SHASH: the build's sort area, records and bucket index as in
+// k_pairs_fused (f.cap_t, f.rmax, f.hslots from pairs_fused_layout), then the source; TABLE_GHASH: the source only. Returns
+// the dynamic shared memory per block; staged = false when the source does not fit (global reads, TABLE_GHASH only).
+size_t search_layout(SearchArgs &s, const PairFusedArgs *f, int64_t max_source_points, int smem_optin, bool &staged)
+{
+    auto up16 = [](size_t v) { return (v + 15) & ~(size_t)15; };
+    size_t off = 0;
+    if (f) {
+        s.cap_t = f->cap_t;
+        s.hslots = f->hslots;
+        s.off_r = (unsigned)up16((size_t)f->cap_t * 4 + 2 * ((size_t)f->cap_t + 2) * 2);
+        s.off_h = (unsigned)(s.off_r + up16(std::max<size_t>(((size_t)f->rmax + 1) * 24, 1024)));
+        off = s.off_h + (size_t)f->hslots * 4;
+    }
+    s.off_s = (unsigned)up16(off);
+    const size_t with_src = SEARCH_HEAD_BYTES + s.off_s + (size_t)((std::max<int64_t>(max_source_points, 1) + 63) & ~(int64_t)63) * 16;
+    staged = with_src <= (size_t)smem_optin - 1024;
+    return staged ? with_src : SEARCH_HEAD_BYTES + s.off_s;
+}
+
+template <int OV, int TABLE, bool STAGED>
+static cudaError_t launch_search_sweep_t(const LaunchCfg &c, const SearchArgs &a, size_t smem)
+{
+    auto kern = k_search_sweep<OV, TABLE, STAGED>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+    if (e != cudaSuccess) return e;
+    int per_sm = 0;
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, SEARCH_WARPS * 32, smem);
+    if (e != cudaSuccess) return e;
+    const int64_t need = (int64_t)a.npairs * a.chunks, cap = (int64_t)c.sm_count * std::max(per_sm, 1);
+    kern<<<(int)std::min(need, cap), SEARCH_WARPS * 32, smem, c.stream>>>(a);
+    return cudaGetLastError();
+}
+
+// Hypothesis chunks per pair: enough work items to keep every SM busy when there are few pairs (two items per resident block),
+// but at least SEARCH_WARPS hypotheses per item, since every item builds (or loads) its target's table and stages its source.
+int search_chunks(const LaunchCfg &c, int npairs, long long nhyp)
+{
+    const long long items = 2ll * c.sm_count * 3;   // k_search_sweep keeps three blocks per SM
+    const long long want = (items + npairs - 1) / npairs, most = (nhyp + SEARCH_WARPS - 1) / SEARCH_WARPS;
+    return (int)std::max(1ll, std::min(want, most));
+}
+
+// sweep (counter zeroed here), top-k and refinement jobs: two launches
+cudaError_t launch_search(const LaunchCfg &c, const SearchArgs &a, bool ov, bool shash, bool staged, size_t smem, int64_t *best_idx,
+                          double *best_score, int32_t *jobs, double *init, int64_t *launches)
+{
+    if (a.npairs <= 0) return cudaSuccess;
+    cudaError_t e = cudaMemsetAsync(a.counter, 0, sizeof(unsigned int), c.stream);
+    if (e != cudaSuccess) return e;
+    if (shash) e = launch_search_sweep_t<0, TABLE_SHASH, true>(c, a, smem);
+    else if (ov) e = staged ? launch_search_sweep_t<1, TABLE_GHASH, true>(c, a, smem) : launch_search_sweep_t<1, TABLE_GHASH, false>(c, a, smem);
+    else e = staged ? launch_search_sweep_t<0, TABLE_GHASH, true>(c, a, smem) : launch_search_sweep_t<0, TABLE_GHASH, false>(c, a, smem);
+    if (e != cudaSuccess) return e;
+    k_search_topk<<<a.npairs, 256, 0, c.stream>>>(a, best_idx, best_score, jobs, init);
+    *launches += 2;
+    return cudaGetLastError();
+}
+
+cudaError_t launch_search_clear(const LaunchCfg &c, const int64_t *best_idx, int n, ndt2d_result *res, int64_t *launches)
+{
+    if (n <= 0) return cudaSuccess;
+    k_search_clear<<<(n + 255) / 256, 256, 0, c.stream>>>(best_idx, n, res);
+    ++*launches;
+    return cudaGetLastError();
+}
+
 } // namespace ndt2d
 
 using namespace ndt2d;
-
-extern "C" {
 
 // ---- batched scan-to-scan (north_star stage 3, "batched multi-scan"): many (target scan, source scan) pairs per call ----
 
@@ -540,50 +855,18 @@ static unsigned next_pow2(unsigned v)
     return p;
 }
 
-// d_xy / d_offsets / d_init / d_res: device; h_offsets / pairs: host (the chunking and the target list are host work).
-// One chunk = as many pairs as fit the table budget. Asynchronous on the handle's stream apart from the uploads of the
-// small per-chunk index lists; *err_out (optional) receives the device error flag after a synchronisation.
-static int align_pairs_impl(ndt2d_matcher *m, const float *d_xy, const int64_t *d_offsets, const int64_t *h_offsets, int nscans,
-                            const int32_t *pairs, int npairs, const double *d_init, ndt2d_result *d_res)
+// General path (overlapping grids, long scans): per-target hash tables in global memory, built by k_pairs_build for chunks of
+// consecutive pairs whose distinct targets fit the table budget (NDT2D_PAIRS_BYTES, default 8 GB). For chunk [p0, p1),
+// run(p0, p1) finds the chunk's pairs as (target slot, source scan) in b_ppairs and the tables' geometry in b_pgeo.
+template <class Run>
+static int pairs_general(ndt2d_matcher *m, const char *name, const float *d_xy, const int64_t *d_offsets, int nscans, const int32_t *pairs,
+                         int npairs, int64_t max_tgt, Run run)
 {
-    int64_t max_src = 0, max_tgt = 0;
-    for (int p = 0; p < npairs; ++p) {
-        const int t = pairs[2 * p], s = pairs[2 * p + 1];
-        if (t < 0 || t >= nscans || s < 0 || s >= nscans) return fail(m, NDT2D_EINVAL, "pair %d: scan index out of range", p);
-        max_tgt = std::max(max_tgt, h_offsets[t + 1] - h_offsets[t]);
-        max_src = std::max(max_src, h_offsets[s + 1] - h_offsets[s]);
-    }
     const int K = m->prm.overlap ? 4 : 1, L = m->nlevels;
-    CK(m, m->b_perr.ensure(4));
-    CK(m, cudaMemsetAsync(m->b_perr.p, 0, 4, m->cfg.stream));
-    // fused path: K = 1 and scans that fit a warp's shared-memory slice (1080-beam scans: 27 KB per warp, 8 warps per SM)
-    {
-        PairFusedArgs f;
-        memset(&f, 0, sizeof(f));
-        f.prm = m->prm;
-        const char *env = getenv("NDT2D_PAIRS_FUSED");
-        if (K == 1 && !(env && atoi(env) == 0) && pairs_fused_layout(f, max_tgt, max_src, m->cfg.max_smem_optin)) {
-            int rcu;
-            if ((rcu = upload(m, m->b_ppairs, pairs, (size_t)npairs * 8))) return rcu;
-            CK(m, cudaStreamSynchronize(m->cfg.stream));     // `pairs` is the caller's buffer
-            f.xy = reinterpret_cast<const float2 *>(d_xy);
-            f.offsets = d_offsets;
-            f.pairs = m->b_ppairs.as<int32_t>();
-            f.init = d_init;
-            f.res = d_res;
-            f.npairs = npairs; f.nlevels = L; f.explicit_grid = m->explicit_grid ? 1 : 0;
-            for (int l = 0; l < L; ++l) f.res_m[l] = m->res[l];
-            f.gox = m->gox; f.goy = m->goy; f.gex = m->gex; f.gey = m->gey;
-            f.counter = m->b_counter.as<unsigned int>();
-            f.error = m->b_perr.as<int>();
-            CK(m, launch_pairs_fused(m->cfg, f, &m->launches));
-            return NDT2D_OK;
-        }
-    }
-    // general path (overlapping grids, long scans): slots per table: 1.5 x the most cells a target can occupy (every point in cells of its own), rounded up to a power
+    // slots per table: 1.5 x the most cells a target can occupy (every point in cells of its own), rounded up to a power
     // of two: at most 2/3 full in that worst case, typically a quarter (a 1080-beam scan occupies ~500 cells)
     const uint64_t want = 3ull * (uint64_t)std::max<int64_t>(max_tgt, 16) * K / 2;
-    if (want > 65536) return fail(m, NDT2D_EINVAL, "align_pairs: target scans of %lld points need more than 65536 table slots",
+    if (want > 65536) return fail(m, NDT2D_EINVAL, "%s: target scans of %lld points need more than 65536 table slots", name,
                                   (long long)max_tgt);
     const unsigned cap = next_pow2((unsigned)want);
     const size_t per_target = (size_t)L * (((size_t)cap + 1) * 32 + (size_t)cap * 44 + sizeof(LevelDev));
@@ -636,6 +919,56 @@ static int align_pairs_impl(ndt2d_matcher *m, const float *d_xy, const int64_t *
         b.geo = m->b_pgeo.as<LevelDev>();
         b.error = m->b_perr.as<int>();
         CK(m, launch_pairs_build(m->cfg, b, &m->launches));
+        if ((rc = run(p0, p1))) return rc;
+        for (int32_t t : targets) slot[t] = -1;
+        p0 = p1;
+    }
+    return NDT2D_OK;
+}
+
+extern "C" {
+
+// d_xy / d_offsets / d_init / d_res: device; h_offsets / pairs: host (the chunking and the target list are host work).
+// One chunk = as many pairs as fit the table budget. Asynchronous on the handle's stream apart from the uploads of the
+// small per-chunk index lists; *err_out (optional) receives the device error flag after a synchronisation.
+static int align_pairs_impl(ndt2d_matcher *m, const float *d_xy, const int64_t *d_offsets, const int64_t *h_offsets, int nscans,
+                            const int32_t *pairs, int npairs, const double *d_init, ndt2d_result *d_res)
+{
+    int64_t max_src = 0, max_tgt = 0;
+    for (int p = 0; p < npairs; ++p) {
+        const int t = pairs[2 * p], s = pairs[2 * p + 1];
+        if (t < 0 || t >= nscans || s < 0 || s >= nscans) return fail(m, NDT2D_EINVAL, "pair %d: scan index out of range", p);
+        max_tgt = std::max(max_tgt, h_offsets[t + 1] - h_offsets[t]);
+        max_src = std::max(max_src, h_offsets[s + 1] - h_offsets[s]);
+    }
+    const int K = m->prm.overlap ? 4 : 1, L = m->nlevels;
+    CK(m, m->b_perr.ensure(4));
+    CK(m, cudaMemsetAsync(m->b_perr.p, 0, 4, m->cfg.stream));
+    // fused path: K = 1 and scans that fit a warp's shared-memory slice (1080-beam scans: 27 KB per warp, 8 warps per SM)
+    {
+        PairFusedArgs f;
+        memset(&f, 0, sizeof(f));
+        f.prm = m->prm;
+        const char *env = getenv("NDT2D_PAIRS_FUSED");
+        if (K == 1 && !(env && atoi(env) == 0) && pairs_fused_layout(f, max_tgt, max_src, m->cfg.max_smem_optin)) {
+            int rcu;
+            if ((rcu = upload(m, m->b_ppairs, pairs, (size_t)npairs * 8))) return rcu;
+            CK(m, cudaStreamSynchronize(m->cfg.stream));     // `pairs` is the caller's buffer
+            f.xy = reinterpret_cast<const float2 *>(d_xy);
+            f.offsets = d_offsets;
+            f.pairs = m->b_ppairs.as<int32_t>();
+            f.init = d_init;
+            f.res = d_res;
+            f.npairs = npairs; f.nlevels = L; f.explicit_grid = m->explicit_grid ? 1 : 0;
+            for (int l = 0; l < L; ++l) f.res_m[l] = m->res[l];
+            f.gox = m->gox; f.goy = m->goy; f.gex = m->gex; f.gey = m->gey;
+            f.counter = m->b_counter.as<unsigned int>();
+            f.error = m->b_perr.as<int>();
+            CK(m, launch_pairs_fused(m->cfg, f, &m->launches));
+            return NDT2D_OK;
+        }
+    }
+    return pairs_general(m, "align_pairs", d_xy, d_offsets, nscans, pairs, npairs, max_tgt, [&](int p0, int p1) {
         AlignArgs a{};
         a.xy = reinterpret_cast<const float2 *>(d_xy);
         a.offsets = d_offsets;
@@ -644,11 +977,8 @@ static int align_pairs_impl(ndt2d_matcher *m, const float *d_xy, const int64_t *
         a.init = d_init + 3 * (size_t)p0;
         a.res = d_res + p0;
         a.nscans = p1 - p0;
-        if ((rc = align_device(m, a, (int)max_src))) return rc;
-        for (int32_t t : targets) slot[t] = -1;
-        p0 = p1;
-    }
-    return NDT2D_OK;
+        return align_device(m, a, (int)max_src);
+    });
 }
 
 static int align_pairs_check(ndt2d_matcher *m)
@@ -706,6 +1036,180 @@ int ndt2d_align_pairs(ndt2d_matcher *m, const float *xy, const int64_t *offsets,
     if (rc) return rc;
     CK(m, cudaMemcpyAsync(res, m->b_res.p, (size_t)npairs * sizeof(ndt2d_result), cudaMemcpyDeviceToHost, m->cfg.stream));
     return align_pairs_check(m);
+}
+
+// ---- windowed search over pairs (SPEC 6.1): ndt2d_set_target(target) + ndt2d_relocalize(source, window) per pair ----
+
+static int relocalize_pairs_validate(ndt2d_matcher *m, int level, const int64_t *offsets, int nscans, const int32_t *pairs, int npairs,
+                                     const ndt2d_window *win, int k, long long *nhyp)
+{
+    int rc = align_pairs_validate(m, offsets, nscans, pairs, npairs);
+    if (rc) return rc;
+    if (level < 0 || level >= m->nlevels) return fail(m, NDT2D_EINVAL, "level %d out of range [0, %d)", level, m->nlevels);
+    if (k < 1 || k > 32) return fail(m, NDT2D_EINVAL, "relocalize_pairs: k %d not in [1, 32]", k);
+    if ((long long)npairs * k >= (1ll << 31)) return fail(m, NDT2D_EINVAL, "relocalize_pairs: npairs * k must be below 2^31");
+    if (!win) return fail(m, NDT2D_EINVAL, "relocalize_pairs: no window");
+    if (win->nx < 0 || win->ny < 0 || win->nth < 0 || win->reserved != 0)
+        return fail(m, NDT2D_EINVAL, "relocalize_pairs: window half-widths (%d, %d, %d) must be >= 0 and reserved 0", win->nx, win->ny, win->nth);
+    if (!isfinite(win->step_x) || !isfinite(win->step_y) || !isfinite(win->step_th))
+        return fail(m, NDT2D_EINVAL, "relocalize_pairs: window steps must be finite");
+    long long h = 2ll * win->nx + 1;
+    for (long long f : {2ll * win->ny + 1, 2ll * win->nth + 1}) {
+        if (h >= (1ll << 31)) break;
+        h *= f;
+    }
+    if (h >= (1ll << 31)) return fail(m, NDT2D_EINVAL, "relocalize_pairs: the window has 2^31 or more hypotheses");
+    *nhyp = h;
+    for (int p = 0; p < npairs; ++p) {
+        const int t = pairs[2 * p], s = pairs[2 * p + 1];
+        if (t < 0 || t >= nscans || s < 0 || s >= nscans) return fail(m, NDT2D_EINVAL, "pair %d: scan index out of range", p);
+    }
+    return NDT2D_OK;
+}
+
+// Shared-memory path (K = 1 and scans that pairs_fused_layout admits, as ndt2d_align_pairs): sweep, top-k, refinement by
+// k_pairs_fused and the empty slots: four launches whatever the number of pairs. General path: per chunk of the per-target
+// tables, the table build, the same sweep and top-k on the tables, k_align in pairs mode and the empty slots.
+static int relocalize_pairs_impl(ndt2d_matcher *m, int level, const float *d_xy, const int64_t *d_offsets, const int64_t *h_offsets,
+                                 int nscans, const int32_t *pairs, int npairs, const double *d_centres, const ndt2d_window &win,
+                                 long long nhyp, int k, int64_t *d_best_idx, double *d_best_score, ndt2d_result *d_res)
+{
+    int64_t max_src = 0, max_tgt = 0;
+    for (int p = 0; p < npairs; ++p) {
+        max_tgt = std::max(max_tgt, h_offsets[pairs[2 * p] + 1] - h_offsets[pairs[2 * p]]);
+        max_src = std::max(max_src, h_offsets[pairs[2 * p + 1] + 1] - h_offsets[pairs[2 * p + 1]]);
+    }
+    const int L = m->nlevels;
+    const size_t njobs = (size_t)npairs * k;
+    CK(m, m->b_perr.ensure(4));
+    CK(m, cudaMemsetAsync(m->b_perr.p, 0, 4, m->cfg.stream));
+    CK(m, m->b_sjobs.ensure(njobs * 8));
+    CK(m, m->b_sinit.ensure(njobs * 24));
+    SearchArgs s;
+    memset(&s, 0, sizeof(s));
+    s.xy = reinterpret_cast<const float2 *>(d_xy);
+    s.offsets = d_offsets;
+    s.win = win;
+    s.nhyp = nhyp;
+    s.k = k; s.level = level; s.nlevels = L;
+    s.counter = m->b_counter.as<unsigned int>();
+    s.error = m->b_perr.as<int>();
+    int32_t *d_jobs = m->b_sjobs.as<int32_t>();
+    double *d_jinit = m->b_sinit.as<double>();
+    auto cand = [&](int pairs_in_call) -> cudaError_t {
+        s.chunks = search_chunks(m->cfg, pairs_in_call, nhyp);
+        cudaError_t e = m->b_scand.ensure((size_t)pairs_in_call * s.chunks * k * sizeof(SearchCand));
+        s.cand = m->b_scand.as<SearchCand>();
+        return e;
+    };
+    PairFusedArgs f;
+    memset(&f, 0, sizeof(f));
+    f.prm = m->prm;
+    const char *env = getenv("NDT2D_PAIRS_FUSED");
+    bool staged = false;
+    size_t smem = 0;
+    if (!m->prm.overlap && !(env && atoi(env) == 0) && pairs_fused_layout(f, max_tgt, max_src, m->cfg.max_smem_optin) &&
+        (smem = search_layout(s, &f, max_src, m->cfg.max_smem_optin, staged), staged)) {
+        int rc;
+        // `pairs` is the caller's buffer: it is uploaded from a copy, so that nothing waits for the copy to finish
+        m->h_spairs.assign(pairs, pairs + 2 * (size_t)npairs);
+        if ((rc = upload(m, m->b_ppairs, m->h_spairs.data(), (size_t)npairs * 8))) return rc;
+        s.pairs = m->b_ppairs.as<int32_t>();
+        s.centres = d_centres;
+        s.npairs = npairs;
+        s.explicit_grid = m->explicit_grid ? 1 : 0;
+        s.res_m = m->res[level];
+        s.gox = m->gox; s.goy = m->goy; s.gex = m->gex; s.gey = m->gey;
+        s.min_points = m->prm.min_points; s.eig_ratio = m->prm.eig_ratio;
+        CK(m, cand(npairs));
+        CK(m, launch_search(m->cfg, s, false, true, true, smem, d_best_idx, d_best_score, d_jobs, d_jinit, &m->launches));
+        f.xy = s.xy;
+        f.offsets = d_offsets;
+        f.pairs = d_jobs;
+        f.init = d_jinit;
+        f.res = d_res;
+        f.npairs = (int)njobs; f.nlevels = L; f.explicit_grid = s.explicit_grid;
+        for (int l = 0; l < L; ++l) f.res_m[l] = m->res[l];
+        f.gox = m->gox; f.goy = m->goy; f.gex = m->gex; f.gey = m->gey;
+        f.counter = s.counter;
+        f.error = s.error;
+        CK(m, launch_pairs_fused(m->cfg, f, &m->launches));
+        CK(m, launch_search_clear(m->cfg, d_best_idx, (int)njobs, d_res, &m->launches));
+        return NDT2D_OK;
+    }
+    memset(&f, 0, sizeof(f));
+    smem = search_layout(s, nullptr, max_src, m->cfg.max_smem_optin, staged);
+    return pairs_general(m, "relocalize_pairs", d_xy, d_offsets, nscans, pairs, npairs, max_tgt, [&](int p0, int p1) -> int {
+        const size_t j0 = (size_t)p0 * k, nj = (size_t)(p1 - p0) * k;
+        s.pairs = m->b_ppairs.as<int32_t>();
+        s.geo = m->b_pgeo.as<LevelDev>();
+        s.centres = d_centres + 3 * (size_t)p0;
+        s.npairs = p1 - p0;
+        CK(m, cand(p1 - p0));
+        CK(m, launch_search(m->cfg, s, m->prm.overlap != 0, false, staged, smem, d_best_idx + j0, d_best_score ? d_best_score + j0 : nullptr,
+                            d_jobs, d_jinit, &m->launches));
+        AlignArgs a{};
+        a.xy = s.xy;
+        a.offsets = d_offsets;
+        a.pairs = d_jobs;
+        a.geo = s.geo;
+        a.init = d_jinit;
+        a.res = d_res + j0;
+        a.nscans = (int)nj;
+        int rc = align_device(m, a, (int)max_src);
+        if (rc) return rc;
+        CK(m, launch_search_clear(m->cfg, d_best_idx + j0, (int)nj, d_res + j0, &m->launches));
+        return NDT2D_OK;
+    });
+}
+
+int ndt2d_relocalize_pairs_device(ndt2d_matcher *m, int level, const float *d_xy, const int64_t *d_offsets, const int64_t *offsets,
+                                  int nscans, const int32_t *pairs, int npairs, const double *d_centres, const ndt2d_window *win, int k,
+                                  int64_t *d_best_idx, double *d_best_score, ndt2d_result *d_res)
+{
+    if (!m) return NDT2D_EINVAL;
+    long long nhyp = 0;
+    int rc = relocalize_pairs_validate(m, level, offsets, nscans, pairs, npairs, win, k, &nhyp);
+    if (rc) return rc;
+    if (npairs == 0) return NDT2D_OK;
+    if (!d_offsets || !d_centres || !d_best_idx || !d_res) return fail(m, NDT2D_EINVAL, "bad arguments");
+    DeviceGuard g(m->device);
+    return relocalize_pairs_impl(m, level, d_xy, d_offsets, offsets, nscans, pairs, npairs, d_centres, *win, nhyp, k, d_best_idx,
+                                 d_best_score, d_res);
+}
+
+int ndt2d_relocalize_pairs(ndt2d_matcher *m, int level, const float *xy, const int64_t *offsets, int nscans, const int32_t *pairs,
+                           int npairs, const double *centres, const ndt2d_window *win, int k, int64_t *best_idx, double *best_score,
+                           ndt2d_result *res)
+{
+    if (!m) return NDT2D_EINVAL;
+    long long nhyp = 0;
+    int rc = relocalize_pairs_validate(m, level, offsets, nscans, pairs, npairs, win, k, &nhyp);
+    if (rc) return rc;
+    if (npairs == 0) return NDT2D_OK;
+    if (!centres || !best_idx || !res) return fail(m, NDT2D_EINVAL, "bad arguments");
+    const int64_t total = offsets[nscans];
+    if (total > 0 && !xy) return fail(m, NDT2D_EINVAL, "bad offsets / xy");
+    DeviceGuard g(m->device);
+    const size_t njobs = (size_t)npairs * k;
+    if ((rc = upload(m, m->b_xy, xy, (size_t)total * 8))) return rc;
+    if ((rc = upload(m, m->b_off, offsets, (size_t)(nscans + 1) * 8))) return rc;
+    if ((rc = upload(m, m->b_init, centres, (size_t)npairs * 24))) return rc;
+    CK(m, m->b_tki.ensure(njobs * 8));
+    CK(m, m->b_tkv.ensure(njobs * 8));
+    CK(m, m->b_res.ensure(njobs * sizeof(ndt2d_result)));
+    rc = relocalize_pairs_impl(m, level, m->b_xy.as<float>(), m->b_off.as<int64_t>(), offsets, nscans, pairs, npairs, m->b_init.as<double>(),
+                               *win, nhyp, k, m->b_tki.as<int64_t>(), m->b_tkv.as<double>(), m->b_res.as<ndt2d_result>());
+    if (rc) return rc;
+    CK(m, cudaMemcpyAsync(best_idx, m->b_tki.p, njobs * 8, cudaMemcpyDeviceToHost, m->cfg.stream));
+    if (best_score) CK(m, cudaMemcpyAsync(best_score, m->b_tkv.p, njobs * 8, cudaMemcpyDeviceToHost, m->cfg.stream));
+    CK(m, cudaMemcpyAsync(res, m->b_res.p, njobs * sizeof(ndt2d_result), cudaMemcpyDeviceToHost, m->cfg.stream));
+    int err = 0;
+    CK(m, cudaMemcpyAsync(&err, m->b_perr.p, 4, cudaMemcpyDeviceToHost, m->cfg.stream));
+    if ((rc = ndt2d_synchronize(m))) return rc;     // the one synchronisation of the call (shared-memory path)
+    if (err) return fail(m, NDT2D_EINVAL, "relocalize_pairs: the auto-fitted lattice of a target scan exceeds 2^31 cells "
+                                          "(a point far from the rest?); its pairs were returned with status NO_OVERLAP");
+    return NDT2D_OK;
 }
 
 } // extern "C"

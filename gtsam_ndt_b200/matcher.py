@@ -54,6 +54,27 @@ def pinned_array(shape, dtype, write_combined=False):
     return np.frombuffer(buf, dtype=dt, count=int(np.prod(shape))).reshape(shape)
 
 
+def _window(window):
+    """A search window as ndt2d_window: a _lib.Window, or (nx, ny, nth, step_x, step_y, step_th)."""
+    if isinstance(window, _lib.Window):
+        return window
+    nx, ny, nth, sx, sy, st = window
+    return _lib.Window(int(nx), int(ny), int(nth), 0, float(sx), float(sy), float(st))
+
+
+def window_hypotheses(centre, window):
+    """The hypotheses of a search window around centre, as ndt2d_relocalize_pairs sweeps them (SPEC.md section 6.1):
+    f32 (H, 3), index j = ((ix + nx)(2ny + 1) + (iy + ny))(2nth + 1) + (it + nth), value (float)(c + (double)i * step)."""
+    w = _window(window)
+    if min(w.nx, w.ny, w.nth) < 0:
+        raise ValueError("window half-widths must be >= 0")
+    c = np.asarray(centre, np.float64).reshape(3)
+    ix, iy, it = np.meshgrid(np.arange(-w.nx, w.nx + 1, dtype=np.float64), np.arange(-w.ny, w.ny + 1, dtype=np.float64),
+                             np.arange(-w.nth, w.nth + 1, dtype=np.float64), indexing="ij")
+    # numpy evaluates each f64 product and sum on its own (no fused multiply-add), then rounds once to f32
+    return np.stack([c[0] + ix * w.step_x, c[1] + iy * w.step_y, c[2] + it * w.step_th], -1).reshape(-1, 3).astype(np.float32)
+
+
 class NdtMatcher2D:
     """One handle = one CUDA device + one stream (not thread-safe)."""
 
@@ -297,6 +318,38 @@ class NdtMatcher2D:
         pairs = np.ascontiguousarray(pairs, np.int32).reshape(-1, 2)
         self._ck(self._L.ndt2d_align_pairs_device(self._h, _ptr(d_xy), _ptr(d_offsets), _ptr(offsets), len(offsets) - 1, _ptr(pairs),
                                                   len(pairs), _ptr(d_init), _ptr(d_res)))
+
+    def relocalize_pairs(self, xy, offsets, pairs, centres, window, k=4, level=0):
+        """Windowed search over scan pairs (loop-closure candidates): for pairs[p] = (target scan, source scan), sweep the window
+        hypotheses around centres[p] on `level`, keep the k best by (-score, index) and align the source from each of them.
+        Equals set_target(target) + relocalize(source, window_hypotheses(centres[p], window), k, level) for every pair.
+        Returns (best_idx[npairs, k], best_score[npairs, k], res[npairs, k]); an empty slot has index -1."""
+        xy = np.ascontiguousarray(xy, np.float32).reshape(-1, 2)
+        offsets = np.ascontiguousarray(offsets, np.int64)
+        pairs = np.ascontiguousarray(pairs, np.int32).reshape(-1, 2)
+        centres = np.ascontiguousarray(centres, np.float64).reshape(-1, 3)
+        nb = len(offsets) - 1
+        if nb < 0 or len(centres) != len(pairs) or (nb and (offsets[0] < 0 or offsets[-1] > len(xy))):
+            raise ValueError("offsets / pairs / centres / xy sizes disagree")
+        kk = max(int(k), 0)
+        bi = np.full((len(pairs), kk), -1, np.int64)
+        bs = np.zeros((len(pairs), kk), np.float64)
+        res = np.zeros((len(pairs), kk), RESULT_DTYPE)
+        w = _window(window)
+        self._ck(self._L.ndt2d_relocalize_pairs(self._h, level, _ptr(xy), _ptr(offsets), nb, _ptr(pairs), len(pairs), _ptr(centres),
+                                                C.byref(w), int(k), _ptr(bi), _ptr(bs), _ptr(res)))
+        return bi, bs, res
+
+    def relocalize_pairs_device(self, d_xy, d_offsets, offsets, pairs, d_centres, window, k, d_best_idx, d_best_score, d_res,
+                                level=0):
+        """Device-resident scans / centres / outputs ([npairs * k] each; d_best_score may be None); offsets (host copy) and
+        pairs on the host. Asynchronous on the handle's stream."""
+        offsets = np.ascontiguousarray(offsets, np.int64)
+        pairs = np.ascontiguousarray(pairs, np.int32).reshape(-1, 2)
+        w = _window(window)
+        self._ck(self._L.ndt2d_relocalize_pairs_device(self._h, level, _ptr(d_xy), _ptr(d_offsets), _ptr(offsets), len(offsets) - 1,
+                                                       _ptr(pairs), len(pairs), _ptr(d_centres), C.byref(w), int(k), _ptr(d_best_idx),
+                                                       _ptr(d_best_score), _ptr(d_res)))
 
     # ---- multi-GPU sweep: best-hypothesis exchange over peer memory (one process per GPU) ----
     def exchange_create(self, world, rank, nslots=64):

@@ -180,6 +180,30 @@ int ndt2d_align_pairs(ndt2d_matcher *m, const float *xy, const int64_t *offsets,
 int ndt2d_align_pairs_device(ndt2d_matcher *m, const float *d_xy, const int64_t *d_offsets, const int64_t *offsets,
                              int nscans, const int32_t *pairs, int npairs, const double *d_init, ndt2d_result *d_res);
 
+/* ---- windowed search over scan pairs (loop-closure candidates, SPEC 6.1) ----
+ * A search window is H = (2nx+1)(2ny+1)(2nth+1) hypotheses around a centre pose c: hypothesis
+ * j = ((ix+nx)(2ny+1) + (iy+ny))(2nth+1) + (it+nth) is ((float)(c0 + ix*step_x), (float)(c1 + iy*step_y),
+ * (float)(c2 + it*step_th)) in f64 without contraction, theta not wrapped. nx, ny, nth >= 0, steps finite, reserved = 0,
+ * H < 2^31. */
+typedef struct ndt2d_window {
+    int32_t nx, ny, nth, reserved;
+    double step_x, step_y, step_th;
+} ndt2d_window;
+/* Scans packed as for ndt2d_align_pairs. Pair p = (target scan pairs[2p], source scan pairs[2p+1]) with centre
+ * centres[3p..]: best_idx[p*k..], best_score[p*k..] and res[p*k..] equal, bit for bit, ndt2d_set_target(target scan) followed
+ * by ndt2d_relocalize(level, source scan, the window's hypotheses around the centre, k) (best_score: ndt2d_sweep's top-k
+ * scores). A slot without a candidate (H < k) has index -1, score 0 and an all-zero record with status NDT2D_NO_OVERLAP.
+ * 1 <= k <= 32; best_score may be NULL. Needs ndt2d_set_resolution(s) only; the handle's own target is not touched. */
+int ndt2d_relocalize_pairs(ndt2d_matcher *m, int level, const float *xy, const int64_t *offsets, int nscans,
+                           const int32_t *pairs, int npairs, const double *centres, const ndt2d_window *win, int k,
+                           int64_t *best_idx, double *best_score, ndt2d_result *res);
+/* scans, centres and outputs on the device; offsets (also given on the host), pairs and the window on the host, as for
+ * ndt2d_align_pairs_device. Asynchronous on the handle's stream. */
+int ndt2d_relocalize_pairs_device(ndt2d_matcher *m, int level, const float *d_xy, const int64_t *d_offsets,
+                                  const int64_t *offsets, int nscans, const int32_t *pairs, int npairs,
+                                  const double *d_centres, const ndt2d_window *win, int k, int64_t *d_best_idx,
+                                  double *d_best_score, ndt2d_result *d_res);
+
 /* ---- sweep (kernel stage 3: multi-hypothesis search for relocalisation / loop closure, SPEC 6) - */
 /* hyp[3*j..] = (tx, ty, theta) f32. scores (optional, nhyp doubles). Top-k (k >= 1) by
  * (-score, index) into best_idx[k], best_score[k]. */

@@ -151,6 +151,31 @@ class Matcher {
         return out;
     }
 
+    // windowed search over scan pairs (loop-closure candidates): for every pair, the window's hypotheses around centres[p] are
+    // swept on `level`, the k best refined; equals setTarget(target) + relocalize(source, window hypotheses, k, level) per pair.
+    // Returns npairs * k records, pair-major; indices / scores (optional) receive the k sweep indices and scores per pair
+    // (index -1: no candidate).
+    std::vector<Result> relocalizePairs(const std::vector<Point2f> &points, const std::vector<std::int64_t> &offsets,
+                                        const std::vector<std::pair<std::int32_t, std::int32_t>> &pairs, const std::vector<Pose2d> &centres,
+                                        const ndt2d_window &window, int k, int level = 0, std::vector<std::int64_t> *indices = nullptr,
+                                        std::vector<double> *scores = nullptr)
+    {
+        if (pairs.size() != centres.size()) throw std::invalid_argument("relocalizePairs: one centre per pair");
+        if (offsets.empty()) throw std::invalid_argument("relocalizePairs: offsets must have nscans + 1 entries");
+        if (offsets.front() < 0 || static_cast<size_t>(offsets.back()) > points.size()) throw std::invalid_argument("relocalizePairs: offsets overrun points");
+        if (k < 1) throw std::invalid_argument("relocalizePairs: k >= 1");
+        const size_t n = pairs.size() * static_cast<size_t>(k);
+        std::vector<Result> out(n);
+        std::vector<std::int64_t> idx(n, -1);
+        std::vector<double> val(n, 0.0);
+        ck(ndt2d_relocalize_pairs(h_, level, reinterpret_cast<const float *>(points.data()), offsets.data(), static_cast<int>(offsets.size() - 1),
+                                  reinterpret_cast<const std::int32_t *>(pairs.data()), static_cast<int>(pairs.size()),
+                                  reinterpret_cast<const double *>(centres.data()), &window, k, idx.data(), val.data(), out.data()));
+        if (indices) *indices = std::move(idx);
+        if (scores) *scores = std::move(val);
+        return out;
+    }
+
     // ---- multi-hypothesis search (relocalisation, loop-closure candidates) --------------------------
     // hypotheses: (x, y, theta) float triples. Returns the k best (index, score), best first.
     std::vector<std::pair<std::int64_t, double>> sweep(const std::vector<Point2f> &scan, const std::vector<float> &hyp_xyt, int k,

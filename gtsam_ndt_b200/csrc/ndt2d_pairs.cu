@@ -556,7 +556,9 @@ cudaError_t launch_pairs_build(const LaunchCfg &c, const PairBuildArgs &a, int64
 // ------------------------------------------------------------------------------------------------
 // windowed search over pairs (ndt2d_relocalize_pairs, SPEC 6.1): k_search_sweep scores every window hypothesis of every pair
 // and keeps the k best per (pair, hypothesis chunk); k_search_topk merges a pair's chunks into its exact top-k and turns it
-// into refinement jobs, which k_pairs_fused (shared-memory tables) or k_align in pairs mode (per-target hash tables) align
+// into refinement jobs, which k_pairs_fused (shared-memory tables) or k_align in pairs mode (per-target hash tables) align.
+// The same two kernels search a batch of scans against the handle's dense target (ndt2d_relocalize_batch, SPEC 6.2), whose
+// jobs k_align_block or k_align refine in job_scan mode.
 // ------------------------------------------------------------------------------------------------
 
 static constexpr int SEARCH_WARPS = 8;
@@ -568,11 +570,13 @@ struct SearchCand {
     long long idx;      // -1: no candidate
 };
 
+// A work item p is a pair (ndt2d_relocalize_pairs) or, with TABLE_DENSE, scan p of the batch against the handle's target
+// (ndt2d_relocalize_batch); npairs then counts scans and pairs is unused.
 struct SearchArgs {
     const float2 *xy;
     const int64_t *offsets;
     const int32_t *pairs;    // (target scan, source scan) per pair; with geo: (target slot, source scan)
-    const LevelDev *geo;     // per-target tables (TABLE_GHASH): geo[slot * nlevels + level]
+    const LevelDev *geo;     // per-target tables (TABLE_GHASH): geo[slot * nlevels + level]; TABLE_DENSE: the handle's levels
     const double *centres;   // 3 per pair
     ndt2d_window win;
     long long nhyp;          // hypotheses per pair (< 2^31)
@@ -623,7 +627,9 @@ __device__ __forceinline__ void topk_insert(double &ms, long long &mi, double s,
 // level in shared memory (build_table_shared, as k_pairs_fused) while the other warps stage the source as f64; TABLE_GHASH:
 // the prebuilt per-target table. Each warp then scores its hypotheses with the dense sweep's evaluation (the same bits as
 // ndt2d_sweep on ndt2d_set_target(target scan)), keeps a running top-k, and warp 0 merges the warps' lists into the item's k
-// candidates. STAGED = false: sources too long for shared memory are read from global memory, as by k_eval_poses.
+// candidates. TABLE_DENSE: item p is scan p of the batch swept over the handle's dense table geo[level] (ndt2d_relocalize_batch;
+// every warp stages, the same eval_warp instantiation as k_eval_poses, so the scores are ndt2d_sweep's on that target).
+// STAGED = false: sources too long for shared memory are read from global memory, as by k_eval_poses.
 template <int OV, int TABLE, bool STAGED>
 __global__ void __launch_bounds__(SEARCH_WARPS * 32, 3) k_search_sweep(const __grid_constant__ SearchArgs a)
 {
@@ -642,7 +648,8 @@ __global__ void __launch_bounds__(SEARCH_WARPS * 32, 3) k_search_sweep(const __g
         const unsigned item = s_item;
         if (item >= nitems) break;
         const int p = (int)(item / (unsigned)a.chunks), c = (int)(item % (unsigned)a.chunks);
-        const int tsel = __ldg(a.pairs + 2 * (size_t)p), sscan = __ldg(a.pairs + 2 * (size_t)p + 1);
+        const int tsel = TABLE == TABLE_DENSE ? 0 : __ldg(a.pairs + 2 * (size_t)p);
+        const int sscan = TABLE == TABLE_DENSE ? p : __ldg(a.pairs + 2 * (size_t)p + 1);
         const int64_t s0 = __ldg(a.offsets + sscan), s1 = __ldg(a.offsets + sscan + 1);
         const int sn = (int)(s1 - s0);
         const float2 *__restrict__ ssrc = a.xy + s0;
@@ -714,7 +721,9 @@ __global__ void __launch_bounds__(SEARCH_WARPS * 32, 3) k_search_sweep(const __g
 
 // One block per pair: its exact top-k by (-score, index) in k passes of a block-wide arg-max over its chunks' candidates (every
 // member of the pair's top-k is among its own chunk's k best), written to best_idx / best_score as by ndt2d_sweep, and the
-// refinement job of each: the pair's (target, source) and the hypothesis widened to f64, as k_topk_to_jobs does.
+// refinement job of each: the pair's (target, source) and the hypothesis widened to f64, as k_topk_to_jobs does. SCAN_JOBS
+// (batch against the handle's target): the job is AlignArgs::job_scan[j] = p, or -1 for an empty slot (no LM work).
+template <bool SCAN_JOBS>
 __global__ void __launch_bounds__(256) k_search_topk(const __grid_constant__ SearchArgs a, int64_t *__restrict__ best_idx,
                                                      double *__restrict__ best_score, int32_t *__restrict__ jobs, double *__restrict__ init)
 {
@@ -751,8 +760,12 @@ __global__ void __launch_bounds__(256) k_search_topk(const __grid_constant__ Sea
         if (threadIdx.x == 0) {
             best_idx[j] = bi;
             if (best_score) best_score[j] = bi >= 0 ? bv : 0.0;
-            jobs[2 * j] = __ldg(a.pairs + 2 * (size_t)p);
-            jobs[2 * j + 1] = __ldg(a.pairs + 2 * (size_t)p + 1);
+            if (SCAN_JOBS) {
+                jobs[j] = bi >= 0 ? p : -1;
+            } else {
+                jobs[2 * j] = __ldg(a.pairs + 2 * (size_t)p);
+                jobs[2 * j + 1] = __ldg(a.pairs + 2 * (size_t)p + 1);
+            }
             double h[3] = {0.0, 0.0, 0.0};
             if (bi >= 0) window_pose(a.centres + 3 * (size_t)p, a.win, bi, h);
             init[3 * j] = h[0]; init[3 * j + 1] = h[1]; init[3 * j + 2] = h[2];
@@ -818,18 +831,24 @@ int search_chunks(const LaunchCfg &c, int npairs, long long nhyp)
     return (int)std::max(1ll, std::min(want, most));
 }
 
-// sweep (counter zeroed here), top-k and refinement jobs: two launches
-cudaError_t launch_search(const LaunchCfg &c, const SearchArgs &a, bool ov, bool shash, bool staged, size_t smem, int64_t *best_idx,
+// sweep (counter zeroed here), top-k and refinement jobs: two launches. table: TABLE_SHASH or TABLE_GHASH (pairs, jobs as
+// pairs) or TABLE_DENSE (a batch against the handle's target, jobs as job_scan)
+cudaError_t launch_search(const LaunchCfg &c, const SearchArgs &a, bool ov, int table, bool staged, size_t smem, int64_t *best_idx,
                           double *best_score, int32_t *jobs, double *init, int64_t *launches)
 {
     if (a.npairs <= 0) return cudaSuccess;
     cudaError_t e = cudaMemsetAsync(a.counter, 0, sizeof(unsigned int), c.stream);
     if (e != cudaSuccess) return e;
-    if (shash) e = launch_search_sweep_t<0, TABLE_SHASH, true>(c, a, smem);
+    if (table == TABLE_SHASH) e = launch_search_sweep_t<0, TABLE_SHASH, true>(c, a, smem);
+    else if (table == TABLE_DENSE && ov)
+        e = staged ? launch_search_sweep_t<1, TABLE_DENSE, true>(c, a, smem) : launch_search_sweep_t<1, TABLE_DENSE, false>(c, a, smem);
+    else if (table == TABLE_DENSE)
+        e = staged ? launch_search_sweep_t<0, TABLE_DENSE, true>(c, a, smem) : launch_search_sweep_t<0, TABLE_DENSE, false>(c, a, smem);
     else if (ov) e = staged ? launch_search_sweep_t<1, TABLE_GHASH, true>(c, a, smem) : launch_search_sweep_t<1, TABLE_GHASH, false>(c, a, smem);
     else e = staged ? launch_search_sweep_t<0, TABLE_GHASH, true>(c, a, smem) : launch_search_sweep_t<0, TABLE_GHASH, false>(c, a, smem);
     if (e != cudaSuccess) return e;
-    k_search_topk<<<a.npairs, 256, 0, c.stream>>>(a, best_idx, best_score, jobs, init);
+    if (table == TABLE_DENSE) k_search_topk<true><<<a.npairs, 256, 0, c.stream>>>(a, best_idx, best_score, jobs, init);
+    else k_search_topk<false><<<a.npairs, 256, 0, c.stream>>>(a, best_idx, best_score, jobs, init);
     *launches += 2;
     return cudaGetLastError();
 }
@@ -1040,26 +1059,34 @@ int ndt2d_align_pairs(ndt2d_matcher *m, const float *xy, const int64_t *offsets,
 
 // ---- windowed search over pairs (SPEC 6.1): ndt2d_set_target(target) + ndt2d_relocalize(source, window) per pair ----
 
+// k, the output size and the window (SPEC 6.1) of a windowed search over `count` items (`what`: "npairs" or "nscans"); *nhyp = H
+static int search_validate(ndt2d_matcher *m, const char *name, const char *what, int count, const ndt2d_window *win, int k,
+                           long long *nhyp)
+{
+    if (k < 1 || k > 32) return fail(m, NDT2D_EINVAL, "%s: k %d not in [1, 32]", name, k);
+    if ((long long)count * k >= (1ll << 31)) return fail(m, NDT2D_EINVAL, "%s: %s * k must be below 2^31", name, what);
+    if (!win) return fail(m, NDT2D_EINVAL, "%s: no window", name);
+    if (win->nx < 0 || win->ny < 0 || win->nth < 0 || win->reserved != 0)
+        return fail(m, NDT2D_EINVAL, "%s: window half-widths (%d, %d, %d) must be >= 0 and reserved 0", name, win->nx, win->ny, win->nth);
+    if (!isfinite(win->step_x) || !isfinite(win->step_y) || !isfinite(win->step_th))
+        return fail(m, NDT2D_EINVAL, "%s: window steps must be finite", name);
+    long long h = 2ll * win->nx + 1;
+    for (long long f : {2ll * win->ny + 1, 2ll * win->nth + 1}) {
+        if (h >= (1ll << 31)) break;
+        h *= f;
+    }
+    if (h >= (1ll << 31)) return fail(m, NDT2D_EINVAL, "%s: the window has 2^31 or more hypotheses", name);
+    *nhyp = h;
+    return NDT2D_OK;
+}
+
 static int relocalize_pairs_validate(ndt2d_matcher *m, int level, const int64_t *offsets, int nscans, const int32_t *pairs, int npairs,
                                      const ndt2d_window *win, int k, long long *nhyp)
 {
     int rc = align_pairs_validate(m, offsets, nscans, pairs, npairs);
     if (rc) return rc;
     if (level < 0 || level >= m->nlevels) return fail(m, NDT2D_EINVAL, "level %d out of range [0, %d)", level, m->nlevels);
-    if (k < 1 || k > 32) return fail(m, NDT2D_EINVAL, "relocalize_pairs: k %d not in [1, 32]", k);
-    if ((long long)npairs * k >= (1ll << 31)) return fail(m, NDT2D_EINVAL, "relocalize_pairs: npairs * k must be below 2^31");
-    if (!win) return fail(m, NDT2D_EINVAL, "relocalize_pairs: no window");
-    if (win->nx < 0 || win->ny < 0 || win->nth < 0 || win->reserved != 0)
-        return fail(m, NDT2D_EINVAL, "relocalize_pairs: window half-widths (%d, %d, %d) must be >= 0 and reserved 0", win->nx, win->ny, win->nth);
-    if (!isfinite(win->step_x) || !isfinite(win->step_y) || !isfinite(win->step_th))
-        return fail(m, NDT2D_EINVAL, "relocalize_pairs: window steps must be finite");
-    long long h = 2ll * win->nx + 1;
-    for (long long f : {2ll * win->ny + 1, 2ll * win->nth + 1}) {
-        if (h >= (1ll << 31)) break;
-        h *= f;
-    }
-    if (h >= (1ll << 31)) return fail(m, NDT2D_EINVAL, "relocalize_pairs: the window has 2^31 or more hypotheses");
-    *nhyp = h;
+    if ((rc = search_validate(m, "relocalize_pairs", "npairs", npairs, win, k, nhyp))) return rc;
     for (int p = 0; p < npairs; ++p) {
         const int t = pairs[2 * p], s = pairs[2 * p + 1];
         if (t < 0 || t >= nscans || s < 0 || s >= nscans) return fail(m, NDT2D_EINVAL, "pair %d: scan index out of range", p);
@@ -1122,7 +1149,7 @@ static int relocalize_pairs_impl(ndt2d_matcher *m, int level, const float *d_xy,
         s.gox = m->gox; s.goy = m->goy; s.gex = m->gex; s.gey = m->gey;
         s.min_points = m->prm.min_points; s.eig_ratio = m->prm.eig_ratio;
         CK(m, cand(npairs));
-        CK(m, launch_search(m->cfg, s, false, true, true, smem, d_best_idx, d_best_score, d_jobs, d_jinit, &m->launches));
+        CK(m, launch_search(m->cfg, s, false, TABLE_SHASH, true, smem, d_best_idx, d_best_score, d_jobs, d_jinit, &m->launches));
         f.xy = s.xy;
         f.offsets = d_offsets;
         f.pairs = d_jobs;
@@ -1146,7 +1173,7 @@ static int relocalize_pairs_impl(ndt2d_matcher *m, int level, const float *d_xy,
         s.centres = d_centres + 3 * (size_t)p0;
         s.npairs = p1 - p0;
         CK(m, cand(p1 - p0));
-        CK(m, launch_search(m->cfg, s, m->prm.overlap != 0, false, staged, smem, d_best_idx + j0, d_best_score ? d_best_score + j0 : nullptr,
+        CK(m, launch_search(m->cfg, s, m->prm.overlap != 0, TABLE_GHASH, staged, smem, d_best_idx + j0, d_best_score ? d_best_score + j0 : nullptr,
                             d_jobs, d_jinit, &m->launches));
         AlignArgs a{};
         a.xy = s.xy;
@@ -1210,6 +1237,102 @@ int ndt2d_relocalize_pairs(ndt2d_matcher *m, int level, const float *xy, const i
     if (err) return fail(m, NDT2D_EINVAL, "relocalize_pairs: the auto-fitted lattice of a target scan exceeds 2^31 cells "
                                           "(a point far from the rest?); its pairs were returned with status NO_OVERLAP");
     return NDT2D_OK;
+}
+
+// ---- windowed search of a batch of scans against the handle's target (SPEC 6.2): ndt2d_relocalize(scan, window) per scan ----
+
+// Sweep of every scan over its window on the dense table of `level`, top-k, refinement of the nscans * k jobs by align_device
+// (k_align_block or k_align, job_scan mode) and the empty slots: four launches whatever the number of scans.
+static int relocalize_batch_impl(ndt2d_matcher *m, int level, const float *d_xy, const int64_t *d_offsets, int nscans, int max_points,
+                                 const double *d_centres, const ndt2d_window &win, long long nhyp, int k, int64_t *d_best_idx,
+                                 double *d_best_score, ndt2d_result *d_res)
+{
+    const size_t njobs = (size_t)nscans * k;
+    CK(m, m->b_sjobs.ensure(njobs * 4));
+    CK(m, m->b_sinit.ensure(njobs * 24));
+    // the sweep reads the level from the device (SearchArgs::geo); the copy is taken now, so a later set_target cannot reach it
+    int rc = upload(m, m->b_slevels, m->lv, (size_t)m->nlevels * sizeof(LevelDev));
+    if (rc) return rc;
+    SearchArgs s;
+    memset(&s, 0, sizeof(s));
+    s.xy = reinterpret_cast<const float2 *>(d_xy);
+    s.offsets = d_offsets;
+    s.geo = m->b_slevels.as<LevelDev>();
+    s.centres = d_centres;
+    s.win = win;
+    s.nhyp = nhyp;
+    s.npairs = nscans;
+    s.k = k; s.level = level; s.nlevels = m->nlevels;
+    s.counter = m->b_counter.as<unsigned int>();
+    // every item stages only its scan (no table build), so the chunking is the pairs' one without a table to amortise
+    s.chunks = search_chunks(m->cfg, nscans, nhyp);
+    CK(m, m->b_scand.ensure((size_t)nscans * s.chunks * k * sizeof(SearchCand)));
+    s.cand = m->b_scand.as<SearchCand>();
+    bool staged = false;
+    const size_t smem = search_layout(s, nullptr, max_points, m->cfg.max_smem_optin, staged);
+    int32_t *d_jobs = m->b_sjobs.as<int32_t>();
+    double *d_jinit = m->b_sinit.as<double>();
+    CK(m, launch_search(m->cfg, s, m->prm.overlap != 0, TABLE_DENSE, staged, smem, d_best_idx, d_best_score, d_jobs, d_jinit, &m->launches));
+    AlignArgs a{};
+    a.xy = s.xy;
+    a.offsets = d_offsets;
+    a.job_scan = d_jobs;
+    a.init = d_jinit;
+    a.res = d_res;
+    a.nscans = (int)njobs;
+    if ((rc = align_device(m, a, max_points))) return rc;
+    CK(m, launch_search_clear(m->cfg, d_best_idx, (int)njobs, d_res, &m->launches));
+    return NDT2D_OK;
+}
+
+int ndt2d_relocalize_batch_device(ndt2d_matcher *m, int level, const float *d_xy, const int64_t *d_offsets, int nscans, int max_points,
+                                  const double *d_centres, const ndt2d_window *win, int k, int64_t *d_best_idx, double *d_best_score,
+                                  ndt2d_result *d_res)
+{
+    int rc = check_level(m, level);
+    if (rc) return rc;
+    long long nhyp = 0;
+    if ((rc = search_validate(m, "relocalize_batch", "nscans", nscans, win, k, &nhyp))) return rc;
+    if (nscans < 0 || max_points < 0 || (nscans > 0 && (!d_offsets || !d_centres || !d_best_idx || !d_res)))
+        return fail(m, NDT2D_EINVAL, "relocalize_batch: bad arguments");
+    if (nscans == 0) return NDT2D_OK;
+    DeviceGuard g(m->device);
+    return relocalize_batch_impl(m, level, d_xy, d_offsets, nscans, max_points, d_centres, *win, nhyp, k, d_best_idx, d_best_score, d_res);
+}
+
+int ndt2d_relocalize_batch(ndt2d_matcher *m, int level, const float *xy, const int64_t *offsets, int nscans, const double *centres,
+                           const ndt2d_window *win, int k, int64_t *best_idx, double *best_score, ndt2d_result *res)
+{
+    int rc = check_level(m, level);
+    if (rc) return rc;
+    long long nhyp = 0;
+    if ((rc = search_validate(m, "relocalize_batch", "nscans", nscans, win, k, &nhyp))) return rc;
+    if (nscans < 0 || (nscans > 0 && (!offsets || !centres || !best_idx || !res))) return fail(m, NDT2D_EINVAL, "relocalize_batch: bad arguments");
+    if (nscans == 0) return NDT2D_OK;
+    if (offsets[0] < 0) return fail(m, NDT2D_EINVAL, "relocalize_batch: bad offsets");
+    int64_t max_points = 0;
+    for (int b = 0; b < nscans; ++b) {
+        const int64_t nb = offsets[b + 1] - offsets[b];
+        if (nb < 0 || nb > 0x7fffffff) return fail(m, NDT2D_EINVAL, "relocalize_batch: offsets not monotone at scan %d", b);
+        max_points = std::max(max_points, nb);
+    }
+    const int64_t total = offsets[nscans];
+    if (total > 0 && !xy) return fail(m, NDT2D_EINVAL, "relocalize_batch: bad offsets / xy");
+    DeviceGuard g(m->device);
+    const size_t njobs = (size_t)nscans * k;
+    if ((rc = upload(m, m->b_xy, xy, (size_t)total * 8))) return rc;
+    if ((rc = upload(m, m->b_off, offsets, (size_t)(nscans + 1) * 8))) return rc;
+    if ((rc = upload(m, m->b_init, centres, (size_t)nscans * 24))) return rc;
+    CK(m, m->b_tki.ensure(njobs * 8));
+    CK(m, m->b_tkv.ensure(njobs * 8));
+    CK(m, m->b_res.ensure(njobs * sizeof(ndt2d_result)));
+    rc = relocalize_batch_impl(m, level, m->b_xy.as<float>(), m->b_off.as<int64_t>(), nscans, (int)max_points, m->b_init.as<double>(), *win,
+                               nhyp, k, m->b_tki.as<int64_t>(), m->b_tkv.as<double>(), m->b_res.as<ndt2d_result>());
+    if (rc) return rc;
+    CK(m, cudaMemcpyAsync(best_idx, m->b_tki.p, njobs * 8, cudaMemcpyDeviceToHost, m->cfg.stream));
+    if (best_score) CK(m, cudaMemcpyAsync(best_score, m->b_tkv.p, njobs * 8, cudaMemcpyDeviceToHost, m->cfg.stream));
+    CK(m, cudaMemcpyAsync(res, m->b_res.p, njobs * sizeof(ndt2d_result), cudaMemcpyDeviceToHost, m->cfg.stream));
+    return ndt2d_synchronize(m);        // the one synchronisation of the call
 }
 
 } // extern "C"

@@ -351,6 +351,35 @@ class NdtMatcher2D:
                                                        _ptr(pairs), len(pairs), _ptr(d_centres), C.byref(w), int(k), _ptr(d_best_idx),
                                                        _ptr(d_best_score), _ptr(d_res)))
 
+    def relocalize_batch(self, xy, offsets, centres, window, k=4, level=0):
+        """Windowed relocalisation of a batch of scans in the handle's map (SPEC.md section 6.2): for scan b, sweep the window
+        hypotheses around centres[b] on `level`, keep the k best by (-score, index) and align the scan from each of them.
+        Equals relocalize(scan b, window_hypotheses(centres[b], window), k, level) for every scan.
+        Returns (best_idx[nscans, k], best_score[nscans, k], res[nscans, k]); an empty slot has index -1."""
+        xy = np.ascontiguousarray(xy, np.float32).reshape(-1, 2)
+        offsets = np.ascontiguousarray(offsets, np.int64)
+        centres = np.ascontiguousarray(centres, np.float64).reshape(-1, 3)
+        nb = len(offsets) - 1
+        if nb < 0 or len(centres) != nb or (nb and (offsets[0] < 0 or offsets[-1] > len(xy))):
+            raise ValueError("offsets / centres / xy sizes disagree")
+        kk = max(int(k), 0)
+        bi = np.full((nb, kk), -1, np.int64)
+        bs = np.zeros((nb, kk), np.float64)
+        res = np.zeros((nb, kk), RESULT_DTYPE)
+        w = _window(window)
+        self._ck(self._L.ndt2d_relocalize_batch(self._h, level, _ptr(xy), _ptr(offsets), nb, _ptr(centres), C.byref(w), int(k),
+                                                _ptr(bi), _ptr(bs), _ptr(res)))
+        return bi, bs, res
+
+    def relocalize_batch_device(self, d_xy, d_offsets, nscans, max_points, d_centres, window, k, d_best_idx, d_best_score, d_res,
+                                level=0):
+        """Device-resident scans / offsets / centres / outputs ([nscans * k] each; d_best_score may be None); max_points >= the
+        longest scan. Asynchronous on the handle's stream."""
+        w = _window(window)
+        self._ck(self._L.ndt2d_relocalize_batch_device(self._h, level, _ptr(d_xy), _ptr(d_offsets), int(nscans), int(max_points),
+                                                       _ptr(d_centres), C.byref(w), int(k), _ptr(d_best_idx), _ptr(d_best_score),
+                                                       _ptr(d_res)))
+
     # ---- multi-GPU sweep: best-hypothesis exchange over peer memory (one process per GPU) ----
     def exchange_create(self, world, rank, nslots=64):
         """Allocate this rank's exchange table; returns its 64-byte CUDA IPC handle (bytes) for the other ranks."""

@@ -204,6 +204,21 @@ int ndt2d_relocalize_pairs_device(ndt2d_matcher *m, int level, const float *d_xy
                                   const double *d_centres, const ndt2d_window *win, int k, int64_t *d_best_idx,
                                   double *d_best_score, ndt2d_result *d_res);
 
+/* ---- windowed search of a batch of scans against the handle's target (relocalisation in a known map, SPEC 6.2) ----
+ * Scans packed as for ndt2d_align_batch. Scan b with centre centres[3b..]: best_idx[b*k..], best_score[b*k..] and
+ * res[b*k..] equal, bit for bit, ndt2d_relocalize(level, scan b, the window's hypotheses around the centre, k) on this
+ * handle (best_score: ndt2d_sweep's top-k scores). A slot without a candidate (H < k) has index -1, score 0 and an
+ * all-zero record with status NDT2D_NO_OVERLAP. 1 <= k <= 32, nscans * k < 2^31; best_score may be NULL. Needs a
+ * target; the target, the parameters and other results are not touched. One synchronisation. */
+int ndt2d_relocalize_batch(ndt2d_matcher *m, int level, const float *xy, const int64_t *offsets, int nscans,
+                           const double *centres, const ndt2d_window *win, int k, int64_t *best_idx,
+                           double *best_score, ndt2d_result *res);
+/* scans, offsets, centres and outputs on the device, the window on the host; max_points >= longest scan (sizes the
+ * shared-memory staging, as for ndt2d_align_batch_device). Asynchronous on the handle's stream, reads nothing back. */
+int ndt2d_relocalize_batch_device(ndt2d_matcher *m, int level, const float *d_xy, const int64_t *d_offsets, int nscans,
+                                  int max_points, const double *d_centres, const ndt2d_window *win, int k,
+                                  int64_t *d_best_idx, double *d_best_score, ndt2d_result *d_res);
+
 /* ---- sweep (kernel stage 3: multi-hypothesis search for relocalisation / loop closure, SPEC 6) - */
 /* hyp[3*j..] = (tx, ty, theta) f32. scores (optional, nhyp doubles). Top-k (k >= 1) by
  * (-score, index) into best_idx[k], best_score[k]. */

@@ -176,6 +176,29 @@ class Matcher {
         return out;
     }
 
+    // windowed relocalisation of a batch of scans in this handle's map: for scan b, the window's hypotheses around centres[b]
+    // are swept on `level` and the k best refined; equals relocalize(scan b, window hypotheses, k, level) per scan.
+    // Returns nscans * k records, scan-major; indices / scores (optional) receive the k sweep indices and scores per scan
+    // (index -1: no candidate).
+    std::vector<Result> relocalizeBatch(const std::vector<Point2f> &points, const std::vector<std::int64_t> &offsets,
+                                        const std::vector<Pose2d> &centres, const ndt2d_window &window, int k, int level = 0,
+                                        std::vector<std::int64_t> *indices = nullptr, std::vector<double> *scores = nullptr)
+    {
+        if (offsets.empty()) throw std::invalid_argument("relocalizeBatch: offsets must have nscans + 1 entries");
+        if (centres.size() != offsets.size() - 1) throw std::invalid_argument("relocalizeBatch: one centre per scan");
+        if (offsets.front() < 0 || static_cast<size_t>(offsets.back()) > points.size()) throw std::invalid_argument("relocalizeBatch: offsets overrun points");
+        if (k < 1) throw std::invalid_argument("relocalizeBatch: k >= 1");
+        const size_t n = centres.size() * static_cast<size_t>(k);
+        std::vector<Result> out(n);
+        std::vector<std::int64_t> idx(n, -1);
+        std::vector<double> val(n, 0.0);
+        ck(ndt2d_relocalize_batch(h_, level, reinterpret_cast<const float *>(points.data()), offsets.data(), static_cast<int>(centres.size()),
+                                  reinterpret_cast<const double *>(centres.data()), &window, k, idx.data(), val.data(), out.data()));
+        if (indices) *indices = std::move(idx);
+        if (scores) *scores = std::move(val);
+        return out;
+    }
+
     // ---- multi-hypothesis search (relocalisation, loop-closure candidates) --------------------------
     // hypotheses: (x, y, theta) float triples. Returns the k best (index, score), best first.
     std::vector<std::pair<std::int64_t, double>> sweep(const std::vector<Point2f> &scan, const std::vector<float> &hyp_xyt, int k,

@@ -14,6 +14,37 @@ static constexpr unsigned FULL_MASK = 0xffffffffu;
 // the cells of its bounding box, so the cells live in an open-addressing hash table keyed by the dense cell index.
 static constexpr int PAIRS_LIST_CAP = 2304; // claimed-slot list per warp (u16 entries, 36 KB per block); longer: full-table scan
 
+// SPEC 2 geometry of one level of a target's grid from its bounding box: the f32 expressions of setup_level() in
+// ndt2d_capi.cu (every lane computes the same values). Returns false when the lattice is unusable (empty or >= 2^31
+// cells): nothing is inside then and every align against this target ends NO_OVERLAP.
+__device__ __forceinline__ bool pair_level_geometry(LevelDev &L, float res, int ov, bool explicit_grid, float gox, float goy, float gex,
+                                                    float gey, float xmin, float ymin, float xmax, float ymax)
+{
+    L.res = res;
+    L.ov = ov;
+    L.st = L.ov ? __fmul_rn(L.res, 0.5f) : L.res;
+    L.inv_st = __fdiv_rn(1.0f, L.st);
+    if (explicit_grid) {
+        L.ox = gox; L.oy = goy;
+        L.nhx = (int)ceilf(__fdiv_rn(gex, L.st));
+        L.nhy = (int)ceilf(__fdiv_rn(gey, L.st));
+    } else {
+        if (!(xmin <= xmax)) { xmin = xmax = ymin = ymax = 0.0f; }
+        L.ox = __fsub_rn(__fmul_rn(floorf(__fdiv_rn(xmin, L.res)), L.res), L.res);
+        L.oy = __fsub_rn(__fmul_rn(floorf(__fdiv_rn(ymin, L.res)), L.res), L.res);
+        L.nhx = (int)ceilf(__fdiv_rn(__fsub_rn(xmax, L.ox), L.st)) + 2;
+        L.nhy = (int)ceilf(__fdiv_rn(__fsub_rn(ymax, L.oy), L.st)) + 2;
+    }
+    const bool bad = L.nhx < 1 || L.nhy < 1 || (int64_t)(L.nhx + L.ov) * (int64_t)(L.nhy + L.ov) >= ((int64_t)1 << 31);
+    if (bad) { L.nhx = L.nhy = 0; }
+    L.njx = L.nhx + L.ov;
+    L.njy = L.nhy + L.ov;
+    L.inv_std = __ddiv_rn(1.0, (double)L.st);
+    L.qs = __ddiv_rn(4194304.0, (double)L.res);
+    L.qu = __dmul_rn((double)L.res, 1.0 / 4194304.0);
+    return !bad;
+}
+
 template <int OV>
 __global__ void __launch_bounds__(256) k_pairs_build(const PairBuildArgs a)
 {
@@ -48,30 +79,8 @@ __global__ void __launch_bounds__(256) k_pairs_build(const PairBuildArgs a)
             ymax = fmaxf(ymax, __shfl_xor_sync(FULL_MASK, ymax, o));
         }
     }
-    // geometry, the f32 expressions of setup_level() in ndt2d_capi.cu (every lane computes the same values)
     LevelDev L;
-    L.res = a.res[l];
-    L.ov = a.ov;
-    L.st = L.ov ? __fmul_rn(L.res, 0.5f) : L.res;
-    L.inv_st = __fdiv_rn(1.0f, L.st);
-    if (a.explicit_grid) {
-        L.ox = a.gox; L.oy = a.goy;
-        L.nhx = (int)ceilf(__fdiv_rn(a.gex, L.st));
-        L.nhy = (int)ceilf(__fdiv_rn(a.gey, L.st));
-    } else {
-        if (!(xmin <= xmax)) { xmin = xmax = ymin = ymax = 0.0f; }
-        L.ox = __fsub_rn(__fmul_rn(floorf(__fdiv_rn(xmin, L.res)), L.res), L.res);
-        L.oy = __fsub_rn(__fmul_rn(floorf(__fdiv_rn(ymin, L.res)), L.res), L.res);
-        L.nhx = (int)ceilf(__fdiv_rn(__fsub_rn(xmax, L.ox), L.st)) + 2;
-        L.nhy = (int)ceilf(__fdiv_rn(__fsub_rn(ymax, L.oy), L.st)) + 2;
-    }
-    bool too_big = L.nhx < 1 || L.nhy < 1 || (int64_t)(L.nhx + L.ov) * (int64_t)(L.nhy + L.ov) >= ((int64_t)1 << 31);
-    if (too_big) { L.nhx = L.nhy = 0; }      // nothing is inside: every align against this target ends NO_OVERLAP
-    L.njx = L.nhx + L.ov;
-    L.njy = L.nhy + L.ov;
-    L.inv_std = __ddiv_rn(1.0, (double)L.st);
-    L.qs = __ddiv_rn(4194304.0, (double)L.res);
-    L.qu = __dmul_rn((double)L.res, 1.0 / 4194304.0);
+    const bool too_big = !pair_level_geometry(L, a.res[l], a.ov, a.explicit_grid != 0, a.gox, a.goy, a.gex, a.gey, xmin, ymin, xmax, ymax);
     L.hash_mask = a.cap - 1u;
     float4 *rec = a.tab + (size_t)wid * ((size_t)a.cap + 1) * 2;
     uint32_t *cnt = a.cnt + (size_t)wid * a.cap;
@@ -162,37 +171,6 @@ __global__ void __launch_bounds__(256) k_pairs_build(const PairBuildArgs a)
 static constexpr int FUSED_WARPS_MAX = 8;        // warps per block: as many as let two blocks share an SM, at most this (5 at 1080-point scans)
 static constexpr unsigned FUSED_WS_BYTES = 224;    // room for the WarpState (216 B)
 static constexpr unsigned FUSED_STATE_BYTES = 352; // WarpState + LevelDev (112 B), rounded up to 16
-
-// SPEC 2 geometry of one level of a target's grid from its bounding box: the f32 expressions of setup_level() in
-// ndt2d_capi.cu (every lane computes the same values). Returns false when the lattice is unusable (empty or >= 2^31
-// cells): nothing is inside then and every align against this target ends NO_OVERLAP.
-__device__ __forceinline__ bool pair_level_geometry(LevelDev &L, float res, int ov, bool explicit_grid, float gox, float goy, float gex,
-                                                    float gey, float xmin, float ymin, float xmax, float ymax)
-{
-    L.res = res;
-    L.ov = ov;
-    L.st = L.ov ? __fmul_rn(L.res, 0.5f) : L.res;
-    L.inv_st = __fdiv_rn(1.0f, L.st);
-    if (explicit_grid) {
-        L.ox = gox; L.oy = goy;
-        L.nhx = (int)ceilf(__fdiv_rn(gex, L.st));
-        L.nhy = (int)ceilf(__fdiv_rn(gey, L.st));
-    } else {
-        if (!(xmin <= xmax)) { xmin = xmax = ymin = ymax = 0.0f; }
-        L.ox = __fsub_rn(__fmul_rn(floorf(__fdiv_rn(xmin, L.res)), L.res), L.res);
-        L.oy = __fsub_rn(__fmul_rn(floorf(__fdiv_rn(ymin, L.res)), L.res), L.res);
-        L.nhx = (int)ceilf(__fdiv_rn(__fsub_rn(xmax, L.ox), L.st)) + 2;
-        L.nhy = (int)ceilf(__fdiv_rn(__fsub_rn(ymax, L.oy), L.st)) + 2;
-    }
-    const bool bad = L.nhx < 1 || L.nhy < 1 || (int64_t)(L.nhx + L.ov) * (int64_t)(L.nhy + L.ov) >= ((int64_t)1 << 31);
-    if (bad) { L.nhx = L.nhy = 0; }
-    L.njx = L.nhx + L.ov;
-    L.njy = L.nhy + L.ov;
-    L.inv_std = __ddiv_rn(1.0, (double)L.st);
-    L.qs = __ddiv_rn(4194304.0, (double)L.res);
-    L.qu = __dmul_rn((double)L.res, 1.0 / 4194304.0);
-    return !bad;
-}
 
 // SPEC 3 for one (target scan, level) by ONE warp, entirely in its shared-memory slice. The integer sums are order
 // independent, so grouping the points by cell with a sort and summing each group in one lane gives the sums - and
@@ -789,11 +767,17 @@ __global__ void k_search_clear(const int64_t *__restrict__ best_idx, int n, ndt2
 // Shared-memory layout of k_search_sweep behind its head: TABLE_SHASH: the build's sort area, records and bucket index as in
 // k_pairs_fused (f.cap_t, f.rmax, f.hslots from pairs_fused_layout), then the source; TABLE_GHASH: the source only. Returns
 // the dynamic shared memory per block; staged = false when the source does not fit (global reads, TABLE_GHASH only).
+// TABLE_SHASH also takes the lattice of level s.level, the cell parameters and the error flag from f.
 size_t search_layout(SearchArgs &s, const PairFusedArgs *f, int64_t max_source_points, int smem_optin, bool &staged)
 {
     auto up16 = [](size_t v) { return (v + 15) & ~(size_t)15; };
     size_t off = 0;
     if (f) {
+        s.explicit_grid = f->explicit_grid;
+        s.res_m = f->res_m[s.level];
+        s.gox = f->gox; s.goy = f->goy; s.gex = f->gex; s.gey = f->gey;
+        s.min_points = f->prm.min_points; s.eig_ratio = f->prm.eig_ratio;
+        s.error = f->error;
         s.cap_t = f->cap_t;
         s.hslots = f->hslots;
         s.off_r = (unsigned)up16((size_t)f->cap_t * 4 + 2 * ((size_t)f->cap_t + 2) * 2);
@@ -947,45 +931,111 @@ static int pairs_general(ndt2d_matcher *m, const char *name, const float *d_xy, 
 
 extern "C" {
 
-// d_xy / d_offsets / d_init / d_res: device; h_offsets / pairs: host (the chunking and the target list are host work).
-// One chunk = as many pairs as fit the table budget. Asynchronous on the handle's stream apart from the uploads of the
-// small per-chunk index lists; *err_out (optional) receives the device error flag after a synchronisation.
-static int align_pairs_impl(ndt2d_matcher *m, const float *d_xy, const int64_t *d_offsets, const int64_t *h_offsets, int nscans,
-                            const int32_t *pairs, int npairs, const double *d_init, ndt2d_result *d_res)
+// ---- checks, set-up and host buffers shared by the calls over packed scans ----
+
+// Packed scans: offsets[0] >= 0, scan b = [offsets[b], offsets[b + 1]) of at most INT_MAX points. *max_points (optional):
+// the longest scan.
+static int scans_validate(ndt2d_matcher *m, const char *name, const int64_t *offsets, int nscans, int64_t *max_points)
 {
-    int64_t max_src = 0, max_tgt = 0;
+    if (nscans > 0 && offsets[0] < 0) return fail(m, NDT2D_EINVAL, "%s: bad offsets", name);
+    int64_t longest = 0;
+    for (int b = 0; b < nscans; ++b) {
+        const int64_t nb = offsets[b + 1] - offsets[b];
+        if (nb < 0 || nb > 0x7fffffff) return fail(m, NDT2D_EINVAL, "%s: offsets not monotone at scan %d", name, b);
+        longest = std::max(longest, nb);
+    }
+    if (max_points) *max_points = longest;
+    return NDT2D_OK;
+}
+
+// The packed scans and the (target scan, source scan) pairs of a call over pairs; *max_tgt / *max_src: the longest target
+// and source scan of any pair.
+static int pairs_validate(ndt2d_matcher *m, const char *name, const int64_t *offsets, int nscans, const int32_t *pairs, int npairs,
+                          int64_t *max_tgt, int64_t *max_src)
+{
+    if (nscans < 0 || npairs < 0 || (nscans > 0 && !offsets) || (npairs > 0 && !pairs)) return fail(m, NDT2D_EINVAL, "%s: bad arguments", name);
+    if (m->nlevels < 1) return fail(m, NDT2D_EINVAL, "%s: no resolution set", name);
+    int rc = scans_validate(m, name, offsets, nscans, nullptr);
+    if (rc) return rc;
+    *max_tgt = *max_src = 0;
     for (int p = 0; p < npairs; ++p) {
         const int t = pairs[2 * p], s = pairs[2 * p + 1];
-        if (t < 0 || t >= nscans || s < 0 || s >= nscans) return fail(m, NDT2D_EINVAL, "pair %d: scan index out of range", p);
-        max_tgt = std::max(max_tgt, h_offsets[t + 1] - h_offsets[t]);
-        max_src = std::max(max_src, h_offsets[s + 1] - h_offsets[s]);
+        if (t < 0 || t >= nscans || s < 0 || s >= nscans) return fail(m, NDT2D_EINVAL, "%s: pair %d: scan index out of range", name, p);
+        *max_tgt = std::max(*max_tgt, offsets[t + 1] - offsets[t]);
+        *max_src = std::max(*max_src, offsets[s + 1] - offsets[s]);
     }
-    const int K = m->prm.overlap ? 4 : 1, L = m->nlevels;
+    return NDT2D_OK;
+}
+
+// Host-buffer form: uploads the packed scans, their offsets and one pose per item (initial pose or window centre).
+static int upload_scans(ndt2d_matcher *m, const char *name, const float *xy, const int64_t *offsets, int nscans, const double *poses,
+                        int nitems)
+{
+    const int64_t total = offsets[nscans];
+    if (total > 0 && !xy) return fail(m, NDT2D_EINVAL, "%s: bad offsets / xy", name);
+    int rc;
+    if ((rc = upload(m, m->b_xy, xy, (size_t)total * 8))) return rc;
+    if ((rc = upload(m, m->b_off, offsets, (size_t)(nscans + 1) * 8))) return rc;
+    return upload(m, m->b_init, poses, (size_t)nitems * 24);
+}
+
+// End of a host-buffer call: copies best_idx and best_score (when given) and the n records back, synchronises once and
+// reports the device error flag d_error (nullptr: the call has none).
+static int finish_host_call(ndt2d_matcher *m, const char *name, size_t n, int64_t *best_idx, double *best_score, ndt2d_result *res,
+                            const int *d_error)
+{
+    if (best_idx) CK(m, cudaMemcpyAsync(best_idx, m->b_tki.p, n * 8, cudaMemcpyDeviceToHost, m->cfg.stream));
+    if (best_score) CK(m, cudaMemcpyAsync(best_score, m->b_tkv.p, n * 8, cudaMemcpyDeviceToHost, m->cfg.stream));
+    CK(m, cudaMemcpyAsync(res, m->b_res.p, n * sizeof(ndt2d_result), cudaMemcpyDeviceToHost, m->cfg.stream));
+    int err = 0;
+    if (d_error) CK(m, cudaMemcpyAsync(&err, d_error, 4, cudaMemcpyDeviceToHost, m->cfg.stream));
+    int rc = ndt2d_synchronize(m);
+    if (rc) return rc;
+    if (err) return fail(m, NDT2D_EINVAL, "%s: the auto-fitted lattice of a target scan exceeds 2^31 cells "
+                                          "(a point far from the rest?); its pairs were returned with status NO_OVERLAP", name);
+    return NDT2D_OK;
+}
+
+// Whether the shared-memory path (k_pairs_fused; k_search_sweep with TABLE_SHASH) runs: grids without overlap (K = 1), the
+// path not switched off by NDT2D_PAIRS_FUSED=0, and scans that fit a warp's shared-memory slice (1080-beam scans: 27 KB per
+// warp, 8 warps per SM). When it does, f holds the handle's parameters, levels and lattice, the slice layout, the work-queue
+// counter and the error flag; the caller sets the scans, pairs, initial poses and results.
+static bool pairs_fused_setup(ndt2d_matcher *m, int64_t max_tgt, int64_t max_src, PairFusedArgs &f)
+{
+    memset(&f, 0, sizeof(f));
+    f.prm = m->prm;
+    const char *env = getenv("NDT2D_PAIRS_FUSED");
+    if (m->prm.overlap || (env && atoi(env) == 0) || !pairs_fused_layout(f, max_tgt, max_src, m->cfg.max_smem_optin)) return false;
+    f.nlevels = m->nlevels;
+    f.explicit_grid = m->explicit_grid ? 1 : 0;
+    for (int l = 0; l < m->nlevels; ++l) f.res_m[l] = m->res[l];
+    f.gox = m->gox; f.goy = m->goy; f.gex = m->gex; f.gey = m->gey;
+    f.counter = m->b_counter.as<unsigned int>();
+    f.error = m->b_perr.as<int>();
+    return true;
+}
+
+// d_xy / d_offsets / d_init / d_res: device; pairs: host (the chunking and the target list are host work). One chunk = as
+// many pairs as fit the table budget. Asynchronous on the handle's stream apart from the uploads of `pairs` (shared-memory
+// path) or of the small per-chunk index lists (general path); a target whose lattice exceeds 2^31 cells sets b_perr.
+static int align_pairs_impl(ndt2d_matcher *m, const float *d_xy, const int64_t *d_offsets, int nscans, const int32_t *pairs, int npairs,
+                            int64_t max_tgt, int64_t max_src, const double *d_init, ndt2d_result *d_res)
+{
     CK(m, m->b_perr.ensure(4));
     CK(m, cudaMemsetAsync(m->b_perr.p, 0, 4, m->cfg.stream));
-    // fused path: K = 1 and scans that fit a warp's shared-memory slice (1080-beam scans: 27 KB per warp, 8 warps per SM)
-    {
-        PairFusedArgs f;
-        memset(&f, 0, sizeof(f));
-        f.prm = m->prm;
-        const char *env = getenv("NDT2D_PAIRS_FUSED");
-        if (K == 1 && !(env && atoi(env) == 0) && pairs_fused_layout(f, max_tgt, max_src, m->cfg.max_smem_optin)) {
-            int rcu;
-            if ((rcu = upload(m, m->b_ppairs, pairs, (size_t)npairs * 8))) return rcu;
-            CK(m, cudaStreamSynchronize(m->cfg.stream));     // `pairs` is the caller's buffer
-            f.xy = reinterpret_cast<const float2 *>(d_xy);
-            f.offsets = d_offsets;
-            f.pairs = m->b_ppairs.as<int32_t>();
-            f.init = d_init;
-            f.res = d_res;
-            f.npairs = npairs; f.nlevels = L; f.explicit_grid = m->explicit_grid ? 1 : 0;
-            for (int l = 0; l < L; ++l) f.res_m[l] = m->res[l];
-            f.gox = m->gox; f.goy = m->goy; f.gex = m->gex; f.gey = m->gey;
-            f.counter = m->b_counter.as<unsigned int>();
-            f.error = m->b_perr.as<int>();
-            CK(m, launch_pairs_fused(m->cfg, f, &m->launches));
-            return NDT2D_OK;
-        }
+    PairFusedArgs f;
+    if (pairs_fused_setup(m, max_tgt, max_src, f)) {
+        int rc;
+        if ((rc = upload(m, m->b_ppairs, pairs, (size_t)npairs * 8))) return rc;
+        CK(m, cudaStreamSynchronize(m->cfg.stream));     // `pairs` is the caller's buffer
+        f.xy = reinterpret_cast<const float2 *>(d_xy);
+        f.offsets = d_offsets;
+        f.pairs = m->b_ppairs.as<int32_t>();
+        f.init = d_init;
+        f.res = d_res;
+        f.npairs = npairs;
+        CK(m, launch_pairs_fused(m->cfg, f, &m->launches));
+        return NDT2D_OK;
     }
     return pairs_general(m, "align_pairs", d_xy, d_offsets, nscans, pairs, npairs, max_tgt, [&](int p0, int p1) {
         AlignArgs a{};
@@ -1000,61 +1050,35 @@ static int align_pairs_impl(ndt2d_matcher *m, const float *d_xy, const int64_t *
     });
 }
 
-static int align_pairs_check(ndt2d_matcher *m)
-{
-    int err = 0;
-    CK(m, cudaMemcpyAsync(&err, m->b_perr.p, 4, cudaMemcpyDeviceToHost, m->cfg.stream));
-    int rc = ndt2d_synchronize(m);
-    if (rc) return rc;
-    if (err) return fail(m, NDT2D_EINVAL, "align_pairs: the auto-fitted lattice of a target scan exceeds 2^31 cells "
-                                          "(a point far from the rest?); its pairs were returned with status NO_OVERLAP");
-    return NDT2D_OK;
-}
-
-static int align_pairs_validate(ndt2d_matcher *m, const int64_t *offsets, int nscans, const int32_t *pairs, int npairs)
-{
-    if (nscans < 0 || npairs < 0 || (nscans > 0 && !offsets) || (npairs > 0 && !pairs)) return fail(m, NDT2D_EINVAL, "bad arguments");
-    if (m->nlevels < 1) return fail(m, NDT2D_EINVAL, "no resolution set");
-    for (int b = 0; b < nscans; ++b) {
-        int64_t nb = offsets[b + 1] - offsets[b];
-        if (nb < 0 || nb > 0x7fffffff) return fail(m, NDT2D_EINVAL, "offsets not monotone at scan %d", b);
-    }
-    if (nscans > 0 && offsets[0] < 0) return fail(m, NDT2D_EINVAL, "bad offsets");
-    return NDT2D_OK;
-}
-
 int ndt2d_align_pairs_device(ndt2d_matcher *m, const float *d_xy, const int64_t *d_offsets, const int64_t *offsets, int nscans,
                              const int32_t *pairs, int npairs, const double *d_init, ndt2d_result *d_res)
 {
     if (!m) return NDT2D_EINVAL;
-    int rc = align_pairs_validate(m, offsets, nscans, pairs, npairs);
+    int64_t max_tgt = 0, max_src = 0;
+    int rc = pairs_validate(m, "align_pairs", offsets, nscans, pairs, npairs, &max_tgt, &max_src);
     if (rc) return rc;
     if (npairs == 0) return NDT2D_OK;
     if (!d_offsets || !d_init || !d_res) return fail(m, NDT2D_EINVAL, "bad arguments");
     DeviceGuard g(m->device);
-    return align_pairs_impl(m, d_xy, d_offsets, offsets, nscans, pairs, npairs, d_init, d_res);
+    return align_pairs_impl(m, d_xy, d_offsets, nscans, pairs, npairs, max_tgt, max_src, d_init, d_res);
 }
 
 int ndt2d_align_pairs(ndt2d_matcher *m, const float *xy, const int64_t *offsets, int nscans, const int32_t *pairs, int npairs,
                       const double *init, ndt2d_result *res)
 {
     if (!m) return NDT2D_EINVAL;
-    int rc = align_pairs_validate(m, offsets, nscans, pairs, npairs);
+    int64_t max_tgt = 0, max_src = 0;
+    int rc = pairs_validate(m, "align_pairs", offsets, nscans, pairs, npairs, &max_tgt, &max_src);
     if (rc) return rc;
     if (npairs == 0) return NDT2D_OK;
     if (!init || !res) return fail(m, NDT2D_EINVAL, "bad arguments");
-    const int64_t total = offsets[nscans];
-    if (total > 0 && !xy) return fail(m, NDT2D_EINVAL, "bad offsets / xy");
     DeviceGuard g(m->device);
-    if ((rc = upload(m, m->b_xy, xy, (size_t)total * 8))) return rc;
-    if ((rc = upload(m, m->b_off, offsets, (size_t)(nscans + 1) * 8))) return rc;
-    if ((rc = upload(m, m->b_init, init, (size_t)npairs * 24))) return rc;
+    if ((rc = upload_scans(m, "align_pairs", xy, offsets, nscans, init, npairs))) return rc;
     CK(m, m->b_res.ensure((size_t)npairs * sizeof(ndt2d_result)));
-    rc = align_pairs_impl(m, m->b_xy.as<float>(), m->b_off.as<int64_t>(), offsets, nscans, pairs, npairs, m->b_init.as<double>(),
+    rc = align_pairs_impl(m, m->b_xy.as<float>(), m->b_off.as<int64_t>(), nscans, pairs, npairs, max_tgt, max_src, m->b_init.as<double>(),
                           m->b_res.as<ndt2d_result>());
     if (rc) return rc;
-    CK(m, cudaMemcpyAsync(res, m->b_res.p, (size_t)npairs * sizeof(ndt2d_result), cudaMemcpyDeviceToHost, m->cfg.stream));
-    return align_pairs_check(m);
+    return finish_host_call(m, "align_pairs", (size_t)npairs, nullptr, nullptr, res, m->b_perr.as<int>());
 }
 
 // ---- windowed search over pairs (SPEC 6.1): ndt2d_set_target(target) + ndt2d_relocalize(source, window) per pair ----
@@ -1080,91 +1104,77 @@ static int search_validate(ndt2d_matcher *m, const char *name, const char *what,
     return NDT2D_OK;
 }
 
-static int relocalize_pairs_validate(ndt2d_matcher *m, int level, const int64_t *offsets, int nscans, const int32_t *pairs, int npairs,
-                                     const ndt2d_window *win, int k, long long *nhyp)
+// The SearchArgs fields of every windowed search, and room for njobs refinement jobs of job_bytes each and their initial poses
+static int search_setup(ndt2d_matcher *m, SearchArgs &s, const float *d_xy, const int64_t *d_offsets, const ndt2d_window &win,
+                        long long nhyp, int k, int level, size_t njobs, size_t job_bytes)
 {
-    int rc = align_pairs_validate(m, offsets, nscans, pairs, npairs);
-    if (rc) return rc;
-    if (level < 0 || level >= m->nlevels) return fail(m, NDT2D_EINVAL, "level %d out of range [0, %d)", level, m->nlevels);
-    if ((rc = search_validate(m, "relocalize_pairs", "npairs", npairs, win, k, nhyp))) return rc;
-    for (int p = 0; p < npairs; ++p) {
-        const int t = pairs[2 * p], s = pairs[2 * p + 1];
-        if (t < 0 || t >= nscans || s < 0 || s >= nscans) return fail(m, NDT2D_EINVAL, "pair %d: scan index out of range", p);
-    }
-    return NDT2D_OK;
-}
-
-// Shared-memory path (K = 1 and scans that pairs_fused_layout admits, as ndt2d_align_pairs): sweep, top-k, refinement by
-// k_pairs_fused and the empty slots: four launches whatever the number of pairs. General path: per chunk of the per-target
-// tables, the table build, the same sweep and top-k on the tables, k_align in pairs mode and the empty slots.
-static int relocalize_pairs_impl(ndt2d_matcher *m, int level, const float *d_xy, const int64_t *d_offsets, const int64_t *h_offsets,
-                                 int nscans, const int32_t *pairs, int npairs, const double *d_centres, const ndt2d_window &win,
-                                 long long nhyp, int k, int64_t *d_best_idx, double *d_best_score, ndt2d_result *d_res)
-{
-    int64_t max_src = 0, max_tgt = 0;
-    for (int p = 0; p < npairs; ++p) {
-        max_tgt = std::max(max_tgt, h_offsets[pairs[2 * p] + 1] - h_offsets[pairs[2 * p]]);
-        max_src = std::max(max_src, h_offsets[pairs[2 * p + 1] + 1] - h_offsets[pairs[2 * p + 1]]);
-    }
-    const int L = m->nlevels;
-    const size_t njobs = (size_t)npairs * k;
-    CK(m, m->b_perr.ensure(4));
-    CK(m, cudaMemsetAsync(m->b_perr.p, 0, 4, m->cfg.stream));
-    CK(m, m->b_sjobs.ensure(njobs * 8));
+    CK(m, m->b_sjobs.ensure(njobs * job_bytes));
     CK(m, m->b_sinit.ensure(njobs * 24));
-    SearchArgs s;
     memset(&s, 0, sizeof(s));
     s.xy = reinterpret_cast<const float2 *>(d_xy);
     s.offsets = d_offsets;
     s.win = win;
     s.nhyp = nhyp;
-    s.k = k; s.level = level; s.nlevels = L;
+    s.k = k; s.level = level; s.nlevels = m->nlevels;
     s.counter = m->b_counter.as<unsigned int>();
-    s.error = m->b_perr.as<int>();
+    return NDT2D_OK;
+}
+
+// The hypothesis chunks of one sweep launch over `items` work items, and the candidate buffer for them
+static cudaError_t search_candidates(ndt2d_matcher *m, SearchArgs &s, int items)
+{
+    s.chunks = search_chunks(m->cfg, items, s.nhyp);
+    const cudaError_t e = m->b_scand.ensure((size_t)items * s.chunks * s.k * sizeof(SearchCand));
+    s.cand = m->b_scand.as<SearchCand>();
+    return e;
+}
+
+static int relocalize_pairs_validate(ndt2d_matcher *m, int level, const int64_t *offsets, int nscans, const int32_t *pairs, int npairs,
+                                     const ndt2d_window *win, int k, long long *nhyp, int64_t *max_tgt, int64_t *max_src)
+{
+    int rc = pairs_validate(m, "relocalize_pairs", offsets, nscans, pairs, npairs, max_tgt, max_src);
+    if (rc) return rc;
+    if (level < 0 || level >= m->nlevels) return fail(m, NDT2D_EINVAL, "level %d out of range [0, %d)", level, m->nlevels);
+    return search_validate(m, "relocalize_pairs", "npairs", npairs, win, k, nhyp);
+}
+
+// Shared-memory path (as ndt2d_align_pairs, when k_search_sweep can also stage the longest source): sweep, top-k, refinement
+// by k_pairs_fused and the empty slots: four launches whatever the number of pairs. General path: per chunk of the per-target
+// tables, the table build, the same sweep and top-k on the tables, k_align in pairs mode and the empty slots.
+static int relocalize_pairs_impl(ndt2d_matcher *m, int level, const float *d_xy, const int64_t *d_offsets, int nscans, const int32_t *pairs,
+                                 int npairs, int64_t max_tgt, int64_t max_src, const double *d_centres, const ndt2d_window &win,
+                                 long long nhyp, int k, int64_t *d_best_idx, double *d_best_score, ndt2d_result *d_res)
+{
+    const size_t njobs = (size_t)npairs * k;
+    CK(m, m->b_perr.ensure(4));
+    CK(m, cudaMemsetAsync(m->b_perr.p, 0, 4, m->cfg.stream));
+    SearchArgs s;
+    int rc = search_setup(m, s, d_xy, d_offsets, win, nhyp, k, level, njobs, 8);
+    if (rc) return rc;
     int32_t *d_jobs = m->b_sjobs.as<int32_t>();
     double *d_jinit = m->b_sinit.as<double>();
-    auto cand = [&](int pairs_in_call) -> cudaError_t {
-        s.chunks = search_chunks(m->cfg, pairs_in_call, nhyp);
-        cudaError_t e = m->b_scand.ensure((size_t)pairs_in_call * s.chunks * k * sizeof(SearchCand));
-        s.cand = m->b_scand.as<SearchCand>();
-        return e;
-    };
     PairFusedArgs f;
-    memset(&f, 0, sizeof(f));
-    f.prm = m->prm;
-    const char *env = getenv("NDT2D_PAIRS_FUSED");
     bool staged = false;
     size_t smem = 0;
-    if (!m->prm.overlap && !(env && atoi(env) == 0) && pairs_fused_layout(f, max_tgt, max_src, m->cfg.max_smem_optin) &&
-        (smem = search_layout(s, &f, max_src, m->cfg.max_smem_optin, staged), staged)) {
-        int rc;
+    if (pairs_fused_setup(m, max_tgt, max_src, f) && (smem = search_layout(s, &f, max_src, m->cfg.max_smem_optin, staged), staged)) {
         // `pairs` is the caller's buffer: it is uploaded from a copy, so that nothing waits for the copy to finish
         m->h_spairs.assign(pairs, pairs + 2 * (size_t)npairs);
         if ((rc = upload(m, m->b_ppairs, m->h_spairs.data(), (size_t)npairs * 8))) return rc;
         s.pairs = m->b_ppairs.as<int32_t>();
         s.centres = d_centres;
         s.npairs = npairs;
-        s.explicit_grid = m->explicit_grid ? 1 : 0;
-        s.res_m = m->res[level];
-        s.gox = m->gox; s.goy = m->goy; s.gex = m->gex; s.gey = m->gey;
-        s.min_points = m->prm.min_points; s.eig_ratio = m->prm.eig_ratio;
-        CK(m, cand(npairs));
+        CK(m, search_candidates(m, s, npairs));
         CK(m, launch_search(m->cfg, s, false, TABLE_SHASH, true, smem, d_best_idx, d_best_score, d_jobs, d_jinit, &m->launches));
         f.xy = s.xy;
         f.offsets = d_offsets;
         f.pairs = d_jobs;
         f.init = d_jinit;
         f.res = d_res;
-        f.npairs = (int)njobs; f.nlevels = L; f.explicit_grid = s.explicit_grid;
-        for (int l = 0; l < L; ++l) f.res_m[l] = m->res[l];
-        f.gox = m->gox; f.goy = m->goy; f.gex = m->gex; f.gey = m->gey;
-        f.counter = s.counter;
-        f.error = s.error;
+        f.npairs = (int)njobs;
         CK(m, launch_pairs_fused(m->cfg, f, &m->launches));
         CK(m, launch_search_clear(m->cfg, d_best_idx, (int)njobs, d_res, &m->launches));
         return NDT2D_OK;
     }
-    memset(&f, 0, sizeof(f));
     smem = search_layout(s, nullptr, max_src, m->cfg.max_smem_optin, staged);
     return pairs_general(m, "relocalize_pairs", d_xy, d_offsets, nscans, pairs, npairs, max_tgt, [&](int p0, int p1) -> int {
         const size_t j0 = (size_t)p0 * k, nj = (size_t)(p1 - p0) * k;
@@ -1172,7 +1182,7 @@ static int relocalize_pairs_impl(ndt2d_matcher *m, int level, const float *d_xy,
         s.geo = m->b_pgeo.as<LevelDev>();
         s.centres = d_centres + 3 * (size_t)p0;
         s.npairs = p1 - p0;
-        CK(m, cand(p1 - p0));
+        CK(m, search_candidates(m, s, p1 - p0));
         CK(m, launch_search(m->cfg, s, m->prm.overlap != 0, TABLE_GHASH, staged, smem, d_best_idx + j0, d_best_score ? d_best_score + j0 : nullptr,
                             d_jobs, d_jinit, &m->launches));
         AlignArgs a{};
@@ -1196,12 +1206,13 @@ int ndt2d_relocalize_pairs_device(ndt2d_matcher *m, int level, const float *d_xy
 {
     if (!m) return NDT2D_EINVAL;
     long long nhyp = 0;
-    int rc = relocalize_pairs_validate(m, level, offsets, nscans, pairs, npairs, win, k, &nhyp);
+    int64_t max_tgt = 0, max_src = 0;
+    int rc = relocalize_pairs_validate(m, level, offsets, nscans, pairs, npairs, win, k, &nhyp, &max_tgt, &max_src);
     if (rc) return rc;
     if (npairs == 0) return NDT2D_OK;
     if (!d_offsets || !d_centres || !d_best_idx || !d_res) return fail(m, NDT2D_EINVAL, "bad arguments");
     DeviceGuard g(m->device);
-    return relocalize_pairs_impl(m, level, d_xy, d_offsets, offsets, nscans, pairs, npairs, d_centres, *win, nhyp, k, d_best_idx,
+    return relocalize_pairs_impl(m, level, d_xy, d_offsets, nscans, pairs, npairs, max_tgt, max_src, d_centres, *win, nhyp, k, d_best_idx,
                                  d_best_score, d_res);
 }
 
@@ -1211,32 +1222,21 @@ int ndt2d_relocalize_pairs(ndt2d_matcher *m, int level, const float *xy, const i
 {
     if (!m) return NDT2D_EINVAL;
     long long nhyp = 0;
-    int rc = relocalize_pairs_validate(m, level, offsets, nscans, pairs, npairs, win, k, &nhyp);
+    int64_t max_tgt = 0, max_src = 0;
+    int rc = relocalize_pairs_validate(m, level, offsets, nscans, pairs, npairs, win, k, &nhyp, &max_tgt, &max_src);
     if (rc) return rc;
     if (npairs == 0) return NDT2D_OK;
     if (!centres || !best_idx || !res) return fail(m, NDT2D_EINVAL, "bad arguments");
-    const int64_t total = offsets[nscans];
-    if (total > 0 && !xy) return fail(m, NDT2D_EINVAL, "bad offsets / xy");
     DeviceGuard g(m->device);
     const size_t njobs = (size_t)npairs * k;
-    if ((rc = upload(m, m->b_xy, xy, (size_t)total * 8))) return rc;
-    if ((rc = upload(m, m->b_off, offsets, (size_t)(nscans + 1) * 8))) return rc;
-    if ((rc = upload(m, m->b_init, centres, (size_t)npairs * 24))) return rc;
+    if ((rc = upload_scans(m, "relocalize_pairs", xy, offsets, nscans, centres, npairs))) return rc;
     CK(m, m->b_tki.ensure(njobs * 8));
     CK(m, m->b_tkv.ensure(njobs * 8));
     CK(m, m->b_res.ensure(njobs * sizeof(ndt2d_result)));
-    rc = relocalize_pairs_impl(m, level, m->b_xy.as<float>(), m->b_off.as<int64_t>(), offsets, nscans, pairs, npairs, m->b_init.as<double>(),
-                               *win, nhyp, k, m->b_tki.as<int64_t>(), m->b_tkv.as<double>(), m->b_res.as<ndt2d_result>());
+    rc = relocalize_pairs_impl(m, level, m->b_xy.as<float>(), m->b_off.as<int64_t>(), nscans, pairs, npairs, max_tgt, max_src,
+                               m->b_init.as<double>(), *win, nhyp, k, m->b_tki.as<int64_t>(), m->b_tkv.as<double>(), m->b_res.as<ndt2d_result>());
     if (rc) return rc;
-    CK(m, cudaMemcpyAsync(best_idx, m->b_tki.p, njobs * 8, cudaMemcpyDeviceToHost, m->cfg.stream));
-    if (best_score) CK(m, cudaMemcpyAsync(best_score, m->b_tkv.p, njobs * 8, cudaMemcpyDeviceToHost, m->cfg.stream));
-    CK(m, cudaMemcpyAsync(res, m->b_res.p, njobs * sizeof(ndt2d_result), cudaMemcpyDeviceToHost, m->cfg.stream));
-    int err = 0;
-    CK(m, cudaMemcpyAsync(&err, m->b_perr.p, 4, cudaMemcpyDeviceToHost, m->cfg.stream));
-    if ((rc = ndt2d_synchronize(m))) return rc;     // the one synchronisation of the call (shared-memory path)
-    if (err) return fail(m, NDT2D_EINVAL, "relocalize_pairs: the auto-fitted lattice of a target scan exceeds 2^31 cells "
-                                          "(a point far from the rest?); its pairs were returned with status NO_OVERLAP");
-    return NDT2D_OK;
+    return finish_host_call(m, "relocalize_pairs", njobs, best_idx, best_score, res, m->b_perr.as<int>());
 }
 
 // ---- windowed search of a batch of scans against the handle's target (SPEC 6.2): ndt2d_relocalize(scan, window) per scan ----
@@ -1248,26 +1248,16 @@ static int relocalize_batch_impl(ndt2d_matcher *m, int level, const float *d_xy,
                                  double *d_best_score, ndt2d_result *d_res)
 {
     const size_t njobs = (size_t)nscans * k;
-    CK(m, m->b_sjobs.ensure(njobs * 4));
-    CK(m, m->b_sinit.ensure(njobs * 24));
-    // the sweep reads the level from the device (SearchArgs::geo); the copy is taken now, so a later set_target cannot reach it
-    int rc = upload(m, m->b_slevels, m->lv, (size_t)m->nlevels * sizeof(LevelDev));
-    if (rc) return rc;
     SearchArgs s;
-    memset(&s, 0, sizeof(s));
-    s.xy = reinterpret_cast<const float2 *>(d_xy);
-    s.offsets = d_offsets;
+    int rc = search_setup(m, s, d_xy, d_offsets, win, nhyp, k, level, njobs, 4);
+    if (rc) return rc;
+    // the sweep reads the level from the device (SearchArgs::geo); the copy is taken now, so a later set_target cannot reach it
+    if ((rc = upload(m, m->b_slevels, m->lv, (size_t)m->nlevels * sizeof(LevelDev)))) return rc;
     s.geo = m->b_slevels.as<LevelDev>();
     s.centres = d_centres;
-    s.win = win;
-    s.nhyp = nhyp;
     s.npairs = nscans;
-    s.k = k; s.level = level; s.nlevels = m->nlevels;
-    s.counter = m->b_counter.as<unsigned int>();
     // every item stages only its scan (no table build), so the chunking is the pairs' one without a table to amortise
-    s.chunks = search_chunks(m->cfg, nscans, nhyp);
-    CK(m, m->b_scand.ensure((size_t)nscans * s.chunks * k * sizeof(SearchCand)));
-    s.cand = m->b_scand.as<SearchCand>();
+    CK(m, search_candidates(m, s, nscans));
     bool staged = false;
     const size_t smem = search_layout(s, nullptr, max_points, m->cfg.max_smem_optin, staged);
     int32_t *d_jobs = m->b_sjobs.as<int32_t>();
@@ -1309,30 +1299,18 @@ int ndt2d_relocalize_batch(ndt2d_matcher *m, int level, const float *xy, const i
     if ((rc = search_validate(m, "relocalize_batch", "nscans", nscans, win, k, &nhyp))) return rc;
     if (nscans < 0 || (nscans > 0 && (!offsets || !centres || !best_idx || !res))) return fail(m, NDT2D_EINVAL, "relocalize_batch: bad arguments");
     if (nscans == 0) return NDT2D_OK;
-    if (offsets[0] < 0) return fail(m, NDT2D_EINVAL, "relocalize_batch: bad offsets");
     int64_t max_points = 0;
-    for (int b = 0; b < nscans; ++b) {
-        const int64_t nb = offsets[b + 1] - offsets[b];
-        if (nb < 0 || nb > 0x7fffffff) return fail(m, NDT2D_EINVAL, "relocalize_batch: offsets not monotone at scan %d", b);
-        max_points = std::max(max_points, nb);
-    }
-    const int64_t total = offsets[nscans];
-    if (total > 0 && !xy) return fail(m, NDT2D_EINVAL, "relocalize_batch: bad offsets / xy");
+    if ((rc = scans_validate(m, "relocalize_batch", offsets, nscans, &max_points))) return rc;
     DeviceGuard g(m->device);
     const size_t njobs = (size_t)nscans * k;
-    if ((rc = upload(m, m->b_xy, xy, (size_t)total * 8))) return rc;
-    if ((rc = upload(m, m->b_off, offsets, (size_t)(nscans + 1) * 8))) return rc;
-    if ((rc = upload(m, m->b_init, centres, (size_t)nscans * 24))) return rc;
+    if ((rc = upload_scans(m, "relocalize_batch", xy, offsets, nscans, centres, nscans))) return rc;
     CK(m, m->b_tki.ensure(njobs * 8));
     CK(m, m->b_tkv.ensure(njobs * 8));
     CK(m, m->b_res.ensure(njobs * sizeof(ndt2d_result)));
     rc = relocalize_batch_impl(m, level, m->b_xy.as<float>(), m->b_off.as<int64_t>(), nscans, (int)max_points, m->b_init.as<double>(), *win,
                                nhyp, k, m->b_tki.as<int64_t>(), m->b_tkv.as<double>(), m->b_res.as<ndt2d_result>());
     if (rc) return rc;
-    CK(m, cudaMemcpyAsync(best_idx, m->b_tki.p, njobs * 8, cudaMemcpyDeviceToHost, m->cfg.stream));
-    if (best_score) CK(m, cudaMemcpyAsync(best_score, m->b_tkv.p, njobs * 8, cudaMemcpyDeviceToHost, m->cfg.stream));
-    CK(m, cudaMemcpyAsync(res, m->b_res.p, njobs * sizeof(ndt2d_result), cudaMemcpyDeviceToHost, m->cfg.stream));
-    return ndt2d_synchronize(m);        // the one synchronisation of the call
+    return finish_host_call(m, "relocalize_batch", njobs, best_idx, best_score, res, nullptr);
 }
 
 } // extern "C"

@@ -44,6 +44,18 @@ SIGNATURES = {
     "ndt2d_set_target_device": (C.c_int, [_V, _V, C.c_int64]),
     "ndt2d_add_target": (C.c_int, [_V, _V, C.c_int64]),
     "ndt2d_add_target_device": (C.c_int, [_V, _V, C.c_int64]),
+    "ndt2d_set_target_scans": (C.c_int, [_V, _V, _V, C.c_int, _V]),
+    "ndt2d_add_target_scans": (C.c_int, [_V, _V, _V, C.c_int, _V]),
+    "ndt2d_set_target_scans_device": (C.c_int, [_V, _V, _V, C.c_int, C.c_int64, _V]),
+    "ndt2d_add_target_scans_device": (C.c_int, [_V, _V, _V, C.c_int, C.c_int64, _V]),
+    "ndt2d_set_target_ranges": (C.c_int, [_V, _V, C.c_int, C.c_int, C.c_int, C.c_double, C.c_double, C.c_float, C.c_float,
+                                          C.c_float, _V]),
+    "ndt2d_add_target_ranges": (C.c_int, [_V, _V, C.c_int, C.c_int, C.c_int, C.c_double, C.c_double, C.c_float, C.c_float,
+                                          C.c_float, _V]),
+    "ndt2d_set_target_ranges_device": (C.c_int, [_V, _V, C.c_int, C.c_int, C.c_int, C.c_double, C.c_double, C.c_float,
+                                                 C.c_float, C.c_float, _V]),
+    "ndt2d_add_target_ranges_device": (C.c_int, [_V, _V, C.c_int, C.c_int, C.c_int, C.c_double, C.c_double, C.c_float,
+                                                 C.c_float, C.c_float, _V]),
     "ndt2d_level_geometry": (C.c_int, [_V, C.c_int, c_f32p, c_i32p]),
     "ndt2d_get_cells": (C.c_int, [_V, C.c_int, _V]),
     "ndt2d_get_sums": (C.c_int, [_V, C.c_int, _V, _V]),

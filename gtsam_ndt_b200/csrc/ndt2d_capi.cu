@@ -93,18 +93,18 @@ int setup_level(ndt2d_matcher *m, int l, const float bbox[4])
     return install_level(m, l);
 }
 
-int accumulate_and_finalize(ndt2d_matcher *m, const float2 *d_xy, int64_t n)
+int accumulate_and_finalize(ndt2d_matcher *m, const TargetSrc &src)
 {
     if (m->nlevels > 1) {       // a pyramid: all its levels in one accumulate and one finalise launch
         LevelSet S;
         memset(&S, 0, sizeof(S));
         S.nlevels = m->nlevels;
         for (int l = 0; l < m->nlevels; ++l) { S.lv[l] = m->lv[l]; S.cells[l] = m->mem[l].cells; }
-        CK(m, launch_build_levels(m->cfg, S, m->prm, d_xy, n, &m->launches));
+        CK(m, launch_build_levels(m->cfg, S, m->prm, src, &m->launches));
         return NDT2D_OK;
     }
     for (int l = 0; l < m->nlevels; ++l) {
-        CK(m, launch_accumulate(m->cfg, m->lv[l], d_xy, n, &m->launches));
+        CK(m, launch_accumulate(m->cfg, m->lv[l], src, &m->launches));
         CK(m, launch_finalize(m->cfg, m->lv[l], m->mem[l].cells, m->prm, &m->launches));
     }
     return NDT2D_OK;
@@ -373,7 +373,7 @@ void ndt2d_destroy(ndt2d_matcher *m)
     DevBuf *bufs[] = {&m->b_xy, &m->b_off, &m->b_init, &m->b_res, &m->b_pose, &m->b_out, &m->b_cnt, &m->b_idx, &m->b_terms,
                       &m->b_hyp, &m->b_scores, &m->b_tki, &m->b_tkv, &m->b_scratch, &m->b_counter, &m->b_beams, &m->b_ranges,
                       &m->b_box, &m->b_ptab, &m->b_pcnt, &m->b_psums, &m->b_pgeo, &m->b_ptargets, &m->b_ppairs, &m->b_perr, &m->b_reloc,
-                      &m->b_scand, &m->b_sjobs, &m->b_sinit, &m->b_slevels};
+                      &m->b_scand, &m->b_sjobs, &m->b_sinit, &m->b_slevels, &m->b_tpose};
     for (DevBuf *b : bufs) b->release();
     release_relay(m);
     if (m->copy_stream) {
@@ -456,20 +456,42 @@ int ndt2d_set_grid(ndt2d_matcher *m, float ox, float oy, float ex, float ey)
     return NDT2D_OK;
 }
 
-// host_bbox: the caller already knows the bounding box of the finite points (ndt2d_set_target computes it on the host for
-// small targets while the points are still in its hands: no bbox kernel, no read-back, no synchronisation)
-static int set_target_impl(ndt2d_matcher *m, const float *d_xy, int64_t n, const float *host_bbox)
+static TargetSrc point_src(const float *d_xy, int64_t n)
 {
-    if (!m || n < 0 || (n > 0 && !d_xy)) return m ? fail(m, NDT2D_EINVAL, "bad target arguments") : NDT2D_EINVAL;
+    TargetSrc s{};
+    s.xy = reinterpret_cast<const float2 *>(d_xy);
+    s.n = n;
+    return s;
+}
+
+// Posed sources (SPEC 7.2): their per-scan {cos, sin, p0, p1} table, made from the f64 poses on the device
+static int pose_table(ndt2d_matcher *m, TargetSrc &src, const double *d_poses)
+{
+    CK(m, m->b_tpose.ensure((size_t)(src.nscans > 0 ? src.nscans : 1) * 32));
+    CK(m, launch_pose_table(m->cfg, d_poses, src.nscans, m->b_tpose.as<double>(), &m->launches));
+    src.pose = m->b_tpose.as<double>();
+    return NDT2D_OK;
+}
+
+// Build (replace) the target from `src`, after the caller's argument checks. d_poses: the scans' poses on the device (posed
+// sources), nullptr for map-frame points. host_bbox: the caller already knows the bounding box of the finite points
+// (ndt2d_set_target computes it on the host for small targets while the points are still in its hands: no bbox kernel,
+// no read-back, no synchronisation)
+static int set_target_impl(ndt2d_matcher *m, TargetSrc src, const double *d_poses, const float *host_bbox)
+{
     DeviceGuard g(m->device);
     CK(m, cudaStreamSynchronize(m->cfg.stream));
     drop_target(m, /*keep_memory=*/true);
+    if (d_poses) {
+        int rc = pose_table(m, src, d_poses);
+        if (rc) return rc;
+    }
     float bbox[4] = {0, 0, 0, 0};
     if (host_bbox) {
         for (int i = 0; i < 4; ++i) bbox[i] = host_bbox[i];
     } else if (!m->explicit_grid) {
         int box[4];
-        CK(m, launch_bbox(m->cfg, reinterpret_cast<const float2 *>(d_xy), n, m->b_box.as<int>(), &m->launches));
+        CK(m, launch_bbox(m->cfg, src, m->b_box.as<int>(), &m->launches));
         CK(m, cudaMemcpyAsync(box, m->b_box.p, sizeof(box), cudaMemcpyDeviceToHost, m->cfg.stream));
         CK(m, cudaStreamSynchronize(m->cfg.stream));
         for (int i = 0; i < 4; ++i) bbox[i] = bbox_decode(box[i]);
@@ -481,26 +503,29 @@ static int set_target_impl(ndt2d_matcher *m, const float *d_xy, int64_t n, const
             return rc;
         }
     }
-    int rc = accumulate_and_finalize(m, reinterpret_cast<const float2 *>(d_xy), n);
+    int rc = accumulate_and_finalize(m, src);
     if (rc) return rc;
     m->has_target = true;
     m->sums_valid = true;
     return NDT2D_OK;
 }
 
-int ndt2d_set_target_device(ndt2d_matcher *m, const float *d_xy, int64_t n) { return set_target_impl(m, d_xy, n, nullptr); }
-
-int ndt2d_add_target_device(ndt2d_matcher *m, const float *d_xy, int64_t n)
+// Extend the target with `src` (SPEC 7), after the caller's argument checks; without a target, set_target_impl
+static int add_target_impl(ndt2d_matcher *m, TargetSrc src, const double *d_poses)
 {
-    if (!m || n < 0 || (n > 0 && !d_xy)) return m ? fail(m, NDT2D_EINVAL, "bad target arguments") : NDT2D_EINVAL;
-    if (!m->has_target) return ndt2d_set_target_device(m, d_xy, n);
+    if (!m->has_target) return set_target_impl(m, src, d_poses, nullptr);
     if (!m->sums_valid) return fail(m, NDT2D_EINVAL, "target was loaded with ndt2d_set_cells; it has no sums to extend");
     DeviceGuard g(m->device);
+    if (d_poses) {
+        int rc = pose_table(m, src, d_poses);
+        if (rc) return rc;
+    }
     // small additions (a scan into a large map) finalise only the cells they touch; large ones take the dense pass
+    const int64_t n = src.n;
     const int K = m->prm.overlap ? 4 : 1;
     bool sparse = n > 0;
     for (int l = 0; l < m->nlevels; ++l) sparse = sparse && n * K * 8 < (int64_t)m->lv[l].njx * m->lv[l].njy;
-    if (!sparse) return accumulate_and_finalize(m, reinterpret_cast<const float2 *>(d_xy), n);
+    if (!sparse) return accumulate_and_finalize(m, src);
     CK(m, m->b_idx.ensure((size_t)n * K * 4 + 16));
     for (int l = 0; l < m->nlevels; ++l) {
         LevelMem &M = m->mem[l];
@@ -509,10 +534,21 @@ int ndt2d_add_target_device(ndt2d_matcher *m, const float *d_xy, int64_t n)
             CK(m, cudaMemsetAsync(M.dirty, 0, (size_t)M.cap * 4, m->cfg.stream));
         }
         unsigned *list = m->b_idx.as<unsigned>() + 4;
-        CK(m, launch_add_points(m->cfg, m->lv[l], M.cells, m->prm, reinterpret_cast<const float2 *>(d_xy), n, M.dirty, list,
-                                m->b_idx.as<unsigned>(), &m->launches));
+        CK(m, launch_add_points(m->cfg, m->lv[l], M.cells, m->prm, src, M.dirty, list, m->b_idx.as<unsigned>(), &m->launches));
     }
     return NDT2D_OK;
+}
+
+int ndt2d_set_target_device(ndt2d_matcher *m, const float *d_xy, int64_t n)
+{
+    if (!m || n < 0 || (n > 0 && !d_xy)) return m ? fail(m, NDT2D_EINVAL, "bad target arguments") : NDT2D_EINVAL;
+    return set_target_impl(m, point_src(d_xy, n), nullptr, nullptr);
+}
+
+int ndt2d_add_target_device(ndt2d_matcher *m, const float *d_xy, int64_t n)
+{
+    if (!m || n < 0 || (n > 0 && !d_xy)) return m ? fail(m, NDT2D_EINVAL, "bad target arguments") : NDT2D_EINVAL;
+    return add_target_impl(m, point_src(d_xy, n), nullptr);
 }
 
 int ndt2d_set_target(ndt2d_matcher *m, const float *xy, int64_t n)
@@ -533,7 +569,7 @@ int ndt2d_set_target(ndt2d_matcher *m, const float *xy, int64_t n)
             bbox[1] = fminf(bbox[1], y); bbox[3] = fmaxf(bbox[3], y);
         }
     }
-    rc = set_target_impl(m, m->b_xy.as<float>(), n, on_host ? bbox : nullptr);
+    rc = set_target_impl(m, point_src(m->b_xy.as<float>(), n), nullptr, on_host ? bbox : nullptr);
     if (rc) return rc;
     return ndt2d_synchronize(m);
 }
@@ -547,6 +583,129 @@ int ndt2d_add_target(ndt2d_matcher *m, const float *xy, int64_t n)
     rc = ndt2d_add_target_device(m, m->b_xy.as<float>(), n);
     if (rc) return rc;
     return ndt2d_synchronize(m);
+}
+
+// ---- targets from posed scans (SPEC 7.2): one implementation for packed points and LaserScan ranges, host and device
+// buffers, set and add. The checks come first, so a refused call leaves the target as it was.
+
+// packed scans: d_offsets[0..nscans] index d_xy[0..npoints); host: the arrays are host memory (checked, then uploaded)
+static int scans_target(ndt2d_matcher *m, bool add, const float *xy, const int64_t *offsets, int nscans, int64_t npoints,
+                        const double *poses, bool host)
+{
+    if (!m) return NDT2D_EINVAL;
+    if (nscans < 0 || (nscans > 0 && (!offsets || !poses))) return fail(m, NDT2D_EINVAL, "bad arguments");
+    if (host) {
+        if (nscans > 0 && offsets[0] != 0) return fail(m, NDT2D_EINVAL, "offsets[0] = %lld, not 0", (long long)offsets[0]);
+        for (int b = 0; b < nscans; ++b)
+            if (offsets[b + 1] < offsets[b]) return fail(m, NDT2D_EINVAL, "offsets not monotone at scan %d", b);
+        npoints = nscans > 0 ? offsets[nscans] : 0;
+        for (int64_t i = 0; i < 3 * (int64_t)nscans; ++i)
+            if (!std::isfinite(poses[i])) return fail(m, NDT2D_EINVAL, "pose of scan %lld is not finite", (long long)(i / 3));
+    }
+    if (npoints < 0 || (npoints > 0 && (!xy || nscans == 0))) return fail(m, NDT2D_EINVAL, "bad arguments");
+    DeviceGuard g(m->device);
+    if (host) {
+        int rc = upload(m, m->b_xy, xy, (size_t)npoints * 8);
+        if (!rc) rc = upload(m, m->b_off, offsets, nscans > 0 ? (size_t)(nscans + 1) * 8 : 0);
+        if (!rc) rc = upload(m, m->b_pose, poses, (size_t)nscans * 24);
+        if (rc) return rc;
+        xy = m->b_xy.as<float>();
+        offsets = m->b_off.as<int64_t>();
+        poses = m->b_pose.as<double>();
+    }
+    TargetSrc src{};
+    src.xy = reinterpret_cast<const float2 *>(xy);
+    src.n = npoints;
+    src.offsets = offsets;
+    src.nscans = nscans;
+    int rc = add ? add_target_impl(m, src, poses) : set_target_impl(m, src, poses, nullptr);
+    if (rc || !host) return rc;
+    return ndt2d_synchronize(m);
+}
+
+// LaserScan scans (SPEC 8): nscans rows of nbeams ranges
+static int ranges_target(ndt2d_matcher *m, bool add, const void *ranges, int ranges_are_u16, int nscans, int nbeams, double angle_min,
+                         double angle_inc, float range_scale, float range_min, float range_max, const double *poses, bool host)
+{
+    if (!m) return NDT2D_EINVAL;
+    if (nscans < 0 || nbeams < 1 || (nscans > 0 && (!ranges || !poses))) return fail(m, NDT2D_EINVAL, "bad arguments");
+    if (host)
+        for (int64_t i = 0; i < 3 * (int64_t)nscans; ++i)
+            if (!std::isfinite(poses[i])) return fail(m, NDT2D_EINVAL, "pose of scan %lld is not finite", (long long)(i / 3));
+    DeviceGuard g(m->device);
+    int rc = ensure_beams(m, nbeams, angle_min, angle_inc);
+    if (rc) return rc;
+    const size_t bytes = (size_t)nscans * nbeams * (ranges_are_u16 ? 2 : 4);
+    if (host) {
+        rc = upload(m, m->b_ranges, ranges, bytes);
+        if (!rc) rc = upload(m, m->b_pose, poses, (size_t)nscans * 24);
+        if (rc) return rc;
+        ranges = m->b_ranges.p;
+        poses = m->b_pose.as<double>();
+    }
+    TargetSrc src{};
+    src.n = (int64_t)nscans * nbeams;
+    src.nscans = nscans;
+    src.ranges = ranges;
+    src.beams = m->b_beams.as<float2>();
+    src.ranges_u16 = ranges_are_u16 ? 1 : 0;
+    src.nbeams = nbeams;
+    src.range_scale = range_scale; src.range_min = range_min; src.range_max = range_max;
+    rc = add ? add_target_impl(m, src, poses) : set_target_impl(m, src, poses, nullptr);
+    if (rc || !host) return rc;
+    return ndt2d_synchronize(m);
+}
+
+int ndt2d_set_target_scans(ndt2d_matcher *m, const float *xy, const int64_t *offsets, int nscans, const double *poses)
+{
+    return scans_target(m, false, xy, offsets, nscans, 0, poses, true);
+}
+
+int ndt2d_add_target_scans(ndt2d_matcher *m, const float *xy, const int64_t *offsets, int nscans, const double *poses)
+{
+    return scans_target(m, true, xy, offsets, nscans, 0, poses, true);
+}
+
+int ndt2d_set_target_scans_device(ndt2d_matcher *m, const float *d_xy, const int64_t *d_offsets, int nscans, int64_t npoints,
+                                  const double *d_poses)
+{
+    return scans_target(m, false, d_xy, d_offsets, nscans, npoints, d_poses, false);
+}
+
+int ndt2d_add_target_scans_device(ndt2d_matcher *m, const float *d_xy, const int64_t *d_offsets, int nscans, int64_t npoints,
+                                  const double *d_poses)
+{
+    return scans_target(m, true, d_xy, d_offsets, nscans, npoints, d_poses, false);
+}
+
+int ndt2d_set_target_ranges(ndt2d_matcher *m, const void *ranges, int ranges_are_u16, int nscans, int nbeams, double angle_min,
+                            double angle_inc, float range_scale, float range_min, float range_max, const double *poses)
+{
+    return ranges_target(m, false, ranges, ranges_are_u16, nscans, nbeams, angle_min, angle_inc, range_scale, range_min, range_max,
+                         poses, true);
+}
+
+int ndt2d_add_target_ranges(ndt2d_matcher *m, const void *ranges, int ranges_are_u16, int nscans, int nbeams, double angle_min,
+                            double angle_inc, float range_scale, float range_min, float range_max, const double *poses)
+{
+    return ranges_target(m, true, ranges, ranges_are_u16, nscans, nbeams, angle_min, angle_inc, range_scale, range_min, range_max,
+                         poses, true);
+}
+
+int ndt2d_set_target_ranges_device(ndt2d_matcher *m, const void *d_ranges, int ranges_are_u16, int nscans, int nbeams,
+                                   double angle_min, double angle_inc, float range_scale, float range_min, float range_max,
+                                   const double *d_poses)
+{
+    return ranges_target(m, false, d_ranges, ranges_are_u16, nscans, nbeams, angle_min, angle_inc, range_scale, range_min,
+                         range_max, d_poses, false);
+}
+
+int ndt2d_add_target_ranges_device(ndt2d_matcher *m, const void *d_ranges, int ranges_are_u16, int nscans, int nbeams,
+                                   double angle_min, double angle_inc, float range_scale, float range_min, float range_max,
+                                   const double *d_poses)
+{
+    return ranges_target(m, true, d_ranges, ranges_are_u16, nscans, nbeams, angle_min, angle_inc, range_scale, range_min,
+                         range_max, d_poses, false);
 }
 
 int ndt2d_level_geometry(const ndt2d_matcher *m, int level, float geom[5], int32_t dims[4])

@@ -82,12 +82,13 @@ __device__ __forceinline__ bool lattice_of(double fx, double fy, unsigned nhx, u
     return (wx == 0x43380000u) & (wy == 0x43380000u) & (hx < nhx) & (hy < nhy);
 }
 
-// a target point (no pose): f = ((double)X - (double)origin) * inv_st
-__device__ __forceinline__ bool lattice_of_point(const LevelDev &L, float X, float Y, int &hx, int &hy)
+// a target point (no pose): f = (X - (double)origin) * inv_st, X = (double) of an f32 map point or the f64 map coordinate of
+// a posed scan point (SPEC 7.2)
+__device__ __forceinline__ bool lattice_of_point(const LevelDev &L, double X, double Y, int &hx, int &hy)
 {
     unsigned ux, uy;
     float dfx, dfy;
-    const bool in = lattice_of(__dmul_rn(__dsub_rn((double)X, (double)L.ox), L.inv_std), __dmul_rn(__dsub_rn((double)Y, (double)L.oy), L.inv_std),
+    const bool in = lattice_of(__dmul_rn(__dsub_rn(X, (double)L.ox), L.inv_std), __dmul_rn(__dsub_rn(Y, (double)L.oy), L.inv_std),
                                (unsigned)L.nhx, (unsigned)L.nhy, ux, uy, dfx, dfy);
     hx = (int)ux;
     hy = (int)uy;
@@ -130,8 +131,9 @@ __device__ __forceinline__ void finalize_record(unsigned n, long long s0, long l
 // head of each run hands the run's count and five integer sums to `sink(key, count, sx, sy, sxx, sxy, syy)`, key being
 // the table index jy * njx + jx. Integer sums are associative, so any sink (global atomics into the dense table,
 // compare-and-swap into a hash table, ...) gives the cells SPEC 3 defines. Used by k_accumulate and k_pairs_build.
+// (X, Y): the map coordinates in f64 - an f32 point widened, or a posed scan point's unrounded transform (SPEC 7.2).
 template <int OV, class Sink>
-__device__ __forceinline__ void accumulate_window(const LevelDev &L, bool valid, float X, float Y, int lane, Sink sink)
+__device__ __forceinline__ void accumulate_window(const LevelDev &L, bool valid, double X, double Y, int lane, Sink sink)
 {
     constexpr unsigned FULL = 0xffffffffu;
     constexpr int K = OV ? 2 : 1;
@@ -145,7 +147,7 @@ __device__ __forceinline__ void accumulate_window(const LevelDev &L, bool valid,
             const int key = inside ? jy * L.njx + jx : -1;
             const double cx = (double)L.ox + ((double)(jx - L.ov)) * (double)L.st + 0.5 * (double)L.res;
             const double cy = (double)L.oy + ((double)(jy - L.ov)) * (double)L.st + 0.5 * (double)L.res;
-            const double dx = (double)X - cx, dy = (double)Y - cy;
+            const double dx = X - cx, dy = Y - cy;
             const long long qx = inside ? __double2ll_rn(dx * L.qs) : 0;
             const long long qy = inside ? __double2ll_rn(dy * L.qs) : 0;
             int c = inside ? 1 : 0;

@@ -107,7 +107,8 @@ struct ndt2d_matcher {
     ndt2d::DevBuf b_xy, b_off, b_init, b_res, b_pose, b_out, b_cnt, b_idx, b_terms, b_hyp, b_scores, b_tki, b_tkv, b_scratch,
         b_counter, b_beams, b_ranges, b_box, b_ptab, b_pcnt, b_psums, b_pgeo, b_ptargets, b_ppairs, b_perr, b_reloc,
         b_scand, b_sjobs, b_sinit,    // ndt2d_relocalize_pairs / _batch: per-chunk candidates, refinement jobs and their initial poses
-        b_slevels;                    // ndt2d_relocalize_batch: the device copy of lv[] its sweep reads
+        b_slevels,                    // ndt2d_relocalize_batch: the device copy of lv[] its sweep reads
+        b_tpose;                      // targets from posed scans: per scan {cos, sin, p0, p1}
     std::vector<int32_t> h_spairs;  // ndt2d_relocalize_pairs: the host copy its pairs are uploaded from
     int64_t reloc_off[2] = {0, 0}; // source of the asynchronous offsets upload of ndt2d_relocalize_device
     double beams_amin = 0, beams_ainc = 0;

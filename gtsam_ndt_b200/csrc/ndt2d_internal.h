@@ -32,6 +32,20 @@ struct LevelSet {
     int nlevels;
 };
 
+// The points a target is built from, as the build kernels read them (SPEC 3, 7.2): map-frame points (pose == nullptr), or
+// scans with one pose each, as packed points (xy, offsets) or as LaserScan ranges (ranges, beams; SPEC 8).
+struct TargetSrc {
+    const float2 *xy;         // map-frame points, or the packed scan points
+    int64_t n;                // points; nscans * nbeams beams for ranges
+    const double *pose;       // per scan {cos, sin, p0, p1} (launch_pose_table); nullptr: xy are map-frame points
+    const int64_t *offsets;   // packed scans: nscans + 1 entries
+    int nscans;
+    const void *ranges;       // LaserScan ranges: nscans rows of nbeams, f32 or u16
+    const float2 *beams;      // (cb, sb) per beam
+    int ranges_u16, nbeams;
+    float range_scale, range_min, range_max;
+};
+
 struct AlignArgs {
     LevelDev lv[NDT2D_MAX_LEVELS];
     int nlevels;
@@ -68,12 +82,14 @@ struct LaunchCfg {
 };
 
 // all launchers return the cudaError_t of the launch; *launches is incremented per kernel launched
-cudaError_t launch_accumulate(const LaunchCfg &c, const LevelDev &L, const float2 *d_xy, int64_t n, int64_t *launches);
+cudaError_t launch_accumulate(const LaunchCfg &c, const LevelDev &L, const TargetSrc &src, int64_t *launches);
 cudaError_t launch_finalize(const LaunchCfg &c, const LevelDev &L, float4 *cells_out, const ndt2d_params &p, int64_t *launches);
 // accumulate + finalise every level of S from the same points: two launches whatever the number of levels
-cudaError_t launch_build_levels(const LaunchCfg &c, const LevelSet &S, const ndt2d_params &p, const float2 *d_xy, int64_t n, int64_t *launches);
-cudaError_t launch_add_points(const LaunchCfg &c, const LevelDev &L, float4 *cells_out, const ndt2d_params &p, const float2 *d_xy,
-                              int64_t n, unsigned *dirty, unsigned *list, unsigned *nlist, int64_t *launches);
+cudaError_t launch_build_levels(const LaunchCfg &c, const LevelSet &S, const ndt2d_params &p, const TargetSrc &src, int64_t *launches);
+cudaError_t launch_add_points(const LaunchCfg &c, const LevelDev &L, float4 *cells_out, const ndt2d_params &p, const TargetSrc &src,
+                              unsigned *dirty, unsigned *list, unsigned *nlist, int64_t *launches);
+// SPEC 7.2: table[4b..4b+3] = {cos_spec, sin_spec of poses[3b+2], poses[3b], poses[3b+1]} for the posed target sources
+cudaError_t launch_pose_table(const LaunchCfg &c, const double *d_poses, int nscans, double *d_table, int64_t *launches);
 cudaError_t launch_cell_index(const LaunchCfg &c, const LevelDev &L, const float2 *d_xy, int n, const double *d_pose,
                               int32_t *d_idx, int64_t *launches);
 cudaError_t launch_point_terms(const LaunchCfg &c, const LevelDev &L, const float2 *d_xy, int n, const double *d_pose,
@@ -156,8 +172,8 @@ int topk_scratch_words(int sm_count);
 // refinement jobs of a relocalisation: init[j] = hypothesis best_idx[j] widened to f64, job_scan[j] = 0 (or -1 when best_idx[j] < 0)
 cudaError_t launch_topk_to_jobs(const LaunchCfg &c, const float *d_hyp, const int64_t *d_best_idx, int k, double *d_init, int32_t *d_job_scan,
                                 int64_t *launches);
-// finite bounding box of points: d_box[4] = ordered-int encoded {xmin, ymin, xmax, ymax} (see bbox_decode)
-cudaError_t launch_bbox(const LaunchCfg &c, const float2 *d_xy, int64_t n, int *d_box, int64_t *launches);
+// finite bounding box of the target's points (SPEC 2, 7.2): d_box[4] = ordered-int encoded {xmin, ymin, xmax, ymax} (see bbox_decode)
+cudaError_t launch_bbox(const LaunchCfg &c, const TargetSrc &src, int *d_box, int64_t *launches);
 float bbox_decode(int v);
 
 } // namespace ndt2d

@@ -9,6 +9,8 @@
 #include <math.h>
 #include <string.h>
 
+#include <type_traits>
+
 namespace ndt2d {
 
 static constexpr unsigned FULL_MASK = 0xffffffffu;
@@ -17,24 +19,93 @@ static constexpr unsigned FULL_MASK = 0xffffffffu;
 // (1) grid build
 // ------------------------------------------------------------------------------------------------
 
+// Target point sources (TargetSrc): map-frame points, or posed scans as packed points or as LaserScan ranges.
+enum { SRC_POINTS = 0, SRC_SCANS = 1, SRC_RANGES = 2 };
+
+// Point i of the source in f64 map coordinates; false when there is no such point (i >= n, a dropped beam, a non-finite
+// scan coordinate). Map-frame points are widened (SPEC 3); a scan point is transformed by its scan's pose and not rounded
+// (SPEC 7.2). A packed point finds its scan by binary search over offsets[1 .. nscans-1]: whatever the offsets hold, the
+// scan index stays in [0, nscans) and only points below n are read.
+template <int SRC>
+__device__ __forceinline__ bool target_point(const TargetSrc &s, int64_t i, double &X, double &Y)
+{
+    X = Y = 0.0;
+    if (i >= s.n) return false;
+    if (SRC == SRC_POINTS) {
+        const float2 p = __ldg(s.xy + i);
+        X = (double)p.x;
+        Y = (double)p.y;
+        return true;
+    }
+    float x, y;
+    int b;
+    bool ok = true;
+    if (SRC == SRC_SCANS) {
+        const float2 p = __ldg(s.xy + i);
+        x = p.x; y = p.y;
+        int lo = 0, hi = s.nscans - 1;
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (__ldg(s.offsets + mid) <= i) lo = mid;
+            else hi = mid - 1;
+        }
+        b = lo;
+    } else {
+        b = (int)(i / s.nbeams);
+        const int beam = (int)(i - (int64_t)b * s.nbeams);
+        float rho;
+        if (s.ranges_u16) {
+            const unsigned short u = __ldg(reinterpret_cast<const unsigned short *>(s.ranges) + i);
+            rho = __fmul_rn((float)u, s.range_scale);
+            ok = (u != 0);
+        } else {
+            rho = __ldg(reinterpret_cast<const float *>(s.ranges) + i);
+        }
+        ok = ok && (rho >= s.range_min) && (rho <= s.range_max);   // SPEC 8
+        const float2 bt = __ldg(s.beams + beam);
+        x = __fmul_rn(rho, bt.x);
+        y = __fmul_rn(rho, bt.y);
+    }
+    if (!ok || !isfinite(x) || !isfinite(y)) return false;
+    const double *P = s.pose + 4 * (size_t)b;
+    const double cs = __ldg(P), sn = __ldg(P + 1), p0 = __ldg(P + 2), p1 = __ldg(P + 3);
+    const double xd = (double)x, yd = (double)y;
+    X = __fma_rn(cs, xd, __fma_rn(-sn, yd, p0));
+    Y = __fma_rn(sn, xd, __fma_rn(cs, yd, p1));
+    return true;
+}
+
+// the posed sources' per-scan {cos, sin, p0, p1}, sin and cos by SPEC 4.2
+__global__ void k_pose_table(const double *__restrict__ poses, int nscans, double *__restrict__ tab)
+{
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= nscans) return;
+    double sn, cs;
+    sincos_spec(poses[3 * (size_t)b + 2], sn, cs);
+    tab[4 * (size_t)b] = cs;
+    tab[4 * (size_t)b + 1] = sn;
+    tab[4 * (size_t)b + 2] = poses[3 * (size_t)b];
+    tab[4 * (size_t)b + 3] = poses[3 * (size_t)b + 1];
+}
+
 // SPEC 3 accumulation. One point per lane; for each of the K cells of the point, lanes holding the
 // same cell in consecutive positions (laser scans are spatially coherent) are combined with a
 // segmented shuffle reduction and only the head of each run issues the integer atomics. Integer
-// sums are associative, so the result is independent of the order of points, warps and atomics.
+// sums are associative, so the result is independent of the order of points, warps and atomics
+// (a window of packed scan points may straddle two scans).
 // TOUCH (incremental update): the first run head to reach a cell since the last finalisation (an exchange on the cell's
 // dirty word) appends it to `list`, so that the finalisation can visit the touched cells only.
-template <int OV, bool TOUCH>
-__global__ void __launch_bounds__(256) k_accumulate(const LevelDev L, const float2 *__restrict__ xy, int64_t n, unsigned *__restrict__ dirty,
+template <int OV, bool TOUCH, int SRC>
+__global__ void __launch_bounds__(256) k_accumulate(const LevelDev L, const TargetSrc src, unsigned *__restrict__ dirty,
                                                     unsigned *__restrict__ list, unsigned *__restrict__ nlist)
 {
     const int lane = threadIdx.x & 31;
     const int64_t warps_total = (int64_t)gridDim.x * (blockDim.x >> 5);
     const int64_t warp_id = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    for (int64_t base = warp_id * 32; base < n; base += warps_total * 32) {
-        const int64_t i = base + lane;
-        float2 p = make_float2(0.0f, 0.0f);
-        if (i < n) p = __ldg(xy + i);
-        accumulate_window<OV>(L, i < n, p.x, p.y, lane, [&](int key, unsigned c, long long sx, long long sy, long long sxx, long long sxy, long long syy) {
+    for (int64_t base = warp_id * 32; base < src.n; base += warps_total * 32) {
+        double X, Y;
+        const bool valid = target_point<SRC>(src, base + lane, X, Y);
+        accumulate_window<OV>(L, valid, X, Y, lane, [&](int key, unsigned c, long long sx, long long sy, long long sxx, long long sxy, long long syy) {
             if (TOUCH && atomicExch(dirty + key, 1u) == 0u) list[atomicAdd(nlist, 1u)] = (unsigned)key;
             atomicAdd(L.cnt + key, c);
             unsigned long long *s = L.sums + 5 * (size_t)key;
@@ -63,18 +134,17 @@ __global__ void __launch_bounds__(256) k_finalize(const LevelDev L, float4 *__re
 // The same two kernels for every level of a pyramid in one launch each (blockIdx.y = level): a target SCAN's grids are so
 // small that the launches, not the work, were the cost of building them (sequential scan-to-scan odometry builds three
 // levels per step).
-template <int OV>
-__global__ void __launch_bounds__(256) k_accumulate_levels(const __grid_constant__ LevelSet S, const float2 *__restrict__ xy, int64_t n)
+template <int OV, int SRC>
+__global__ void __launch_bounds__(256) k_accumulate_levels(const __grid_constant__ LevelSet S, const TargetSrc src)
 {
     const LevelDev &L = S.lv[blockIdx.y];
     const int lane = threadIdx.x & 31;
     const int64_t warps_total = (int64_t)gridDim.x * (blockDim.x >> 5);
     const int64_t warp_id = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    for (int64_t base = warp_id * 32; base < n; base += warps_total * 32) {
-        const int64_t i = base + lane;
-        float2 p = make_float2(0.0f, 0.0f);
-        if (i < n) p = __ldg(xy + i);
-        accumulate_window<OV>(L, i < n, p.x, p.y, lane, [&](int key, unsigned c, long long sx, long long sy, long long sxx, long long sxy, long long syy) {
+    for (int64_t base = warp_id * 32; base < src.n; base += warps_total * 32) {
+        double X, Y;
+        const bool valid = target_point<SRC>(src, base + lane, X, Y);
+        accumulate_window<OV>(L, valid, X, Y, lane, [&](int key, unsigned c, long long sx, long long sy, long long sxx, long long sxy, long long syy) {
             atomicAdd(L.cnt + key, c);
             unsigned long long *s = L.sums + 5 * (size_t)key;
             atomicAdd(s + 0, (unsigned long long)sx);
@@ -574,40 +644,71 @@ static inline int grid_for(int64_t items, int per_block, int sm_count, int block
     return (int)(need < cap ? need : cap);
 }
 
-cudaError_t launch_accumulate(const LaunchCfg &c, const LevelDev &L, const float2 *d_xy, int64_t n, int64_t *launches)
+// calls f(std::integral_constant<int, SRC>()) for the kind of target source
+template <class F>
+static cudaError_t with_src(const TargetSrc &s, F f)
 {
-    if (n <= 0) return cudaSuccess;
-    int grid = grid_for(n, 256, c.sm_count, 8);
-    if (L.ov) k_accumulate<1, false><<<grid, 256, 0, c.stream>>>(L, d_xy, n, nullptr, nullptr, nullptr);
-    else k_accumulate<0, false><<<grid, 256, 0, c.stream>>>(L, d_xy, n, nullptr, nullptr, nullptr);
+    if (!s.pose) return f(std::integral_constant<int, SRC_POINTS>());
+    if (s.ranges) return f(std::integral_constant<int, SRC_RANGES>());
+    return f(std::integral_constant<int, SRC_SCANS>());
+}
+
+cudaError_t launch_pose_table(const LaunchCfg &c, const double *d_poses, int nscans, double *d_table, int64_t *launches)
+{
+    if (nscans <= 0) return cudaSuccess;
+    k_pose_table<<<(nscans + 127) / 128, 128, 0, c.stream>>>(d_poses, nscans, d_table);
     ++*launches;
     return cudaGetLastError();
 }
 
-// incremental update: accumulate n points and finalise only the cells they touched. dirty: one zeroed word per cell
-// (left zeroed), list: room for n * (ov ? 4 : 1) cell indices, nlist: one word (zeroed here)
-cudaError_t launch_add_points(const LaunchCfg &c, const LevelDev &L, float4 *cells_out, const ndt2d_params &p, const float2 *d_xy,
-                              int64_t n, unsigned *dirty, unsigned *list, unsigned *nlist, int64_t *launches)
+cudaError_t launch_accumulate(const LaunchCfg &c, const LevelDev &L, const TargetSrc &src, int64_t *launches)
 {
+    if (src.n <= 0) return cudaSuccess;
+    int grid = grid_for(src.n, 256, c.sm_count, 8);
+    ++*launches;
+    return with_src(src, [&](auto mode) {
+        constexpr int SRC = decltype(mode)::value;
+        if (L.ov) k_accumulate<1, false, SRC><<<grid, 256, 0, c.stream>>>(L, src, nullptr, nullptr, nullptr);
+        else k_accumulate<0, false, SRC><<<grid, 256, 0, c.stream>>>(L, src, nullptr, nullptr, nullptr);
+        return cudaGetLastError();
+    });
+}
+
+// incremental update: accumulate the source's points and finalise only the cells they touched. dirty: one zeroed word per
+// cell (left zeroed), list: room for src.n * (ov ? 4 : 1) cell indices, nlist: one word (zeroed here)
+cudaError_t launch_add_points(const LaunchCfg &c, const LevelDev &L, float4 *cells_out, const ndt2d_params &p, const TargetSrc &src,
+                              unsigned *dirty, unsigned *list, unsigned *nlist, int64_t *launches)
+{
+    const int64_t n = src.n;
     if (n <= 0) return cudaSuccess;
     cudaError_t e = cudaMemsetAsync(nlist, 0, 4, c.stream);
     if (e != cudaSuccess) return e;
     int grid = grid_for(n, 256, c.sm_count, 8);
-    if (L.ov) k_accumulate<1, true><<<grid, 256, 0, c.stream>>>(L, d_xy, n, dirty, list, nlist);
-    else k_accumulate<0, true><<<grid, 256, 0, c.stream>>>(L, d_xy, n, dirty, list, nlist);
+    e = with_src(src, [&](auto mode) {
+        constexpr int SRC = decltype(mode)::value;
+        if (L.ov) k_accumulate<1, true, SRC><<<grid, 256, 0, c.stream>>>(L, src, dirty, list, nlist);
+        else k_accumulate<0, true, SRC><<<grid, 256, 0, c.stream>>>(L, src, dirty, list, nlist);
+        return cudaGetLastError();
+    });
+    if (e != cudaSuccess) return e;
     k_finalize_list<<<grid_for(n * (L.ov ? 4 : 1), 256, c.sm_count, 8), 256, 0, c.stream>>>(L, cells_out, p.min_points, p.eig_ratio, dirty, list, nlist);
     *launches += 2;
     return cudaGetLastError();
 }
 
-cudaError_t launch_build_levels(const LaunchCfg &c, const LevelSet &S, const ndt2d_params &p, const float2 *d_xy, int64_t n, int64_t *launches)
+cudaError_t launch_build_levels(const LaunchCfg &c, const LevelSet &S, const ndt2d_params &p, const TargetSrc &src, int64_t *launches)
 {
     int64_t max_nc = 1;
     for (int l = 0; l < S.nlevels; ++l) max_nc = std::max<int64_t>(max_nc, (int64_t)S.lv[l].njx * S.lv[l].njy);
-    if (n > 0) {
-        dim3 ga(grid_for(n, 256, c.sm_count, 8), S.nlevels);
-        if (S.lv[0].ov) k_accumulate_levels<1><<<ga, 256, 0, c.stream>>>(S, d_xy, n);
-        else k_accumulate_levels<0><<<ga, 256, 0, c.stream>>>(S, d_xy, n);
+    if (src.n > 0) {
+        dim3 ga(grid_for(src.n, 256, c.sm_count, 8), S.nlevels);
+        cudaError_t e = with_src(src, [&](auto mode) {
+            constexpr int SRC = decltype(mode)::value;
+            if (S.lv[0].ov) k_accumulate_levels<1, SRC><<<ga, 256, 0, c.stream>>>(S, src);
+            else k_accumulate_levels<0, SRC><<<ga, 256, 0, c.stream>>>(S, src);
+            return cudaGetLastError();
+        });
+        if (e != cudaSuccess) return e;
         ++*launches;
     }
     dim3 gf(grid_for(max_nc, 256, c.sm_count, 8), S.nlevels);
@@ -843,15 +944,19 @@ float bbox_decode(int v)
     return f;
 }
 
-// auto-fit (SPEC 2): bounding box of the finite points; min/max are order-independent
-__global__ void __launch_bounds__(256) k_bbox(const float2 *__restrict__ xy, int64_t n, int *__restrict__ box)
+// auto-fit (SPEC 2, 7.2): bounding box of the finite points - of the f32 roundings of a posed scan point's map coordinates;
+// min/max are order-independent
+template <int SRC>
+__global__ void __launch_bounds__(256) k_bbox(const TargetSrc src, int *__restrict__ box)
 {
     float xmin = INFINITY, ymin = INFINITY, xmax = -INFINITY, ymax = -INFINITY;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-        float2 p = __ldg(xy + i);
-        if (!isfinite(p.x) || !isfinite(p.y)) continue;
-        xmin = fminf(xmin, p.x); xmax = fmaxf(xmax, p.x);
-        ymin = fminf(ymin, p.y); ymax = fmaxf(ymax, p.y);
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < src.n; i += (int64_t)gridDim.x * blockDim.x) {
+        double X, Y;
+        if (!target_point<SRC>(src, i, X, Y)) continue;
+        const float x = (float)X, y = (float)Y;
+        if (!isfinite(x) || !isfinite(y)) continue;
+        xmin = fminf(xmin, x); xmax = fmaxf(xmax, x);
+        ymin = fminf(ymin, y); ymax = fmaxf(ymax, y);
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
@@ -868,15 +973,17 @@ __global__ void __launch_bounds__(256) k_bbox(const float2 *__restrict__ xy, int
     }
 }
 
-cudaError_t launch_bbox(const LaunchCfg &c, const float2 *d_xy, int64_t n, int *d_box, int64_t *launches)
+cudaError_t launch_bbox(const LaunchCfg &c, const TargetSrc &src, int *d_box, int64_t *launches)
 {
     int init[4] = {float_to_ordered(INFINITY), float_to_ordered(INFINITY), float_to_ordered(-INFINITY),
                    float_to_ordered(-INFINITY)};
     cudaError_t e = cudaMemcpyAsync(d_box, init, sizeof(init), cudaMemcpyHostToDevice, c.stream);
-    if (e != cudaSuccess || n <= 0) return e;
-    k_bbox<<<grid_for(n, 256 * 4, c.sm_count, 4), 256, 0, c.stream>>>(d_xy, n, d_box);
+    if (e != cudaSuccess || src.n <= 0) return e;
     ++*launches;
-    return cudaGetLastError();
+    return with_src(src, [&](auto mode) {
+        k_bbox<decltype(mode)::value><<<grid_for(src.n, 256 * 4, c.sm_count, 4), 256, 0, c.stream>>>(src, d_box);
+        return cudaGetLastError();
+    });
 }
 
 } // namespace ndt2d

@@ -155,6 +155,59 @@ class NdtMatcher2D:
     def add_target_device(self, d_xy, n):
         self._ck(self._L.ndt2d_add_target_device(self._h, _ptr(d_xy), n))
 
+    def set_target_scans(self, xy, offsets, poses):
+        """Target from packed scans (SPEC.md section 7.2): scan b = xy[offsets[b]:offsets[b+1]] at f64 poses[b] = (tx, ty, theta),
+        transformed into the map frame in f64 inside the build (never rounded to f32)."""
+        self._target_scans(self._L.ndt2d_set_target_scans, xy, offsets, poses)
+
+    def add_target_scans(self, xy, offsets, poses):
+        """add_target of posed scans: equals one set_target_scans of every scan added so far, bit for bit (SPEC 7)."""
+        self._target_scans(self._L.ndt2d_add_target_scans, xy, offsets, poses)
+
+    def _target_scans(self, fn, xy, offsets, poses):
+        xy = np.ascontiguousarray(xy, np.float32).reshape(-1, 2)
+        offsets = np.ascontiguousarray(offsets, np.int64)
+        poses = np.ascontiguousarray(poses, np.float64).reshape(-1, 3)
+        nb = len(offsets) - 1
+        if nb < 0 or len(poses) != nb or (nb and offsets[-1] > len(xy)):
+            raise ValueError("offsets / poses / xy sizes disagree")
+        self._ck(fn(self._h, _ptr(xy), _ptr(offsets), nb, _ptr(poses)))
+
+    def set_target_scans_device(self, d_xy, d_offsets, nscans, npoints, d_poses):
+        self._ck(self._L.ndt2d_set_target_scans_device(self._h, _ptr(d_xy), _ptr(d_offsets), nscans, npoints, _ptr(d_poses)))
+
+    def add_target_scans_device(self, d_xy, d_offsets, nscans, npoints, d_poses):
+        self._ck(self._L.ndt2d_add_target_scans_device(self._h, _ptr(d_xy), _ptr(d_offsets), nscans, npoints, _ptr(d_poses)))
+
+    def set_target_ranges(self, ranges, angle_min, angle_inc, poses, range_scale=0.001, range_min=0.0, range_max=3.0e38):
+        """Target from LaserScan ranges[nscans, nbeams] (float32 metres or uint16 * range_scale, SPEC.md section 8) at f64
+        poses[nscans, 3] (SPEC 7.2)."""
+        self._target_ranges(self._L.ndt2d_set_target_ranges, ranges, angle_min, angle_inc, poses, range_scale, range_min, range_max)
+
+    def add_target_ranges(self, ranges, angle_min, angle_inc, poses, range_scale=0.001, range_min=0.0, range_max=3.0e38):
+        self._target_ranges(self._L.ndt2d_add_target_ranges, ranges, angle_min, angle_inc, poses, range_scale, range_min, range_max)
+
+    def _target_ranges(self, fn, ranges, angle_min, angle_inc, poses, range_scale, range_min, range_max):
+        r = np.ascontiguousarray(ranges)
+        if r.dtype not in (np.float32, np.uint16):
+            r = r.astype(np.float32)
+        r = np.atleast_2d(r)
+        poses = np.ascontiguousarray(poses, np.float64).reshape(-1, 3)
+        if r.ndim != 2 or len(poses) != r.shape[0]:
+            raise ValueError("ranges must be (nscans, nbeams) with one pose per scan")
+        self._ck(fn(self._h, _ptr(r), int(r.dtype == np.uint16), r.shape[0], r.shape[1], angle_min, angle_inc, range_scale,
+                    range_min, range_max, _ptr(poses)))
+
+    def set_target_ranges_device(self, d_ranges, is_u16, nscans, nbeams, angle_min, angle_inc, d_poses, range_scale=0.001,
+                                 range_min=0.0, range_max=3.0e38):
+        self._ck(self._L.ndt2d_set_target_ranges_device(self._h, _ptr(d_ranges), int(is_u16), nscans, nbeams, angle_min, angle_inc,
+                                                        range_scale, range_min, range_max, _ptr(d_poses)))
+
+    def add_target_ranges_device(self, d_ranges, is_u16, nscans, nbeams, angle_min, angle_inc, d_poses, range_scale=0.001,
+                                 range_min=0.0, range_max=3.0e38):
+        self._ck(self._L.ndt2d_add_target_ranges_device(self._h, _ptr(d_ranges), int(is_u16), nscans, nbeams, angle_min, angle_inc,
+                                                        range_scale, range_min, range_max, _ptr(d_poses)))
+
     def geometry(self, level=0):
         g = np.zeros(5, np.float32)
         d = np.zeros(4, np.int32)

@@ -118,6 +118,31 @@ int ndt2d_set_target_device(ndt2d_matcher *m, const float *d_xy, int64_t n);
  * or points inside the current lattice; points outside are ignored. */
 int ndt2d_add_target(ndt2d_matcher *m, const float *xy, int64_t n);
 int ndt2d_add_target_device(ndt2d_matcher *m, const float *d_xy, int64_t n);
+/* target from posed scans (SPEC 7.2): scan b, with pose poses[3b..3b+2] (f64 tx, ty, theta), is transformed into the map
+ * frame in f64 inside the build, never rounded to f32. Packed points: offsets[0..nscans] index xy (offsets[0] = 0,
+ * non-decreasing). LaserScan: nscans rows of nbeams ranges, beams kept as in ndt2d_align_batch_ranges (SPEC 8). With
+ * identity poses the target equals ndt2d_set_target of the concatenated points bit for bit; add equals one set from all
+ * the scans (SPEC 7). The host forms refuse (NDT2D_EINVAL, target untouched) a non-finite pose, nscans < 0, bad offsets
+ * and nbeams < 1, and return after the build; the device forms check no array contents and are asynchronous on the
+ * handle's stream, except that an auto-fitted set reads its bounding box back once. A device offsets table must also end
+ * at npoints; a malformed one gives an unspecified target but no access outside the arrays. Add onto a target loaded
+ * with ndt2d_set_cells is refused; add without a target is set. */
+int ndt2d_set_target_scans(ndt2d_matcher *m, const float *xy, const int64_t *offsets, int nscans, const double *poses);
+int ndt2d_add_target_scans(ndt2d_matcher *m, const float *xy, const int64_t *offsets, int nscans, const double *poses);
+int ndt2d_set_target_scans_device(ndt2d_matcher *m, const float *d_xy, const int64_t *d_offsets, int nscans, int64_t npoints,
+                                  const double *d_poses);
+int ndt2d_add_target_scans_device(ndt2d_matcher *m, const float *d_xy, const int64_t *d_offsets, int nscans, int64_t npoints,
+                                  const double *d_poses);
+int ndt2d_set_target_ranges(ndt2d_matcher *m, const void *ranges, int ranges_are_u16, int nscans, int nbeams, double angle_min,
+                            double angle_inc, float range_scale, float range_min, float range_max, const double *poses);
+int ndt2d_add_target_ranges(ndt2d_matcher *m, const void *ranges, int ranges_are_u16, int nscans, int nbeams, double angle_min,
+                            double angle_inc, float range_scale, float range_min, float range_max, const double *poses);
+int ndt2d_set_target_ranges_device(ndt2d_matcher *m, const void *d_ranges, int ranges_are_u16, int nscans, int nbeams,
+                                   double angle_min, double angle_inc, float range_scale, float range_min, float range_max,
+                                   const double *d_poses);
+int ndt2d_add_target_ranges_device(ndt2d_matcher *m, const void *d_ranges, int ranges_are_u16, int nscans, int nbeams,
+                                   double angle_min, double angle_inc, float range_scale, float range_min, float range_max,
+                                   const double *d_poses);
 /* geom = {res, st, inv_st, ox, oy}; dims = {nhx, nhy, njx, njy} */
 int ndt2d_level_geometry(const ndt2d_matcher *m, int level, float geom[5], int32_t dims[4]);
 /* cell table: njx*njy records of 8 floats {mux, muy, B00, B01, B01, B11, n, valid}; (mux, muy) is the mean RELATIVE TO THE

@@ -94,6 +94,28 @@ class Matcher {
     void addToTarget(const Point2f *pts, std::int64_t n) { ck(ndt2d_add_target(h_, reinterpret_cast<const float *>(pts), n)); }
     void addToTarget(const std::vector<Point2f> &pts) { addToTarget(pts.data(), static_cast<std::int64_t>(pts.size())); }
 
+    // target from posed scans (keyframes at their optimised poses): scan b is points [offsets[b], offsets[b+1]) at poses[b],
+    // transformed into the map frame in f64 inside the build; addScansToTarget equals one setTargetScans of all scans so far
+    void setTargetScans(const std::vector<Point2f> &points, const std::vector<std::int64_t> &offsets, const std::vector<Pose2d> &poses)
+    {
+        targetScans(points, offsets, poses, false);
+    }
+    void addScansToTarget(const std::vector<Point2f> &points, const std::vector<std::int64_t> &offsets, const std::vector<Pose2d> &poses)
+    {
+        targetScans(points, offsets, poses, true);
+    }
+    // the same from LaserScan ranges[nscans * nbeams] in metres, beam i at angle_min + i * angle_inc, scan b at poses[b]
+    void setTargetRanges(const std::vector<float> &ranges, int nbeams, double angle_min, double angle_inc, float range_min,
+                         float range_max, const std::vector<Pose2d> &poses)
+    {
+        targetRanges(ranges, nbeams, angle_min, angle_inc, range_min, range_max, poses, false);
+    }
+    void addRangesToTarget(const std::vector<float> &ranges, int nbeams, double angle_min, double angle_inc, float range_min,
+                           float range_max, const std::vector<Pose2d> &poses)
+    {
+        targetRanges(ranges, nbeams, angle_min, angle_inc, range_min, range_max, poses, true);
+    }
+
     // map files: every level's lattice, the cell records and (withSums) the integer sums behind them, so that addToTarget
     // continues a loaded map bit for bit; loadMap replaces the resolutions, the grid and the target of this matcher
     void saveMap(const std::string &path, bool withSums = true) { ck(ndt2d_save_map(h_, path.c_str(), withSums ? 1 : 0)); }
@@ -293,6 +315,27 @@ class Matcher {
     void ck(int rc) const
     {
         if (rc != NDT2D_OK) throw std::runtime_error(std::string("libndt2d (") + std::to_string(rc) + "): " + ndt2d_last_error(h_));
+    }
+    void targetScans(const std::vector<Point2f> &points, const std::vector<std::int64_t> &offsets, const std::vector<Pose2d> &poses,
+                     bool add)
+    {
+        if (offsets.size() != poses.size() + 1) throw std::invalid_argument("setTargetScans: offsets.size() must be poses.size() + 1");
+        if (offsets.back() < 0 || static_cast<size_t>(offsets.back()) > points.size())
+            throw std::invalid_argument("setTargetScans: offsets overrun points");
+        const float *xy = reinterpret_cast<const float *>(points.data());
+        const double *p = reinterpret_cast<const double *>(poses.data());
+        const int nb = static_cast<int>(poses.size());
+        ck(add ? ndt2d_add_target_scans(h_, xy, offsets.data(), nb, p) : ndt2d_set_target_scans(h_, xy, offsets.data(), nb, p));
+    }
+    void targetRanges(const std::vector<float> &ranges, int nbeams, double angle_min, double angle_inc, float range_min,
+                      float range_max, const std::vector<Pose2d> &poses, bool add)
+    {
+        if (nbeams < 1 || ranges.size() != poses.size() * static_cast<size_t>(nbeams))
+            throw std::invalid_argument("setTargetRanges: ranges.size() must be poses.size() * nbeams");
+        const double *p = reinterpret_cast<const double *>(poses.data());
+        const int nb = static_cast<int>(poses.size());
+        ck(add ? ndt2d_add_target_ranges(h_, ranges.data(), 0, nb, nbeams, angle_min, angle_inc, 1.0f, range_min, range_max, p)
+               : ndt2d_set_target_ranges(h_, ranges.data(), 0, nb, nbeams, angle_min, angle_inc, 1.0f, range_min, range_max, p));
     }
     ndt2d_matcher *h_ = nullptr;
 };

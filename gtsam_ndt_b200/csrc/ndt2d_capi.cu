@@ -38,25 +38,11 @@ void drop_target(ndt2d_matcher *m, bool keep_memory = false)
     m->sums_valid = false;
 }
 
-// the quantities SPEC 2 and 3 derive from a level's cell size and overlap mode
-static void derive_strides(LevelDev &L)
-{
-    L.st = L.ov ? L.res * 0.5f : L.res;
-    L.inv_st = 1.0f / L.st;
-    L.inv_std = 1.0 / (double)L.st;
-    L.qs = 4194304.0 / (double)L.res;
-    L.qu = (double)L.res * (1.0 / 4194304.0);
-}
-
-// device memory of level l for the lattice in m->lv[l] (nhx, nhy set): tables allocated and cleared
+// device memory of level l for the lattice in m->lv[l]: tables allocated and cleared
 static int install_level(ndt2d_matcher *m, int l)
 {
     LevelDev &L = m->lv[l];
-    if (L.nhx < 1 || L.nhy < 1) return fail(m, NDT2D_EINVAL, "level %d: empty lattice (%d x %d)", l, L.nhx, L.nhy);
-    L.njx = L.nhx + L.ov;
-    L.njy = L.nhy + L.ov;
-    int64_t nc = (int64_t)L.njx * L.njy;
-    if (nc >= (int64_t)1 << 31) return fail(m, NDT2D_EINVAL, "level %d: %lld cells exceed 2^31", l, (long long)nc);
+    const int64_t nc = (int64_t)L.njx * L.njy;
     LevelMem &M = m->mem[l];
     const int64_t pad = LevelMem::zero_pad(L.njx);
     CK(m, M.ensure(nc, pad));
@@ -70,43 +56,53 @@ static int install_level(ndt2d_matcher *m, int l)
     return NDT2D_OK;
 }
 
-// SPEC 2: geometry of level l. bbox = {xmin, ymin, xmax, ymax}, used for auto-fit only.
-int setup_level(ndt2d_matcher *m, int l, const float bbox[4])
+// SPEC 2: geometry and tables of every level. bbox = {xmin, ymin, xmax, ymax}, used for auto-fit only. On failure the
+// target is dropped.
+static int setup_levels(ndt2d_matcher *m, const float bbox[4])
 {
-    LevelDev &L = m->lv[l];
-    L = LevelDev{};
-    L.res = m->res[l];
-    L.ov = m->prm.overlap;
-    derive_strides(L);
-    if (m->explicit_grid) {
-        L.ox = m->gox; L.oy = m->goy;
-        L.nhx = (int)ceilf(m->gex / L.st);
-        L.nhy = (int)ceilf(m->gey / L.st);
-    } else {
-        float xmin = bbox[0], ymin = bbox[1], xmax = bbox[2], ymax = bbox[3];
-        if (!(xmin <= xmax)) { xmin = xmax = ymin = ymax = 0.0f; }
-        L.ox = floorf(xmin / L.res) * L.res - L.res;
-        L.oy = floorf(ymin / L.res) * L.res - L.res;
-        L.nhx = (int)ceilf((xmax - L.ox) / L.st) + 2;
-        L.nhy = (int)ceilf((ymax - L.oy) / L.st) + 2;
+    for (int l = 0; l < m->nlevels; ++l) {
+        LevelDev &L = m->lv[l];
+        L = LevelDev{};
+        int rc;
+        if (level_geometry(L, m->res[l], m->prm.overlap, m->explicit_grid, m->gox, m->goy, m->gex, m->gey, bbox[0], bbox[1], bbox[2],
+                           bbox[3]))
+            rc = install_level(m, l);
+        else if (L.nhx < 1 || L.nhy < 1)
+            rc = fail(m, NDT2D_EINVAL, "level %d: empty lattice (%d x %d)", l, L.nhx, L.nhy);
+        else
+            rc = fail(m, NDT2D_EINVAL, "level %d: %lld cells exceed 2^31", l, (long long)L.njx * L.njy);
+        if (rc) {
+            drop_target(m);
+            return rc;
+        }
     }
-    return install_level(m, l);
+    return NDT2D_OK;
 }
 
-int accumulate_and_finalize(ndt2d_matcher *m, const TargetSrc &src)
+// SPEC 3: accumulate src into every level of the target and finalise. touch (incremental update): finalise only the
+// cells the points touch, with one list of them per level in b_idx (after the per-level list lengths)
+static int accumulate_and_finalize(ndt2d_matcher *m, const TargetSrc &src, bool touch = false)
 {
-    if (m->nlevels > 1) {       // a pyramid: all its levels in one accumulate and one finalise launch
-        LevelSet S;
-        memset(&S, 0, sizeof(S));
-        S.nlevels = m->nlevels;
-        for (int l = 0; l < m->nlevels; ++l) { S.lv[l] = m->lv[l]; S.cells[l] = m->mem[l].cells; }
-        CK(m, launch_build_levels(m->cfg, S, m->prm, src, &m->launches));
-        return NDT2D_OK;
+    const int64_t list_cap = src.n * (m->prm.overlap ? 4 : 1);
+    LevelSet S;
+    memset(&S, 0, sizeof(S));
+    S.nlevels = m->nlevels;
+    if (touch) {
+        CK(m, m->b_idx.ensure(((size_t)list_cap * m->nlevels + NDT2D_MAX_LEVELS) * 4));
+        S.nlist = m->b_idx.as<unsigned>();
     }
     for (int l = 0; l < m->nlevels; ++l) {
-        CK(m, launch_accumulate(m->cfg, m->lv[l], src, &m->launches));
-        CK(m, launch_finalize(m->cfg, m->lv[l], m->mem[l].cells, m->prm, &m->launches));
+        LevelMem &M = m->mem[l];
+        if (touch && !M.dirty) {
+            CK(m, cudaMalloc(&M.dirty, (size_t)M.cap * 4));
+            CK(m, cudaMemsetAsync(M.dirty, 0, (size_t)M.cap * 4, m->cfg.stream));
+        }
+        S.lv[l] = m->lv[l];
+        S.cells[l] = M.cells;
+        S.dirty[l] = M.dirty;
+        if (touch) S.list[l] = S.nlist + NDT2D_MAX_LEVELS + l * list_cap;
     }
+    CK(m, launch_build(m->cfg, S, m->prm, src, touch, &m->launches));
     return NDT2D_OK;
 }
 
@@ -496,14 +492,8 @@ static int set_target_impl(ndt2d_matcher *m, TargetSrc src, const double *d_pose
         CK(m, cudaStreamSynchronize(m->cfg.stream));
         for (int i = 0; i < 4; ++i) bbox[i] = bbox_decode(box[i]);
     }
-    for (int l = 0; l < m->nlevels; ++l) {
-        int rc = setup_level(m, l, bbox);
-        if (rc) {
-            drop_target(m);
-            return rc;
-        }
-    }
-    int rc = accumulate_and_finalize(m, src);
+    int rc = setup_levels(m, bbox);
+    if (!rc) rc = accumulate_and_finalize(m, src);
     if (rc) return rc;
     m->has_target = true;
     m->sums_valid = true;
@@ -525,18 +515,7 @@ static int add_target_impl(ndt2d_matcher *m, TargetSrc src, const double *d_pose
     const int K = m->prm.overlap ? 4 : 1;
     bool sparse = n > 0;
     for (int l = 0; l < m->nlevels; ++l) sparse = sparse && n * K * 8 < (int64_t)m->lv[l].njx * m->lv[l].njy;
-    if (!sparse) return accumulate_and_finalize(m, src);
-    CK(m, m->b_idx.ensure((size_t)n * K * 4 + 16));
-    for (int l = 0; l < m->nlevels; ++l) {
-        LevelMem &M = m->mem[l];
-        if (!M.dirty) {
-            CK(m, cudaMalloc(&M.dirty, (size_t)M.cap * 4));
-            CK(m, cudaMemsetAsync(M.dirty, 0, (size_t)M.cap * 4, m->cfg.stream));
-        }
-        unsigned *list = m->b_idx.as<unsigned>() + 4;
-        CK(m, launch_add_points(m->cfg, m->lv[l], M.cells, m->prm, src, M.dirty, list, m->b_idx.as<unsigned>(), &m->launches));
-    }
-    return NDT2D_OK;
+    return accumulate_and_finalize(m, src, sparse);
 }
 
 int ndt2d_set_target_device(ndt2d_matcher *m, const float *d_xy, int64_t n)
@@ -752,14 +731,9 @@ int ndt2d_set_cells(ndt2d_matcher *m, int level, const float *cells, int64_t nre
     DeviceGuard g(m->device);
     if (!m->has_target) {
         if (!m->explicit_grid) return fail(m, NDT2D_EINVAL, "ndt2d_set_cells needs ndt2d_set_grid first");
-        float bbox[4] = {0, 0, 0, 0};
-        for (int l = 0; l < m->nlevels; ++l) {
-            int rc = setup_level(m, l, bbox);
-            if (rc) {
-                drop_target(m);
-                return rc;
-            }
-        }
+        const float bbox[4] = {0, 0, 0, 0};
+        int rc = setup_levels(m, bbox);
+        if (rc) return rc;
         m->has_target = true;
     }
     if (level < 0 || level >= m->nlevels) return fail(m, NDT2D_EINVAL, "level %d out of range", level);
@@ -869,9 +843,9 @@ int ndt2d_load_map(ndt2d_matcher *m, const char *path)
         m->res[l] = lv[l].res;
         LevelDev &L = m->lv[l];
         L = LevelDev{};
-        L.res = lv[l].res; L.ov = h.overlap;
-        derive_strides(L);
-        L.ox = lv[l].ox; L.oy = lv[l].oy; L.nhx = lv[l].nhx; L.nhy = lv[l].nhy;   // the saved lattice, exactly (auto-fitted or explicit)
+        level_strides(L, lv[l].res, h.overlap);
+        L.ox = lv[l].ox; L.oy = lv[l].oy;   // the saved lattice, exactly (auto-fitted or explicit)
+        L.nhx = lv[l].nhx; L.nhy = lv[l].nhy; L.njx = lv[l].njx; L.njy = lv[l].njy;
         rc = install_level(m, l);
         if (rc) break;
         const size_t nc = (size_t)L.njx * L.njy;

@@ -25,10 +25,52 @@ struct LevelDev {
 
 static constexpr unsigned kEmptyKey = 0xffffffffu;
 
-// every level of a target's pyramid, for the kernels that build them in one launch (launch_build_levels)
+// SPEC 2 and 3: the strides and fixed-point scales of a level of cell size res (ov: overlapping cells)
+__host__ __device__ inline void level_strides(LevelDev &L, float res, int ov)
+{
+    L.res = res;
+    L.ov = ov;
+    L.st = ov ? res * 0.5f : res;
+    L.inv_st = 1.0f / L.st;
+    L.inv_std = 1.0 / (double)L.st;
+    L.qs = 4194304.0 / (double)res;
+    L.qu = (double)res * (1.0 / 4194304.0);
+}
+
+// SPEC 2 geometry of a level: its strides, and its lattice on the explicit grid (origin gox, goy; extent gex, gey) or
+// auto-fitted to the bounding box {xmin, ymin, xmax, ymax} of the target's finite points. The host builds and the kernels
+// that build a target scan's grid themselves (ndt2d_pairs.cu) share this one definition, so a pairs result equals
+// set_target(scan) + align. The library is compiled with -fmad=false and -ffp-contract=off: every operation here is the
+// IEEE one on both sides. Returns whether the lattice is usable: not empty, and fewer than 2^31 cells.
+__host__ __device__ inline bool level_geometry(LevelDev &L, float res, int ov, bool explicit_grid, float gox, float goy, float gex,
+                                               float gey, float xmin, float ymin, float xmax, float ymax)
+{
+    level_strides(L, res, ov);
+    if (explicit_grid) {
+        L.ox = gox; L.oy = goy;
+        L.nhx = (int)ceilf(gex / L.st);
+        L.nhy = (int)ceilf(gey / L.st);
+    } else {
+        if (!(xmin <= xmax)) { xmin = xmax = ymin = ymax = 0.0f; }
+        L.ox = floorf(xmin / res) * res - res;
+        L.oy = floorf(ymin / res) * res - res;
+        L.nhx = (int)ceilf((xmax - L.ox) / L.st) + 2;
+        L.nhy = (int)ceilf((ymax - L.oy) / L.st) + 2;
+    }
+    L.njx = L.nhx + ov;
+    L.njy = L.nhy + ov;
+    return L.nhx >= 1 && L.nhy >= 1 && (int64_t)L.njx * L.njy < ((int64_t)1 << 31);
+}
+
+// every level of a target's pyramid, for the build kernels (launch_build): blockIdx.y is the level
 struct LevelSet {
     LevelDev lv[NDT2D_MAX_LEVELS];
     float4 *cells[NDT2D_MAX_LEVELS];   // the writable record tables (LevelDev::cells is the read-only view)
+    // incremental update: per level one word per cell (zero between calls) and the list of the cells touched since the
+    // last finalisation; nlist[l] is its length
+    unsigned *dirty[NDT2D_MAX_LEVELS];
+    unsigned *list[NDT2D_MAX_LEVELS];
+    unsigned *nlist;
     int nlevels;
 };
 
@@ -82,12 +124,10 @@ struct LaunchCfg {
 };
 
 // all launchers return the cudaError_t of the launch; *launches is incremented per kernel launched
-cudaError_t launch_accumulate(const LaunchCfg &c, const LevelDev &L, const TargetSrc &src, int64_t *launches);
-cudaError_t launch_finalize(const LaunchCfg &c, const LevelDev &L, float4 *cells_out, const ndt2d_params &p, int64_t *launches);
-// accumulate + finalise every level of S from the same points: two launches whatever the number of levels
-cudaError_t launch_build_levels(const LaunchCfg &c, const LevelSet &S, const ndt2d_params &p, const TargetSrc &src, int64_t *launches);
-cudaError_t launch_add_points(const LaunchCfg &c, const LevelDev &L, float4 *cells_out, const ndt2d_params &p, const TargetSrc &src,
-                              unsigned *dirty, unsigned *list, unsigned *nlist, int64_t *launches);
+// SPEC 3: accumulate the source's points into every level of S and finalise, one accumulate launch (none without points)
+// and one finalise launch whatever the number of levels. touch (incremental update): finalise only the cells the points
+// touched; S.dirty are zero (and left zero), S.list[l] has room for src.n * (ov ? 4 : 1) cells, S.nlist is zeroed here.
+cudaError_t launch_build(const LaunchCfg &c, const LevelSet &S, const ndt2d_params &p, const TargetSrc &src, bool touch, int64_t *launches);
 // SPEC 7.2: table[4b..4b+3] = {cos_spec, sin_spec of poses[3b+2], poses[3b], poses[3b+1]} for the posed target sources
 cudaError_t launch_pose_table(const LaunchCfg &c, const double *d_poses, int nscans, double *d_table, int64_t *launches);
 cudaError_t launch_cell_index(const LaunchCfg &c, const LevelDev &L, const float2 *d_xy, int n, const double *d_pose,

@@ -88,17 +88,19 @@ __global__ void k_pose_table(const double *__restrict__ poses, int nscans, doubl
     tab[4 * (size_t)b + 3] = poses[3 * (size_t)b + 1];
 }
 
-// SPEC 3 accumulation. One point per lane; for each of the K cells of the point, lanes holding the
-// same cell in consecutive positions (laser scans are spatially coherent) are combined with a
-// segmented shuffle reduction and only the head of each run issues the integer atomics. Integer
-// sums are associative, so the result is independent of the order of points, warps and atomics
-// (a window of packed scan points may straddle two scans).
+// SPEC 3 accumulation into level blockIdx.y of S: every level of a pyramid from the same points in one launch (a target
+// SCAN's grids are so small that the launches, not the work, were the cost of building them; sequential scan-to-scan
+// odometry builds three levels per step). One point per lane; for each of the K cells of the point, lanes holding the
+// same cell in consecutive positions (laser scans are spatially coherent) are combined with a segmented shuffle reduction
+// and only the head of each run issues the integer atomics. Integer sums are associative, so the result is independent
+// of the order of points, warps and atomics (a window of packed scan points may straddle two scans).
 // TOUCH (incremental update): the first run head to reach a cell since the last finalisation (an exchange on the cell's
-// dirty word) appends it to `list`, so that the finalisation can visit the touched cells only.
+// dirty word) appends it to the level's list, so that the finalisation can visit the touched cells only.
 template <int OV, bool TOUCH, int SRC>
-__global__ void __launch_bounds__(256) k_accumulate(const LevelDev L, const TargetSrc src, unsigned *__restrict__ dirty,
-                                                    unsigned *__restrict__ list, unsigned *__restrict__ nlist)
+__global__ void __launch_bounds__(256) k_accumulate(const __grid_constant__ LevelSet S, const TargetSrc src)
 {
+    const int l = blockIdx.y;
+    const LevelDev &L = S.lv[l];
     const int lane = threadIdx.x & 31;
     const int64_t warps_total = (int64_t)gridDim.x * (blockDim.x >> 5);
     const int64_t warp_id = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
@@ -106,7 +108,7 @@ __global__ void __launch_bounds__(256) k_accumulate(const LevelDev L, const Targ
         double X, Y;
         const bool valid = target_point<SRC>(src, base + lane, X, Y);
         accumulate_window<OV>(L, valid, X, Y, lane, [&](int key, unsigned c, long long sx, long long sy, long long sxx, long long sxy, long long syy) {
-            if (TOUCH && atomicExch(dirty + key, 1u) == 0u) list[atomicAdd(nlist, 1u)] = (unsigned)key;
+            if (TOUCH && atomicExch(S.dirty[l] + key, 1u) == 0u) S.list[l][atomicAdd(S.nlist + l, 1u)] = (unsigned)key;
             atomicAdd(L.cnt + key, c);
             unsigned long long *s = L.sums + 5 * (size_t)key;
             atomicAdd(s + 0, (unsigned long long)sx);
@@ -118,72 +120,23 @@ __global__ void __launch_bounds__(256) k_accumulate(const LevelDev L, const Targ
     }
 }
 
-// SPEC 3 finalisation: one thread per cell (the arithmetic is finalize_record() in ndt2d_device.cuh).
-__global__ void __launch_bounds__(256) k_finalize(const LevelDev L, float4 *__restrict__ cells, int min_points, double eig_ratio)
+// SPEC 3 finalisation of level blockIdx.y of S, one thread per cell (the arithmetic is finalize_record() in
+// ndt2d_device.cuh): every cell, or with LIST the cells of the level's touched list, whose dirty words are cleared.
+template <bool LIST>
+__global__ void __launch_bounds__(256) k_finalize(const __grid_constant__ LevelSet S, int min_points, double eig_ratio)
 {
-    const int64_t nc = (int64_t)L.njx * L.njy;
-    for (int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c < nc; c += (int64_t)gridDim.x * blockDim.x) {
+    const int l = blockIdx.y;
+    const LevelDev &L = S.lv[l];
+    float4 *__restrict__ cells = S.cells[l];
+    const int64_t n = LIST ? (int64_t)S.nlist[l] : (int64_t)L.njx * L.njy;
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t c = LIST ? (int64_t)S.list[l][e] : e;
         const long long *s = reinterpret_cast<const long long *>(L.sums) + 5 * c;
         float4 ra, rb;
         finalize_record(L.cnt[c], s[0], s[1], s[2], s[3], s[4], L.qu, min_points, eig_ratio, ra, rb);
         cells[2 * c] = ra;
         cells[2 * c + 1] = rb;
-    }
-}
-
-// The same two kernels for every level of a pyramid in one launch each (blockIdx.y = level): a target SCAN's grids are so
-// small that the launches, not the work, were the cost of building them (sequential scan-to-scan odometry builds three
-// levels per step).
-template <int OV, int SRC>
-__global__ void __launch_bounds__(256) k_accumulate_levels(const __grid_constant__ LevelSet S, const TargetSrc src)
-{
-    const LevelDev &L = S.lv[blockIdx.y];
-    const int lane = threadIdx.x & 31;
-    const int64_t warps_total = (int64_t)gridDim.x * (blockDim.x >> 5);
-    const int64_t warp_id = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    for (int64_t base = warp_id * 32; base < src.n; base += warps_total * 32) {
-        double X, Y;
-        const bool valid = target_point<SRC>(src, base + lane, X, Y);
-        accumulate_window<OV>(L, valid, X, Y, lane, [&](int key, unsigned c, long long sx, long long sy, long long sxx, long long sxy, long long syy) {
-            atomicAdd(L.cnt + key, c);
-            unsigned long long *s = L.sums + 5 * (size_t)key;
-            atomicAdd(s + 0, (unsigned long long)sx);
-            atomicAdd(s + 1, (unsigned long long)sy);
-            atomicAdd(s + 2, (unsigned long long)sxx);
-            atomicAdd(s + 3, (unsigned long long)sxy);
-            atomicAdd(s + 4, (unsigned long long)syy);
-        });
-    }
-}
-
-__global__ void __launch_bounds__(256) k_finalize_levels(const __grid_constant__ LevelSet S, int min_points, double eig_ratio)
-{
-    const LevelDev &L = S.lv[blockIdx.y];
-    float4 *__restrict__ cells = S.cells[blockIdx.y];
-    const int64_t nc = (int64_t)L.njx * L.njy;
-    for (int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c < nc; c += (int64_t)gridDim.x * blockDim.x) {
-        const long long *s = reinterpret_cast<const long long *>(L.sums) + 5 * c;
-        float4 ra, rb;
-        finalize_record(L.cnt[c], s[0], s[1], s[2], s[3], s[4], L.qu, min_points, eig_ratio, ra, rb);
-        cells[2 * c] = ra;
-        cells[2 * c + 1] = rb;
-    }
-}
-
-// Finalisation of the touched cells only (incremental update): the list is consumed and the dirty words are cleared.
-__global__ void __launch_bounds__(256) k_finalize_list(const LevelDev L, float4 *__restrict__ cells, int min_points, double eig_ratio,
-                                                       unsigned *__restrict__ dirty, const unsigned *__restrict__ list,
-                                                       const unsigned *__restrict__ nlist)
-{
-    const unsigned len = *nlist;
-    for (unsigned e = blockIdx.x * blockDim.x + threadIdx.x; e < len; e += gridDim.x * blockDim.x) {
-        const unsigned c = list[e];
-        const long long *s = reinterpret_cast<const long long *>(L.sums) + 5 * (size_t)c;
-        float4 ra, rb;
-        finalize_record(L.cnt[c], s[0], s[1], s[2], s[3], s[4], L.qu, min_points, eig_ratio, ra, rb);
-        cells[2 * (size_t)c] = ra;
-        cells[2 * (size_t)c + 1] = rb;
-        dirty[c] = 0u;
+        if (LIST) S.dirty[l][c] = 0u;
     }
 }
 
@@ -661,66 +614,30 @@ cudaError_t launch_pose_table(const LaunchCfg &c, const double *d_poses, int nsc
     return cudaGetLastError();
 }
 
-cudaError_t launch_accumulate(const LaunchCfg &c, const LevelDev &L, const TargetSrc &src, int64_t *launches)
+cudaError_t launch_build(const LaunchCfg &c, const LevelSet &S, const ndt2d_params &p, const TargetSrc &src, bool touch, int64_t *launches)
 {
-    if (src.n <= 0) return cudaSuccess;
-    int grid = grid_for(src.n, 256, c.sm_count, 8);
-    ++*launches;
-    return with_src(src, [&](auto mode) {
-        constexpr int SRC = decltype(mode)::value;
-        if (L.ov) k_accumulate<1, false, SRC><<<grid, 256, 0, c.stream>>>(L, src, nullptr, nullptr, nullptr);
-        else k_accumulate<0, false, SRC><<<grid, 256, 0, c.stream>>>(L, src, nullptr, nullptr, nullptr);
-        return cudaGetLastError();
-    });
-}
-
-// incremental update: accumulate the source's points and finalise only the cells they touched. dirty: one zeroed word per
-// cell (left zeroed), list: room for src.n * (ov ? 4 : 1) cell indices, nlist: one word (zeroed here)
-cudaError_t launch_add_points(const LaunchCfg &c, const LevelDev &L, float4 *cells_out, const ndt2d_params &p, const TargetSrc &src,
-                              unsigned *dirty, unsigned *list, unsigned *nlist, int64_t *launches)
-{
-    const int64_t n = src.n;
-    if (n <= 0) return cudaSuccess;
-    cudaError_t e = cudaMemsetAsync(nlist, 0, 4, c.stream);
-    if (e != cudaSuccess) return e;
-    int grid = grid_for(n, 256, c.sm_count, 8);
-    e = with_src(src, [&](auto mode) {
-        constexpr int SRC = decltype(mode)::value;
-        if (L.ov) k_accumulate<1, true, SRC><<<grid, 256, 0, c.stream>>>(L, src, dirty, list, nlist);
-        else k_accumulate<0, true, SRC><<<grid, 256, 0, c.stream>>>(L, src, dirty, list, nlist);
-        return cudaGetLastError();
-    });
-    if (e != cudaSuccess) return e;
-    k_finalize_list<<<grid_for(n * (L.ov ? 4 : 1), 256, c.sm_count, 8), 256, 0, c.stream>>>(L, cells_out, p.min_points, p.eig_ratio, dirty, list, nlist);
-    *launches += 2;
-    return cudaGetLastError();
-}
-
-cudaError_t launch_build_levels(const LaunchCfg &c, const LevelSet &S, const ndt2d_params &p, const TargetSrc &src, int64_t *launches)
-{
-    int64_t max_nc = 1;
-    for (int l = 0; l < S.nlevels; ++l) max_nc = std::max<int64_t>(max_nc, (int64_t)S.lv[l].njx * S.lv[l].njy);
+    if (touch) {
+        cudaError_t e = cudaMemsetAsync(S.nlist, 0, (size_t)S.nlevels * sizeof(unsigned), c.stream);
+        if (e != cudaSuccess) return e;
+    }
     if (src.n > 0) {
-        dim3 ga(grid_for(src.n, 256, c.sm_count, 8), S.nlevels);
+        const dim3 grid(grid_for(src.n, 256, c.sm_count, 8), S.nlevels);
         cudaError_t e = with_src(src, [&](auto mode) {
             constexpr int SRC = decltype(mode)::value;
-            if (S.lv[0].ov) k_accumulate_levels<1, SRC><<<ga, 256, 0, c.stream>>>(S, src);
-            else k_accumulate_levels<0, SRC><<<ga, 256, 0, c.stream>>>(S, src);
+            auto kern = S.lv[0].ov ? (touch ? k_accumulate<1, true, SRC> : k_accumulate<1, false, SRC>)
+                                   : (touch ? k_accumulate<0, true, SRC> : k_accumulate<0, false, SRC>);
+            kern<<<grid, 256, 0, c.stream>>>(S, src);
             return cudaGetLastError();
         });
         if (e != cudaSuccess) return e;
         ++*launches;
     }
-    dim3 gf(grid_for(max_nc, 256, c.sm_count, 8), S.nlevels);
-    k_finalize_levels<<<gf, 256, 0, c.stream>>>(S, p.min_points, p.eig_ratio);
-    ++*launches;
-    return cudaGetLastError();
-}
-
-cudaError_t launch_finalize(const LaunchCfg &c, const LevelDev &L, float4 *cells_out, const ndt2d_params &p, int64_t *launches)
-{
-    int grid = grid_for((int64_t)L.njx * L.njy, 256, c.sm_count, 8);
-    k_finalize<<<grid, 256, 0, c.stream>>>(L, cells_out, p.min_points, p.eig_ratio);
+    // as many threads as touched cells at most (K per point), or as cells in the largest level
+    int64_t items = 1;
+    if (touch) items = src.n * (S.lv[0].ov ? 4 : 1);
+    else for (int l = 0; l < S.nlevels; ++l) items = std::max<int64_t>(items, (int64_t)S.lv[l].njx * S.lv[l].njy);
+    auto fin = touch ? k_finalize<true> : k_finalize<false>;
+    fin<<<dim3(grid_for(items, 256, c.sm_count, 8), S.nlevels), 256, 0, c.stream>>>(S, p.min_points, p.eig_ratio);
     ++*launches;
     return cudaGetLastError();
 }

@@ -14,37 +14,6 @@ static constexpr unsigned FULL_MASK = 0xffffffffu;
 // the cells of its bounding box, so the cells live in an open-addressing hash table keyed by the dense cell index.
 static constexpr int PAIRS_LIST_CAP = 2304; // claimed-slot list per warp (u16 entries, 36 KB per block); longer: full-table scan
 
-// SPEC 2 geometry of one level of a target's grid from its bounding box: the f32 expressions of setup_level() in
-// ndt2d_capi.cu (every lane computes the same values). Returns false when the lattice is unusable (empty or >= 2^31
-// cells): nothing is inside then and every align against this target ends NO_OVERLAP.
-__device__ __forceinline__ bool pair_level_geometry(LevelDev &L, float res, int ov, bool explicit_grid, float gox, float goy, float gex,
-                                                    float gey, float xmin, float ymin, float xmax, float ymax)
-{
-    L.res = res;
-    L.ov = ov;
-    L.st = L.ov ? __fmul_rn(L.res, 0.5f) : L.res;
-    L.inv_st = __fdiv_rn(1.0f, L.st);
-    if (explicit_grid) {
-        L.ox = gox; L.oy = goy;
-        L.nhx = (int)ceilf(__fdiv_rn(gex, L.st));
-        L.nhy = (int)ceilf(__fdiv_rn(gey, L.st));
-    } else {
-        if (!(xmin <= xmax)) { xmin = xmax = ymin = ymax = 0.0f; }
-        L.ox = __fsub_rn(__fmul_rn(floorf(__fdiv_rn(xmin, L.res)), L.res), L.res);
-        L.oy = __fsub_rn(__fmul_rn(floorf(__fdiv_rn(ymin, L.res)), L.res), L.res);
-        L.nhx = (int)ceilf(__fdiv_rn(__fsub_rn(xmax, L.ox), L.st)) + 2;
-        L.nhy = (int)ceilf(__fdiv_rn(__fsub_rn(ymax, L.oy), L.st)) + 2;
-    }
-    const bool bad = L.nhx < 1 || L.nhy < 1 || (int64_t)(L.nhx + L.ov) * (int64_t)(L.nhy + L.ov) >= ((int64_t)1 << 31);
-    if (bad) { L.nhx = L.nhy = 0; }
-    L.njx = L.nhx + L.ov;
-    L.njy = L.nhy + L.ov;
-    L.inv_std = __ddiv_rn(1.0, (double)L.st);
-    L.qs = __ddiv_rn(4194304.0, (double)L.res);
-    L.qu = __dmul_rn((double)L.res, 1.0 / 4194304.0);
-    return !bad;
-}
-
 template <int OV>
 __global__ void __launch_bounds__(256) k_pairs_build(const PairBuildArgs a)
 {
@@ -80,7 +49,9 @@ __global__ void __launch_bounds__(256) k_pairs_build(const PairBuildArgs a)
         }
     }
     LevelDev L;
-    const bool too_big = !pair_level_geometry(L, a.res[l], a.ov, a.explicit_grid != 0, a.gox, a.goy, a.gex, a.gey, xmin, ymin, xmax, ymax);
+    // an unusable lattice (empty or >= 2^31 cells) is reported and left empty: every align against this target ends NO_OVERLAP
+    const bool too_big = !level_geometry(L, a.res[l], a.ov, a.explicit_grid != 0, a.gox, a.goy, a.gex, a.gey, xmin, ymin, xmax, ymax);
+    if (too_big) { L.nhx = L.nhy = 0; L.njx = L.njy = L.ov; }
     L.hash_mask = a.cap - 1u;
     float4 *rec = a.tab + (size_t)wid * ((size_t)a.cap + 1) * 2;
     uint32_t *cnt = a.cnt + (size_t)wid * a.cap;
@@ -450,7 +421,8 @@ __global__ void __launch_bounds__(FUSED_WARPS_MAX * 32) k_pairs_fused(const __gr
         int evals = 0, status = NDT2D_NO_OVERLAP;
         for (int l = 0; l < a.nlevels; ++l) {
             LevelDev L;
-            const bool usable = pair_level_geometry(L, a.res_m[l], 0, a.explicit_grid != 0, a.gox, a.goy, a.gex, a.gey, xmin, ymin, xmax, ymax);
+            const bool usable = level_geometry(L, a.res_m[l], 0, a.explicit_grid != 0, a.gox, a.goy, a.gex, a.gey, xmin, ymin, xmax, ymax);
+            if (!usable) L.nhx = L.nhy = L.njx = L.njy = 0;  // as k_pairs_build: the target is reported, the pair ends NO_OVERLAP
             L.cells = reinterpret_cast<const float4 *>(rec); // TABLE_SHASH: the compact array of 24-byte records
             L.cnt = hidx;                                    //              and the bucket index
             L.sums = nullptr;
@@ -641,7 +613,8 @@ __global__ void __launch_bounds__(SEARCH_WARPS * 32, 3) k_search_sweep(const __g
                 float xmin = INFINITY, ymin = INFINITY, xmax = -INFINITY, ymax = -INFINITY;
                 if (!a.explicit_grid) target_bbox(tsrc, tn, lane, xmin, ymin, xmax, ymax);
                 LevelDev L;
-                const bool usable = pair_level_geometry(L, a.res_m, 0, a.explicit_grid != 0, a.gox, a.goy, a.gex, a.gey, xmin, ymin, xmax, ymax);
+                const bool usable = level_geometry(L, a.res_m, 0, a.explicit_grid != 0, a.gox, a.goy, a.gex, a.gey, xmin, ymin, xmax, ymax);
+                if (!usable) L.nhx = L.nhy = L.njx = L.njy = 0;   // as k_pairs_build
                 float *rec = reinterpret_cast<float *>(area + a.off_r);
                 unsigned *hidx = reinterpret_cast<unsigned *>(area + a.off_h);
                 L.cells = reinterpret_cast<const float4 *>(rec);

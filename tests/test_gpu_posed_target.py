@@ -321,3 +321,13 @@ def test_launches_per_call(data):
     n0 = m.kernel_launches
     m.set_target_scans(xy, off, data["poses"])
     assert m.kernel_launches - n0 == 3          # explicit grid: no bounding box
+    # a scan added to a large map finalises only the cells it touches: one accumulate and one finalise launch for all levels
+    scan = data["pts_of"](data["r32"][:1], False)[0]
+    for res in ([2.0, 1.0, 0.5], [0.5]):
+        m = g.NdtMatcher2D(res)
+        m.set_grid(-200.0, -200.0, 400.0, 400.0)
+        m.set_target(xy)
+        assert all(len(scan) * 8 < m.geometry(l)["njx"] * m.geometry(l)["njy"] for l in range(len(res)))   # the sparse path
+        n0 = m.kernel_launches
+        m.add_target(scan)
+        assert m.kernel_launches - n0 == 2, res

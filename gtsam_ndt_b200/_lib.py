@@ -79,6 +79,12 @@ SIGNATURES = {
     "ndt2d_relocalize_pairs": (C.c_int, [_V, C.c_int, _V, _V, C.c_int, _V, C.c_int, _V, C.POINTER(Window), C.c_int, _V, _V, _V]),
     "ndt2d_relocalize_pairs_device": (C.c_int, [_V, C.c_int, _V, _V, _V, C.c_int, _V, C.c_int, _V, C.POINTER(Window), C.c_int,
                                                 _V, _V, _V]),
+    "ndt2d_align_submaps": (C.c_int, [_V, _V, _V, C.c_int, _V, C.c_int, _V, _V, _V, C.c_int, _V, _V]),
+    "ndt2d_align_submaps_device": (C.c_int, [_V, _V, _V, _V, C.c_int, _V, C.c_int, _V, _V, _V, C.c_int, _V, _V]),
+    "ndt2d_relocalize_submaps": (C.c_int, [_V, C.c_int, _V, _V, C.c_int, _V, C.c_int, _V, _V, _V, C.c_int, _V, C.POINTER(Window),
+                                           C.c_int, _V, _V, _V]),
+    "ndt2d_relocalize_submaps_device": (C.c_int, [_V, C.c_int, _V, _V, _V, C.c_int, _V, C.c_int, _V, _V, _V, C.c_int, _V,
+                                                  C.POINTER(Window), C.c_int, _V, _V, _V]),
     "ndt2d_relocalize_batch": (C.c_int, [_V, C.c_int, _V, _V, C.c_int, _V, C.POINTER(Window), C.c_int, _V, _V, _V]),
     "ndt2d_relocalize_batch_device": (C.c_int, [_V, C.c_int, _V, _V, C.c_int, C.c_int, _V, C.POINTER(Window), C.c_int, _V, _V, _V]),
     "ndt2d_sweep":(C.c_int, [_V, C.c_int, _V, C.c_int, _V, C.c_int64, _V, C.c_int, _V, _V]),

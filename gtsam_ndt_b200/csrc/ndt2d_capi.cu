@@ -369,7 +369,8 @@ void ndt2d_destroy(ndt2d_matcher *m)
     DevBuf *bufs[] = {&m->b_xy, &m->b_off, &m->b_init, &m->b_res, &m->b_pose, &m->b_out, &m->b_cnt, &m->b_idx, &m->b_terms,
                       &m->b_hyp, &m->b_scores, &m->b_tki, &m->b_tkv, &m->b_scratch, &m->b_counter, &m->b_beams, &m->b_ranges,
                       &m->b_box, &m->b_ptab, &m->b_pcnt, &m->b_psums, &m->b_pgeo, &m->b_ptargets, &m->b_ppairs, &m->b_perr, &m->b_reloc,
-                      &m->b_scand, &m->b_sjobs, &m->b_sinit, &m->b_slevels, &m->b_tpose};
+                      &m->b_scand, &m->b_sjobs, &m->b_sinit, &m->b_slevels, &m->b_tpose, &m->b_sm_off, &m->b_sm_start,
+                      &m->b_sm_base, &m->b_sm_pose, &m->b_sm_tab};
     for (DevBuf *b : bufs) b->release();
     release_relay(m);
     if (m->copy_stream) {

@@ -95,6 +95,17 @@ __device__ __forceinline__ bool lattice_of_point(const LevelDev &L, double X, do
     return in;
 }
 
+// SPEC 7.2: the f64 map coordinates of the finite scan point (x, y) under its scan's pose P = {cos, sin, p0, p1}
+// (launch_pose_table), never rounded to f32. Every build from posed scans (k_accumulate, k_bbox, k_submap_build) goes
+// through here.
+__device__ __forceinline__ void posed_point(const double *__restrict__ P, float x, float y, double &X, double &Y)
+{
+    const double cs = __ldg(P), sn = __ldg(P + 1), p0 = __ldg(P + 2), p1 = __ldg(P + 3);
+    const double xd = (double)x, yd = (double)y;
+    X = __fma_rn(cs, xd, __fma_rn(-sn, yd, p0));
+    Y = __fma_rn(sn, xd, __fma_rn(cs, yd, p1));
+}
+
 // ---- SPEC 3: finalisation of one cell from its integer sums; f64, operations in the order the spec lists ----
 __device__ __forceinline__ void finalize_record(unsigned n, long long s0, long long s1, long long s2, long long s3, long long s4,
                                                 double U, int min_points, double eig_ratio, float4 &ra, float4 &rb)

@@ -108,8 +108,10 @@ struct ndt2d_matcher {
         b_counter, b_beams, b_ranges, b_box, b_ptab, b_pcnt, b_psums, b_pgeo, b_ptargets, b_ppairs, b_perr, b_reloc,
         b_scand, b_sjobs, b_sinit,    // ndt2d_relocalize_pairs / _batch: per-chunk candidates, refinement jobs and their initial poses
         b_slevels,                    // ndt2d_relocalize_batch: the device copy of lv[] its sweep reads
-        b_tpose;                      // targets from posed scans: per scan {cos, sin, p0, p1}
+        b_tpose,                      // targets from posed scans: per scan {cos, sin, p0, p1}
+        b_sm_off, b_sm_start, b_sm_base, b_sm_pose, b_sm_tab;   // calls over submaps: their SubmapDev tables and member poses
     std::vector<int32_t> h_spairs;  // ndt2d_relocalize_pairs: the host copy its pairs are uploaded from
+    std::vector<int64_t> h_sm_start, h_sm_base;   // calls over submaps: the host copies of SubmapDev::start and ::base
     int64_t reloc_off[2] = {0, 0}; // source of the asynchronous offsets upload of ndt2d_relocalize_device
     double beams_amin = 0, beams_ainc = 0;
     int beams_n = 0;

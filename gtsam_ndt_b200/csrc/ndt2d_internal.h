@@ -159,6 +159,19 @@ struct PairBuildArgs {
 };
 cudaError_t launch_pairs_build(const LaunchCfg &c, const PairBuildArgs &a, int64_t *launches);
 
+// The submaps of a call over submaps (SPEC 7.3): submap g is members [offsets[g], offsets[g + 1]); member e is points
+// [base[e], base[e] + start[e + 1] - start[e]) of the packed batch at pose table entry e. start numbers the points of all
+// members in a row, so a submap's points are the flat indices [start[e0], start[e1]) of its members [e0, e1).
+struct SubmapDev {
+    const int64_t *offsets;  // nsubmaps + 1
+    const int64_t *start;    // nmembers + 1
+    const int64_t *base;     // nmembers
+    const double *pose;      // nmembers * {cos, sin, p0, p1} (launch_pose_table)
+};
+// One BLOCK per (submap, level) builds the hash table k_pairs_build would build from the submap's posed points: the same
+// tables and geometry (a.targets holds submap ids; a.offsets is not read), so k_align and k_search_sweep read them unchanged.
+cudaError_t launch_submap_build(const LaunchCfg &c, const PairBuildArgs &a, const SubmapDev &s, int64_t *launches);
+
 // Batched scan-to-scan, fused path (K = 1, scans small enough for shared memory): one warp per PAIR builds the target's
 // grid for one pyramid level in its own shared-memory slice (radix sort of the cell keys, one lane per cell for the sums
 // and the finalisation, compact record array behind a tagged u32 hash index), aligns the source on it, and goes on to the next

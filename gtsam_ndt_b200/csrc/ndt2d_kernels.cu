@@ -67,11 +67,7 @@ __device__ __forceinline__ bool target_point(const TargetSrc &s, int64_t i, doub
         y = __fmul_rn(rho, bt.y);
     }
     if (!ok || !isfinite(x) || !isfinite(y)) return false;
-    const double *P = s.pose + 4 * (size_t)b;
-    const double cs = __ldg(P), sn = __ldg(P + 1), p0 = __ldg(P + 2), p1 = __ldg(P + 3);
-    const double xd = (double)x, yd = (double)y;
-    X = __fma_rn(cs, xd, __fma_rn(-sn, yd, p0));
-    Y = __fma_rn(sn, xd, __fma_rn(cs, yd, p1));
+    posed_point(s.pose + 4 * (size_t)b, x, y, X, Y);
     return true;
 }
 

@@ -504,6 +504,165 @@ cudaError_t launch_pairs_build(const LaunchCfg &c, const PairBuildArgs &a, int64
 }
 
 // ------------------------------------------------------------------------------------------------
+// submaps (SPEC 7.3): the target of a pair is several posed scans
+// ------------------------------------------------------------------------------------------------
+
+static constexpr int SUBMAP_THREADS = 256;
+static constexpr int SUBMAP_LIST_CAP = 16384;   // claimed-slot list per block (u16 entries, 32 KB); longer: full-table scan
+
+// Point q (flat index, in [start[e0], start[e1])) of the submap whose members are [e0, e1), in f64 map coordinates (SPEC 7.2);
+// false for a non-finite scan point. The member is found by binary search over start[e0 .. e1-1]; the last member whose
+// start is <= q holds the point, so empty members are skipped.
+__device__ __forceinline__ bool submap_point(const float2 *__restrict__ xy, const SubmapDev &s, int e0, int e1, int64_t q, double &X,
+                                             double &Y)
+{
+    int lo = e0, hi = e1 - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (__ldg(s.start + mid) <= q) lo = mid;
+        else hi = mid - 1;
+    }
+    const float2 p = __ldg(xy + __ldg(s.base + lo) + (q - __ldg(s.start + lo)));
+    X = Y = 0.0;
+    if (!isfinite(p.x) || !isfinite(p.y)) return false;
+    posed_point(s.pose + 4 * (size_t)lo, p.x, p.y, X, Y);
+    return true;
+}
+
+// k_pairs_build for a submap of up to 43 690 points: one block per (submap slot, level), its eight warps striding over the
+// submap's points. SPEC 2 auto-fit box of the ((float)Xd, (float)Yd) roundings (a block reduction, as k_bbox for
+// set_target_scans), the level's lattice by level_geometry, SPEC 3 accumulation into the slot's hash table (claim by
+// compare-and-swap, as k_pairs_build) and, after a block barrier, the finalisation of the slots the block claimed.
+// (The minimum of one block per SM lifts ptxas's register target: without it the OV = 1 form spilled at 64 registers.)
+template <int OV>
+__global__ void __launch_bounds__(SUBMAP_THREADS, 1) k_submap_build(const __grid_constant__ PairBuildArgs a, const __grid_constant__ SubmapDev s)
+{
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int wid = blockIdx.x;
+    const int t = wid / a.nlevels, l = wid % a.nlevels;
+    __shared__ unsigned short s_list[SUBMAP_LIST_CAP];
+    __shared__ int s_nlist;
+    __shared__ float s_box[4][SUBMAP_THREADS / 32];
+    const int g = __ldg(a.targets + t);
+    const int e0 = (int)__ldg(s.offsets + g), e1 = (int)__ldg(s.offsets + g + 1);
+    const int64_t q0 = __ldg(s.start + e0);
+    const int n = (int)(__ldg(s.start + e1) - q0);
+
+    float xmin = INFINITY, ymin = INFINITY, xmax = -INFINITY, ymax = -INFINITY;
+    if (!a.explicit_grid) {
+        for (int i = threadIdx.x; i < n; i += SUBMAP_THREADS) {
+            double X, Y;
+            if (!submap_point(a.xy, s, e0, e1, q0 + i, X, Y)) continue;
+            const float x = (float)X, y = (float)Y;
+            if (!isfinite(x) || !isfinite(y)) continue;
+            xmin = fminf(xmin, x); xmax = fmaxf(xmax, x);
+            ymin = fminf(ymin, y); ymax = fmaxf(ymax, y);
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            xmin = fminf(xmin, __shfl_xor_sync(FULL_MASK, xmin, o));
+            ymin = fminf(ymin, __shfl_xor_sync(FULL_MASK, ymin, o));
+            xmax = fmaxf(xmax, __shfl_xor_sync(FULL_MASK, xmax, o));
+            ymax = fmaxf(ymax, __shfl_xor_sync(FULL_MASK, ymax, o));
+        }
+        if (lane == 0) { s_box[0][warp] = xmin; s_box[1][warp] = ymin; s_box[2][warp] = xmax; s_box[3][warp] = ymax; }
+        __syncthreads();
+#pragma unroll
+        for (int w = 0; w < SUBMAP_THREADS / 32; ++w) {
+            xmin = fminf(xmin, s_box[0][w]); ymin = fminf(ymin, s_box[1][w]);
+            xmax = fmaxf(xmax, s_box[2][w]); ymax = fmaxf(ymax, s_box[3][w]);
+        }
+    }
+    LevelDev L;
+    // an unusable lattice is reported and left empty, as by k_pairs_build: every pair against this submap ends NO_OVERLAP
+    const bool too_big = !level_geometry(L, a.res[l], a.ov, a.explicit_grid != 0, a.gox, a.goy, a.gex, a.gey, xmin, ymin, xmax, ymax);
+    if (too_big) { L.nhx = L.nhy = 0; L.njx = L.njy = L.ov; }
+    L.hash_mask = a.cap - 1u;
+    float4 *rec = a.tab + (size_t)wid * ((size_t)a.cap + 1) * 2;
+    uint32_t *cnt = a.cnt + (size_t)wid * a.cap;
+    unsigned long long *sums = a.sums + (size_t)wid * a.cap * 5;
+    L.cells = rec;
+    L.cnt = cnt;
+    L.sums = sums;
+    if (threadIdx.x == 0) {
+        a.geo[wid] = L;
+        s_nlist = 0;
+        if (too_big) atomicMax(a.error, t + 1);
+    }
+    const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
+    const float4 empty = make_float4(0.f, 0.f, __int_as_float((int)kEmptyKey), 0.f);
+    for (unsigned sl = threadIdx.x; sl <= a.cap; sl += SUBMAP_THREADS) {
+        rec[2 * (size_t)sl] = zero;
+        rec[2 * (size_t)sl + 1] = sl < a.cap ? empty : zero;
+    }
+    __syncthreads();
+
+    unsigned *keyword = reinterpret_cast<unsigned *>(rec);   // key of slot s = word 8 s + 6
+    for (int base = warp * 32; base < n; base += SUBMAP_THREADS) {
+        const int i = base + lane;
+        double X = 0.0, Y = 0.0;
+        const bool valid = i < n && submap_point(a.xy, s, e0, e1, q0 + i, X, Y);
+        accumulate_window<OV>(L, valid, X, Y, lane, [&](int key, unsigned c, long long sx, long long sy, long long sxx, long long sxy, long long syy) {
+            unsigned sl = hash_slot((unsigned)key, L.hash_mask);
+            bool placed = false;
+            for (unsigned probes = 0; probes <= L.hash_mask; ++probes) {
+                unsigned was = atomicCAS(keyword + 8 * (size_t)sl + 6, kEmptyKey, (unsigned)key);
+                if (was == kEmptyKey) {
+                    const int pos = atomicAdd(&s_nlist, 1);
+                    if (pos < SUBMAP_LIST_CAP) s_list[pos] = (unsigned short)sl;
+                    placed = true;
+                    break;
+                }
+                if (was == (unsigned)key) { placed = true; break; }
+                sl = (sl + 1u) & L.hash_mask;
+            }
+            if (!placed) { atomicMax(a.error, t + 1); return; }
+            atomicAdd(cnt + sl, c);
+            unsigned long long *q = sums + 5 * (size_t)sl;
+            atomicAdd(q + 0, (unsigned long long)sx);
+            atomicAdd(q + 1, (unsigned long long)sy);
+            atomicAdd(q + 2, (unsigned long long)sxx);
+            atomicAdd(q + 3, (unsigned long long)sxy);
+            atomicAdd(q + 4, (unsigned long long)syy);
+        });
+    }
+    __threadfence();
+    __syncthreads();
+
+    // SPEC 3 finalisation of the claimed slots, as k_pairs_build's
+    auto finish = [&](unsigned sl) {
+        const unsigned key = *(volatile unsigned *)(keyword + 8 * (size_t)sl + 6);
+        if (key == kEmptyKey) return;
+        const unsigned nn = *(volatile uint32_t *)(cnt + sl);
+        volatile long long *q = reinterpret_cast<volatile long long *>(sums + 5 * (size_t)sl);
+        const long long q0_ = q[0], q1 = q[1], q2 = q[2], q3 = q[3], q4 = q[4];
+        float4 ra, rb;
+        finalize_record(nn, q0_, q1, q2, q3, q4, L.qu, a.min_points, a.eig_ratio, ra, rb);
+        rb.z = __int_as_float((int)key);
+        rec[2 * (size_t)sl] = ra;
+        rec[2 * (size_t)sl + 1] = rb;
+        cnt[sl] = 0u;
+        q[0] = 0; q[1] = 0; q[2] = 0; q[3] = 0; q[4] = 0;
+    };
+    const int nlist = s_nlist;
+    if (nlist <= SUBMAP_LIST_CAP) {
+        for (int e = threadIdx.x; e < nlist; e += SUBMAP_THREADS) finish(s_list[e]);
+    } else {
+        for (unsigned sl = threadIdx.x; sl < a.cap; sl += SUBMAP_THREADS) finish(sl);
+    }
+}
+
+cudaError_t launch_submap_build(const LaunchCfg &c, const PairBuildArgs &a, const SubmapDev &s, int64_t *launches)
+{
+    const int64_t blocks = (int64_t)a.ntargets * a.nlevels;
+    if (blocks <= 0) return cudaSuccess;
+    if (a.ov) k_submap_build<1><<<(int)blocks, SUBMAP_THREADS, 0, c.stream>>>(a, s);
+    else k_submap_build<0><<<(int)blocks, SUBMAP_THREADS, 0, c.stream>>>(a, s);
+    ++*launches;
+    return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------------------------------------
 // windowed search over pairs (ndt2d_relocalize_pairs, SPEC 6.1): k_search_sweep scores every window hypothesis of every pair
 // and keeps the k best per (pair, hypothesis chunk); k_search_topk merges a pair's chunks into its exact top-k and turns it
 // into refinement jobs, which k_pairs_fused (shared-memory tables) or k_align in pairs mode (per-target hash tables) align.
@@ -831,26 +990,28 @@ static unsigned next_pow2(unsigned v)
     return p;
 }
 
-// General path (overlapping grids, long scans): per-target hash tables in global memory, built by k_pairs_build for chunks of
-// consecutive pairs whose distinct targets fit the table budget (NDT2D_PAIRS_BYTES, default 8 GB). For chunk [p0, p1),
-// run(p0, p1) finds the chunk's pairs as (target slot, source scan) in b_ppairs and the tables' geometry in b_pgeo.
+// General path (overlapping grids, long scans, submaps): per-target hash tables in global memory, built for chunks of
+// consecutive pairs whose distinct targets fit the table budget (NDT2D_PAIRS_BYTES, default 8 GB). A pair's target id
+// is a scan of the packed batch (sub == nullptr; tables by k_pairs_build) or a submap of *sub (k_submap_build); ntargets
+// is the number of ids and max_tgt the most points of any target a pair names. For chunk [p0, p1), run(p0, p1) finds the
+// chunk's pairs as (target slot, source scan) in b_ppairs and the tables' geometry in b_pgeo.
 template <class Run>
-static int pairs_general(ndt2d_matcher *m, const char *name, const float *d_xy, const int64_t *d_offsets, int nscans, const int32_t *pairs,
-                         int npairs, int64_t max_tgt, Run run)
+static int pairs_general(ndt2d_matcher *m, const char *name, const float *d_xy, const int64_t *d_offsets, int ntargets, const int32_t *pairs,
+                         int npairs, int64_t max_tgt, const SubmapDev *sub, Run run)
 {
     const int K = m->prm.overlap ? 4 : 1, L = m->nlevels;
     // slots per table: 1.5 x the most cells a target can occupy (every point in cells of its own), rounded up to a power
     // of two: at most 2/3 full in that worst case, typically a quarter (a 1080-beam scan occupies ~500 cells)
     const uint64_t want = 3ull * (uint64_t)std::max<int64_t>(max_tgt, 16) * K / 2;
-    if (want > 65536) return fail(m, NDT2D_EINVAL, "%s: target scans of %lld points need more than 65536 table slots", name,
-                                  (long long)max_tgt);
+    if (want > 65536) return fail(m, NDT2D_EINVAL, "%s: %s of %lld points need more than 65536 table slots", name,
+                                  sub ? "submaps" : "target scans", (long long)max_tgt);
     const unsigned cap = next_pow2((unsigned)want);
     const size_t per_target = (size_t)L * (((size_t)cap + 1) * 32 + (size_t)cap * 44 + sizeof(LevelDev));
     size_t budget = (size_t)8 << 30;
     if (const char *e = getenv("NDT2D_PAIRS_BYTES")) budget = (size_t)strtoull(e, nullptr, 10);
-    const int tmax = (int)std::max<size_t>(1, std::min<size_t>(budget / per_target, (size_t)nscans));
+    const int tmax = (int)std::max<size_t>(1, std::min<size_t>(budget / per_target, (size_t)ntargets));
     int rc;
-    std::vector<int32_t> slot((size_t)nscans, -1), targets, resolved;
+    std::vector<int32_t> slot((size_t)ntargets, -1), targets, resolved;
     int p0 = 0;
     while (p0 < npairs) {
         // the next chunk: pairs in order until the chunk's distinct targets would exceed the budget
@@ -894,7 +1055,8 @@ static int pairs_general(ndt2d_matcher *m, const char *name, const float *d_xy, 
         b.tab = m->b_ptab.as<float4>(); b.cnt = m->b_pcnt.as<uint32_t>(); b.sums = m->b_psums.as<unsigned long long>();
         b.geo = m->b_pgeo.as<LevelDev>();
         b.error = m->b_perr.as<int>();
-        CK(m, launch_pairs_build(m->cfg, b, &m->launches));
+        if (sub) CK(m, launch_submap_build(m->cfg, b, *sub, &m->launches));
+        else CK(m, launch_pairs_build(m->cfg, b, &m->launches));
         if ((rc = run(p0, p1))) return rc;
         for (int32_t t : targets) slot[t] = -1;
         p0 = p1;
@@ -953,9 +1115,9 @@ static int upload_scans(ndt2d_matcher *m, const char *name, const float *xy, con
 }
 
 // End of a host-buffer call: copies best_idx and best_score (when given) and the n records back, synchronises once and
-// reports the device error flag d_error (nullptr: the call has none).
+// reports the device error flag d_error (nullptr: the call has none) for a target of kind `what` ("target scan", "submap").
 static int finish_host_call(ndt2d_matcher *m, const char *name, size_t n, int64_t *best_idx, double *best_score, ndt2d_result *res,
-                            const int *d_error)
+                            const int *d_error, const char *what = "target scan")
 {
     if (best_idx) CK(m, cudaMemcpyAsync(best_idx, m->b_tki.p, n * 8, cudaMemcpyDeviceToHost, m->cfg.stream));
     if (best_score) CK(m, cudaMemcpyAsync(best_score, m->b_tkv.p, n * 8, cudaMemcpyDeviceToHost, m->cfg.stream));
@@ -964,8 +1126,8 @@ static int finish_host_call(ndt2d_matcher *m, const char *name, size_t n, int64_
     if (d_error) CK(m, cudaMemcpyAsync(&err, d_error, 4, cudaMemcpyDeviceToHost, m->cfg.stream));
     int rc = ndt2d_synchronize(m);
     if (rc) return rc;
-    if (err) return fail(m, NDT2D_EINVAL, "%s: the auto-fitted lattice of a target scan exceeds 2^31 cells "
-                                          "(a point far from the rest?); its pairs were returned with status NO_OVERLAP", name);
+    if (err) return fail(m, NDT2D_EINVAL, "%s: the auto-fitted lattice of a %s exceeds 2^31 cells "
+                                          "(a point far from the rest?); its pairs were returned with status NO_OVERLAP", name, what);
     return NDT2D_OK;
 }
 
@@ -991,13 +1153,15 @@ static bool pairs_fused_setup(ndt2d_matcher *m, int64_t max_tgt, int64_t max_src
 // d_xy / d_offsets / d_init / d_res: device; pairs: host (the chunking and the target list are host work). One chunk = as
 // many pairs as fit the table budget. Asynchronous on the handle's stream apart from the uploads of `pairs` (shared-memory
 // path) or of the small per-chunk index lists (general path); a target whose lattice exceeds 2^31 cells sets b_perr.
-static int align_pairs_impl(ndt2d_matcher *m, const float *d_xy, const int64_t *d_offsets, int nscans, const int32_t *pairs, int npairs,
-                            int64_t max_tgt, int64_t max_src, const double *d_init, ndt2d_result *d_res)
+// sub: the pairs' targets are submaps (always the general path), and ntargets counts them; otherwise it counts the scans.
+static int align_pairs_impl(ndt2d_matcher *m, const char *name, const float *d_xy, const int64_t *d_offsets, int ntargets,
+                            const int32_t *pairs, int npairs, int64_t max_tgt, int64_t max_src, const double *d_init, ndt2d_result *d_res,
+                            const SubmapDev *sub = nullptr)
 {
     CK(m, m->b_perr.ensure(4));
     CK(m, cudaMemsetAsync(m->b_perr.p, 0, 4, m->cfg.stream));
     PairFusedArgs f;
-    if (pairs_fused_setup(m, max_tgt, max_src, f)) {
+    if (!sub && pairs_fused_setup(m, max_tgt, max_src, f)) {
         int rc;
         if ((rc = upload(m, m->b_ppairs, pairs, (size_t)npairs * 8))) return rc;
         CK(m, cudaStreamSynchronize(m->cfg.stream));     // `pairs` is the caller's buffer
@@ -1010,7 +1174,7 @@ static int align_pairs_impl(ndt2d_matcher *m, const float *d_xy, const int64_t *
         CK(m, launch_pairs_fused(m->cfg, f, &m->launches));
         return NDT2D_OK;
     }
-    return pairs_general(m, "align_pairs", d_xy, d_offsets, nscans, pairs, npairs, max_tgt, [&](int p0, int p1) {
+    return pairs_general(m, name, d_xy, d_offsets, ntargets, pairs, npairs, max_tgt, sub, [&](int p0, int p1) {
         AlignArgs a{};
         a.xy = reinterpret_cast<const float2 *>(d_xy);
         a.offsets = d_offsets;
@@ -1033,7 +1197,7 @@ int ndt2d_align_pairs_device(ndt2d_matcher *m, const float *d_xy, const int64_t 
     if (npairs == 0) return NDT2D_OK;
     if (!d_offsets || !d_init || !d_res) return fail(m, NDT2D_EINVAL, "bad arguments");
     DeviceGuard g(m->device);
-    return align_pairs_impl(m, d_xy, d_offsets, nscans, pairs, npairs, max_tgt, max_src, d_init, d_res);
+    return align_pairs_impl(m, "align_pairs", d_xy, d_offsets, nscans, pairs, npairs, max_tgt, max_src, d_init, d_res);
 }
 
 int ndt2d_align_pairs(ndt2d_matcher *m, const float *xy, const int64_t *offsets, int nscans, const int32_t *pairs, int npairs,
@@ -1048,8 +1212,8 @@ int ndt2d_align_pairs(ndt2d_matcher *m, const float *xy, const int64_t *offsets,
     DeviceGuard g(m->device);
     if ((rc = upload_scans(m, "align_pairs", xy, offsets, nscans, init, npairs))) return rc;
     CK(m, m->b_res.ensure((size_t)npairs * sizeof(ndt2d_result)));
-    rc = align_pairs_impl(m, m->b_xy.as<float>(), m->b_off.as<int64_t>(), nscans, pairs, npairs, max_tgt, max_src, m->b_init.as<double>(),
-                          m->b_res.as<ndt2d_result>());
+    rc = align_pairs_impl(m, "align_pairs", m->b_xy.as<float>(), m->b_off.as<int64_t>(), nscans, pairs, npairs, max_tgt, max_src,
+                          m->b_init.as<double>(), m->b_res.as<ndt2d_result>());
     if (rc) return rc;
     return finish_host_call(m, "align_pairs", (size_t)npairs, nullptr, nullptr, res, m->b_perr.as<int>());
 }
@@ -1113,10 +1277,12 @@ static int relocalize_pairs_validate(ndt2d_matcher *m, int level, const int64_t 
 
 // Shared-memory path (as ndt2d_align_pairs, when k_search_sweep can also stage the longest source): sweep, top-k, refinement
 // by k_pairs_fused and the empty slots: four launches whatever the number of pairs. General path: per chunk of the per-target
-// tables, the table build, the same sweep and top-k on the tables, k_align in pairs mode and the empty slots.
-static int relocalize_pairs_impl(ndt2d_matcher *m, int level, const float *d_xy, const int64_t *d_offsets, int nscans, const int32_t *pairs,
-                                 int npairs, int64_t max_tgt, int64_t max_src, const double *d_centres, const ndt2d_window &win,
-                                 long long nhyp, int k, int64_t *d_best_idx, double *d_best_score, ndt2d_result *d_res)
+// tables, the table build, the same sweep and top-k on the tables, k_align in pairs mode and the empty slots. sub and
+// ntargets: as for align_pairs_impl.
+static int relocalize_pairs_impl(ndt2d_matcher *m, const char *name, int level, const float *d_xy, const int64_t *d_offsets, int ntargets,
+                                 const int32_t *pairs, int npairs, int64_t max_tgt, int64_t max_src, const double *d_centres,
+                                 const ndt2d_window &win, long long nhyp, int k, int64_t *d_best_idx, double *d_best_score,
+                                 ndt2d_result *d_res, const SubmapDev *sub = nullptr)
 {
     const size_t njobs = (size_t)npairs * k;
     CK(m, m->b_perr.ensure(4));
@@ -1129,7 +1295,7 @@ static int relocalize_pairs_impl(ndt2d_matcher *m, int level, const float *d_xy,
     PairFusedArgs f;
     bool staged = false;
     size_t smem = 0;
-    if (pairs_fused_setup(m, max_tgt, max_src, f) && (smem = search_layout(s, &f, max_src, m->cfg.max_smem_optin, staged), staged)) {
+    if (!sub && pairs_fused_setup(m, max_tgt, max_src, f) && (smem = search_layout(s, &f, max_src, m->cfg.max_smem_optin, staged), staged)) {
         // `pairs` is the caller's buffer: it is uploaded from a copy, so that nothing waits for the copy to finish
         m->h_spairs.assign(pairs, pairs + 2 * (size_t)npairs);
         if ((rc = upload(m, m->b_ppairs, m->h_spairs.data(), (size_t)npairs * 8))) return rc;
@@ -1149,7 +1315,7 @@ static int relocalize_pairs_impl(ndt2d_matcher *m, int level, const float *d_xy,
         return NDT2D_OK;
     }
     smem = search_layout(s, nullptr, max_src, m->cfg.max_smem_optin, staged);
-    return pairs_general(m, "relocalize_pairs", d_xy, d_offsets, nscans, pairs, npairs, max_tgt, [&](int p0, int p1) -> int {
+    return pairs_general(m, name, d_xy, d_offsets, ntargets, pairs, npairs, max_tgt, sub, [&](int p0, int p1) -> int {
         const size_t j0 = (size_t)p0 * k, nj = (size_t)(p1 - p0) * k;
         s.pairs = m->b_ppairs.as<int32_t>();
         s.geo = m->b_pgeo.as<LevelDev>();
@@ -1185,8 +1351,8 @@ int ndt2d_relocalize_pairs_device(ndt2d_matcher *m, int level, const float *d_xy
     if (npairs == 0) return NDT2D_OK;
     if (!d_offsets || !d_centres || !d_best_idx || !d_res) return fail(m, NDT2D_EINVAL, "bad arguments");
     DeviceGuard g(m->device);
-    return relocalize_pairs_impl(m, level, d_xy, d_offsets, nscans, pairs, npairs, max_tgt, max_src, d_centres, *win, nhyp, k, d_best_idx,
-                                 d_best_score, d_res);
+    return relocalize_pairs_impl(m, "relocalize_pairs", level, d_xy, d_offsets, nscans, pairs, npairs, max_tgt, max_src, d_centres, *win,
+                                 nhyp, k, d_best_idx, d_best_score, d_res);
 }
 
 int ndt2d_relocalize_pairs(ndt2d_matcher *m, int level, const float *xy, const int64_t *offsets, int nscans, const int32_t *pairs,
@@ -1206,10 +1372,177 @@ int ndt2d_relocalize_pairs(ndt2d_matcher *m, int level, const float *xy, const i
     CK(m, m->b_tki.ensure(njobs * 8));
     CK(m, m->b_tkv.ensure(njobs * 8));
     CK(m, m->b_res.ensure(njobs * sizeof(ndt2d_result)));
-    rc = relocalize_pairs_impl(m, level, m->b_xy.as<float>(), m->b_off.as<int64_t>(), nscans, pairs, npairs, max_tgt, max_src,
-                               m->b_init.as<double>(), *win, nhyp, k, m->b_tki.as<int64_t>(), m->b_tkv.as<double>(), m->b_res.as<ndt2d_result>());
+    rc = relocalize_pairs_impl(m, "relocalize_pairs", level, m->b_xy.as<float>(), m->b_off.as<int64_t>(), nscans, pairs, npairs, max_tgt,
+                               max_src, m->b_init.as<double>(), *win, nhyp, k, m->b_tki.as<int64_t>(), m->b_tkv.as<double>(),
+                               m->b_res.as<ndt2d_result>());
     if (rc) return rc;
     return finish_host_call(m, "relocalize_pairs", njobs, best_idx, best_score, res, m->b_perr.as<int>());
+}
+
+// ---- pairs against submaps of posed scans (SPEC 7.3): ndt2d_set_target_scans(members) + align / relocalize per pair ----
+
+// The scans, the submaps and the (submap, source scan) pairs of a call over submaps. host_poses: the member poses are host
+// memory and are checked finite (the device forms pass nullptr and false). *max_tgt: the most points of any submap a pair
+// names; *max_src: the longest source. Leaves each member's first flat point index and first point in xy in
+// m->h_sm_start / m->h_sm_base, for submaps_setup.
+static int submaps_validate(ndt2d_matcher *m, const char *name, const int64_t *offsets, int nscans, const int64_t *submap_offsets,
+                            int nsubmaps, const int32_t *member_scans, const double *poses, bool host_poses, const int32_t *pairs,
+                            int npairs, int64_t *max_tgt, int64_t *max_src)
+{
+    if (nscans < 0 || nsubmaps < 0 || npairs < 0 || (nscans > 0 && !offsets) || !submap_offsets || (npairs > 0 && !pairs))
+        return fail(m, NDT2D_EINVAL, "%s: bad arguments", name);
+    if (m->nlevels < 1) return fail(m, NDT2D_EINVAL, "%s: no resolution set", name);
+    int rc = scans_validate(m, name, offsets, nscans, nullptr);
+    if (rc) return rc;
+    if (submap_offsets[0] != 0) return fail(m, NDT2D_EINVAL, "%s: submap_offsets[0] = %lld, not 0", name, (long long)submap_offsets[0]);
+    for (int g = 0; g < nsubmaps; ++g)
+        if (submap_offsets[g + 1] < submap_offsets[g] || submap_offsets[g + 1] > 0x7fffffff)
+            return fail(m, NDT2D_EINVAL, "%s: submap offsets not monotone at submap %d", name, g);
+    const int64_t nmembers = submap_offsets[nsubmaps];
+    if (nmembers > 0 && (!member_scans || (host_poses && !poses))) return fail(m, NDT2D_EINVAL, "%s: bad arguments", name);
+    m->h_sm_start.resize((size_t)nmembers + 1);
+    m->h_sm_base.resize((size_t)nmembers);
+    int64_t flat = 0;
+    for (int64_t e = 0; e < nmembers; ++e) {
+        const int32_t b = member_scans[e];
+        if (b < 0 || b >= nscans) return fail(m, NDT2D_EINVAL, "%s: member %lld: scan index %d out of range", name, (long long)e, b);
+        if (host_poses && (!std::isfinite(poses[3 * e]) || !std::isfinite(poses[3 * e + 1]) || !std::isfinite(poses[3 * e + 2])))
+            return fail(m, NDT2D_EINVAL, "%s: pose of member %lld is not finite", name, (long long)e);
+        m->h_sm_start[(size_t)e] = flat;
+        m->h_sm_base[(size_t)e] = offsets[b];
+        flat += offsets[b + 1] - offsets[b];
+    }
+    m->h_sm_start[(size_t)nmembers] = flat;
+    *max_tgt = *max_src = 0;
+    for (int p = 0; p < npairs; ++p) {
+        const int g = pairs[2 * p], s = pairs[2 * p + 1];
+        if (g < 0 || g >= nsubmaps) return fail(m, NDT2D_EINVAL, "%s: pair %d: submap index out of range", name, p);
+        if (s < 0 || s >= nscans) return fail(m, NDT2D_EINVAL, "%s: pair %d: scan index out of range", name, p);
+        *max_tgt = std::max(*max_tgt, m->h_sm_start[(size_t)submap_offsets[g + 1]] - m->h_sm_start[(size_t)submap_offsets[g]]);
+        *max_src = std::max(*max_src, offsets[s + 1] - offsets[s]);
+    }
+    return NDT2D_OK;
+}
+
+// Uploads the submap offsets and the tables submaps_validate left on the host, and makes the members' pose table from the
+// f64 poses on the device (one launch): *sub is then what k_submap_build reads.
+static int submaps_setup(ndt2d_matcher *m, const int64_t *submap_offsets, int nsubmaps, const double *d_poses, SubmapDev *sub)
+{
+    const size_t nmembers = m->h_sm_base.size();
+    int rc;
+    if ((rc = upload(m, m->b_sm_off, submap_offsets, ((size_t)nsubmaps + 1) * 8))) return rc;
+    if ((rc = upload(m, m->b_sm_start, m->h_sm_start.data(), (nmembers + 1) * 8))) return rc;
+    if ((rc = upload(m, m->b_sm_base, m->h_sm_base.data(), nmembers * 8))) return rc;
+    CK(m, m->b_sm_tab.ensure(std::max<size_t>(nmembers, 1) * 32));
+    CK(m, launch_pose_table(m->cfg, d_poses, (int)nmembers, m->b_sm_tab.as<double>(), &m->launches));
+    sub->offsets = m->b_sm_off.as<int64_t>();
+    sub->start = m->b_sm_start.as<int64_t>();
+    sub->base = m->b_sm_base.as<int64_t>();
+    sub->pose = m->b_sm_tab.as<double>();
+    return NDT2D_OK;
+}
+
+int ndt2d_align_submaps_device(ndt2d_matcher *m, const float *d_xy, const int64_t *d_offsets, const int64_t *offsets, int nscans,
+                               const int64_t *submap_offsets, int nsubmaps, const int32_t *member_scans, const double *d_member_poses,
+                               const int32_t *pairs, int npairs, const double *d_init, ndt2d_result *d_res)
+{
+    if (!m) return NDT2D_EINVAL;
+    int64_t max_tgt = 0, max_src = 0;
+    int rc = submaps_validate(m, "align_submaps", offsets, nscans, submap_offsets, nsubmaps, member_scans, nullptr, false, pairs, npairs,
+                              &max_tgt, &max_src);
+    if (rc) return rc;
+    if (npairs == 0) return NDT2D_OK;
+    if (!d_offsets || !d_init || !d_res || (!m->h_sm_base.empty() && !d_member_poses))
+        return fail(m, NDT2D_EINVAL, "align_submaps: bad arguments");
+    DeviceGuard g(m->device);
+    SubmapDev sub;
+    if ((rc = submaps_setup(m, submap_offsets, nsubmaps, d_member_poses, &sub))) return rc;
+    return align_pairs_impl(m, "align_submaps", d_xy, d_offsets, nsubmaps, pairs, npairs, max_tgt, max_src, d_init, d_res, &sub);
+}
+
+int ndt2d_align_submaps(ndt2d_matcher *m, const float *xy, const int64_t *offsets, int nscans, const int64_t *submap_offsets, int nsubmaps,
+                        const int32_t *member_scans, const double *member_poses, const int32_t *pairs, int npairs, const double *init,
+                        ndt2d_result *res)
+{
+    if (!m) return NDT2D_EINVAL;
+    int64_t max_tgt = 0, max_src = 0;
+    int rc = submaps_validate(m, "align_submaps", offsets, nscans, submap_offsets, nsubmaps, member_scans, member_poses, true, pairs,
+                              npairs, &max_tgt, &max_src);
+    if (rc) return rc;
+    if (npairs == 0) return NDT2D_OK;
+    if (!init || !res) return fail(m, NDT2D_EINVAL, "align_submaps: bad arguments");
+    DeviceGuard g(m->device);
+    if ((rc = upload_scans(m, "align_submaps", xy, offsets, nscans, init, npairs))) return rc;
+    if ((rc = upload(m, m->b_sm_pose, member_poses, m->h_sm_base.size() * 24))) return rc;
+    CK(m, m->b_res.ensure((size_t)npairs * sizeof(ndt2d_result)));
+    SubmapDev sub;
+    if ((rc = submaps_setup(m, submap_offsets, nsubmaps, m->b_sm_pose.as<double>(), &sub))) return rc;
+    rc = align_pairs_impl(m, "align_submaps", m->b_xy.as<float>(), m->b_off.as<int64_t>(), nsubmaps, pairs, npairs, max_tgt, max_src,
+                          m->b_init.as<double>(), m->b_res.as<ndt2d_result>(), &sub);
+    if (rc) return rc;
+    return finish_host_call(m, "align_submaps", (size_t)npairs, nullptr, nullptr, res, m->b_perr.as<int>(), "submap");
+}
+
+static int relocalize_submaps_validate(ndt2d_matcher *m, int level, const int64_t *offsets, int nscans, const int64_t *submap_offsets,
+                                       int nsubmaps, const int32_t *member_scans, const double *poses, bool host_poses, const int32_t *pairs,
+                                       int npairs, const ndt2d_window *win, int k, long long *nhyp, int64_t *max_tgt, int64_t *max_src)
+{
+    int rc = submaps_validate(m, "relocalize_submaps", offsets, nscans, submap_offsets, nsubmaps, member_scans, poses, host_poses, pairs,
+                              npairs, max_tgt, max_src);
+    if (rc) return rc;
+    if (level < 0 || level >= m->nlevels)
+        return fail(m, NDT2D_EINVAL, "relocalize_submaps: level %d out of range [0, %d)", level, m->nlevels);
+    return search_validate(m, "relocalize_submaps", "npairs", npairs, win, k, nhyp);
+}
+
+int ndt2d_relocalize_submaps_device(ndt2d_matcher *m, int level, const float *d_xy, const int64_t *d_offsets, const int64_t *offsets,
+                                    int nscans, const int64_t *submap_offsets, int nsubmaps, const int32_t *member_scans,
+                                    const double *d_member_poses, const int32_t *pairs, int npairs, const double *d_centres,
+                                    const ndt2d_window *win, int k, int64_t *d_best_idx, double *d_best_score, ndt2d_result *d_res)
+{
+    if (!m) return NDT2D_EINVAL;
+    long long nhyp = 0;
+    int64_t max_tgt = 0, max_src = 0;
+    int rc = relocalize_submaps_validate(m, level, offsets, nscans, submap_offsets, nsubmaps, member_scans, nullptr, false, pairs, npairs,
+                                         win, k, &nhyp, &max_tgt, &max_src);
+    if (rc) return rc;
+    if (npairs == 0) return NDT2D_OK;
+    if (!d_offsets || !d_centres || !d_best_idx || !d_res || (!m->h_sm_base.empty() && !d_member_poses))
+        return fail(m, NDT2D_EINVAL, "relocalize_submaps: bad arguments");
+    DeviceGuard g(m->device);
+    SubmapDev sub;
+    if ((rc = submaps_setup(m, submap_offsets, nsubmaps, d_member_poses, &sub))) return rc;
+    return relocalize_pairs_impl(m, "relocalize_submaps", level, d_xy, d_offsets, nsubmaps, pairs, npairs, max_tgt, max_src, d_centres,
+                                 *win, nhyp, k, d_best_idx, d_best_score, d_res, &sub);
+}
+
+int ndt2d_relocalize_submaps(ndt2d_matcher *m, int level, const float *xy, const int64_t *offsets, int nscans, const int64_t *submap_offsets,
+                             int nsubmaps, const int32_t *member_scans, const double *member_poses, const int32_t *pairs, int npairs,
+                             const double *centres, const ndt2d_window *win, int k, int64_t *best_idx, double *best_score,
+                             ndt2d_result *res)
+{
+    if (!m) return NDT2D_EINVAL;
+    long long nhyp = 0;
+    int64_t max_tgt = 0, max_src = 0;
+    int rc = relocalize_submaps_validate(m, level, offsets, nscans, submap_offsets, nsubmaps, member_scans, member_poses, true, pairs,
+                                         npairs, win, k, &nhyp, &max_tgt, &max_src);
+    if (rc) return rc;
+    if (npairs == 0) return NDT2D_OK;
+    if (!centres || !best_idx || !res) return fail(m, NDT2D_EINVAL, "relocalize_submaps: bad arguments");
+    DeviceGuard g(m->device);
+    const size_t njobs = (size_t)npairs * k;
+    if ((rc = upload_scans(m, "relocalize_submaps", xy, offsets, nscans, centres, npairs))) return rc;
+    if ((rc = upload(m, m->b_sm_pose, member_poses, m->h_sm_base.size() * 24))) return rc;
+    CK(m, m->b_tki.ensure(njobs * 8));
+    CK(m, m->b_tkv.ensure(njobs * 8));
+    CK(m, m->b_res.ensure(njobs * sizeof(ndt2d_result)));
+    SubmapDev sub;
+    if ((rc = submaps_setup(m, submap_offsets, nsubmaps, m->b_sm_pose.as<double>(), &sub))) return rc;
+    rc = relocalize_pairs_impl(m, "relocalize_submaps", level, m->b_xy.as<float>(), m->b_off.as<int64_t>(), nsubmaps, pairs, npairs,
+                               max_tgt, max_src, m->b_init.as<double>(), *win, nhyp, k, m->b_tki.as<int64_t>(), m->b_tkv.as<double>(),
+                               m->b_res.as<ndt2d_result>(), &sub);
+    if (rc) return rc;
+    return finish_host_call(m, "relocalize_submaps", njobs, best_idx, best_score, res, m->b_perr.as<int>(), "submap");
 }
 
 // ---- windowed search of a batch of scans against the handle's target (SPEC 6.2): ndt2d_relocalize(scan, window) per scan ----

@@ -75,6 +75,36 @@ def window_hypotheses(centre, window):
     return np.stack([c[0] + ix * w.step_x, c[1] + iy * w.step_y, c[2] + it * w.step_th], -1).reshape(-1, 3).astype(np.float32)
 
 
+def pack_submaps(submaps):
+    """Submaps for align_submaps / relocalize_submaps (SPEC.md section 7.3) from a list of (scan_indices, poses[n, 3]):
+    returns (submap_offsets int64 [nsubmaps + 1], member_scans int32 [nmembers], member_poses float64 [nmembers, 3])."""
+    offsets, scans, poses = [0], [], []
+    for idx, pp in submaps:
+        idx = np.asarray(idx, np.int64).reshape(-1)
+        pp = np.asarray(pp, np.float64).reshape(-1, 3)
+        if len(idx) != len(pp):
+            raise ValueError("every member scan needs one pose")
+        scans.append(idx)
+        poses.append(pp)
+        offsets.append(offsets[-1] + len(idx))
+    member_scans = np.concatenate(scans).astype(np.int32) if scans else np.zeros(0, np.int32)
+    member_poses = np.ascontiguousarray(np.concatenate(poses) if poses else np.zeros((0, 3)), np.float64)
+    return np.array(offsets, np.int64), member_scans, member_poses
+
+
+def _submap_args(submap_offsets, member_scans, member_poses=None):
+    so = np.ascontiguousarray(submap_offsets, np.int64).reshape(-1)
+    ms = np.ascontiguousarray(member_scans, np.int32).reshape(-1)
+    if len(so) < 1 or so[-1] != len(ms):
+        raise ValueError("submap_offsets must have nsubmaps + 1 entries and end at the number of member scans")
+    if member_poses is None:
+        return so, ms
+    mp = np.ascontiguousarray(member_poses, np.float64).reshape(-1, 3)
+    if len(mp) != len(ms):
+        raise ValueError("member_scans / member_poses sizes disagree")
+    return so, ms, mp
+
+
 class NdtMatcher2D:
     """One handle = one CUDA device + one stream (not thread-safe)."""
 
@@ -403,6 +433,67 @@ class NdtMatcher2D:
         self._ck(self._L.ndt2d_relocalize_pairs_device(self._h, level, _ptr(d_xy), _ptr(d_offsets), _ptr(offsets), len(offsets) - 1,
                                                        _ptr(pairs), len(pairs), _ptr(d_centres), C.byref(w), int(k), _ptr(d_best_idx),
                                                        _ptr(d_best_score), _ptr(d_res)))
+
+    def align_submaps(self, xy, offsets, submap_offsets, member_scans, member_poses, pairs, init):
+        """Batched align against submaps of posed scans (SPEC.md section 7.3; pack_submaps builds the three submap arrays):
+        pairs[p] = (submap, source scan); equals set_target_scans(the submap's member scans, their poses) + align(source,
+        init[p]) for every pair, in one call. The handle's own target is not touched."""
+        xy = np.ascontiguousarray(xy, np.float32).reshape(-1, 2)
+        offsets = np.ascontiguousarray(offsets, np.int64)
+        so, ms, mp = _submap_args(submap_offsets, member_scans, member_poses)
+        pairs = np.ascontiguousarray(pairs, np.int32).reshape(-1, 2)
+        init = np.ascontiguousarray(init, np.float64).reshape(-1, 3)
+        nb = len(offsets) - 1
+        if nb < 0 or len(init) != len(pairs) or (nb and (offsets[0] < 0 or offsets[-1] > len(xy))):
+            raise ValueError("offsets / pairs / init / xy sizes disagree")
+        res = np.zeros(len(pairs), RESULT_DTYPE)
+        self._ck(self._L.ndt2d_align_submaps(self._h, _ptr(xy), _ptr(offsets), nb, _ptr(so), len(so) - 1, _ptr(ms), _ptr(mp),
+                                             _ptr(pairs), len(pairs), _ptr(init), _ptr(res)))
+        return res
+
+    def align_submaps_device(self, d_xy, d_offsets, offsets, submap_offsets, member_scans, d_member_poses, pairs, d_init, d_res):
+        """Device-resident scans / member poses / initial poses / results; offsets (host copy), submap offsets, member scans
+        and pairs on the host. Asynchronous."""
+        offsets = np.ascontiguousarray(offsets, np.int64)
+        so, ms = _submap_args(submap_offsets, member_scans)
+        pairs = np.ascontiguousarray(pairs, np.int32).reshape(-1, 2)
+        self._ck(self._L.ndt2d_align_submaps_device(self._h, _ptr(d_xy), _ptr(d_offsets), _ptr(offsets), len(offsets) - 1, _ptr(so),
+                                                    len(so) - 1, _ptr(ms), _ptr(d_member_poses), _ptr(pairs), len(pairs), _ptr(d_init),
+                                                    _ptr(d_res)))
+
+    def relocalize_submaps(self, xy, offsets, submap_offsets, member_scans, member_poses, pairs, centres, window, k=4, level=0):
+        """Windowed search against submaps of posed scans (SPEC.md section 7.3): for pairs[p] = (submap, source scan), equals
+        set_target_scans(the submap's members) + relocalize(source, window_hypotheses(centres[p], window), k, level).
+        Returns (best_idx[npairs, k], best_score[npairs, k], res[npairs, k]); an empty slot has index -1."""
+        xy = np.ascontiguousarray(xy, np.float32).reshape(-1, 2)
+        offsets = np.ascontiguousarray(offsets, np.int64)
+        so, ms, mp = _submap_args(submap_offsets, member_scans, member_poses)
+        pairs = np.ascontiguousarray(pairs, np.int32).reshape(-1, 2)
+        centres = np.ascontiguousarray(centres, np.float64).reshape(-1, 3)
+        nb = len(offsets) - 1
+        if nb < 0 or len(centres) != len(pairs) or (nb and (offsets[0] < 0 or offsets[-1] > len(xy))):
+            raise ValueError("offsets / pairs / centres / xy sizes disagree")
+        kk = max(int(k), 0)
+        bi = np.full((len(pairs), kk), -1, np.int64)
+        bs = np.zeros((len(pairs), kk), np.float64)
+        res = np.zeros((len(pairs), kk), RESULT_DTYPE)
+        w = _window(window)
+        self._ck(self._L.ndt2d_relocalize_submaps(self._h, level, _ptr(xy), _ptr(offsets), nb, _ptr(so), len(so) - 1, _ptr(ms), _ptr(mp),
+                                                  _ptr(pairs), len(pairs), _ptr(centres), C.byref(w), int(k), _ptr(bi), _ptr(bs), _ptr(res)))
+        return bi, bs, res
+
+    def relocalize_submaps_device(self, d_xy, d_offsets, offsets, submap_offsets, member_scans, d_member_poses, pairs, d_centres,
+                                  window, k, d_best_idx, d_best_score, d_res, level=0):
+        """Device-resident scans / member poses / centres / outputs ([npairs * k] each; d_best_score may be None); offsets
+        (host copy), submap offsets, member scans, pairs and the window on the host. Asynchronous on the handle's stream."""
+        offsets = np.ascontiguousarray(offsets, np.int64)
+        so, ms = _submap_args(submap_offsets, member_scans)
+        pairs = np.ascontiguousarray(pairs, np.int32).reshape(-1, 2)
+        w = _window(window)
+        self._ck(self._L.ndt2d_relocalize_submaps_device(self._h, level, _ptr(d_xy), _ptr(d_offsets), _ptr(offsets), len(offsets) - 1,
+                                                         _ptr(so), len(so) - 1, _ptr(ms), _ptr(d_member_poses), _ptr(pairs), len(pairs),
+                                                         _ptr(d_centres), C.byref(w), int(k), _ptr(d_best_idx), _ptr(d_best_score),
+                                                         _ptr(d_res)))
 
     def relocalize_batch(self, xy, offsets, centres, window, k=4, level=0):
         """Windowed relocalisation of a batch of scans in the handle's map (SPEC.md section 6.2): for scan b, sweep the window

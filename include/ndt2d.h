@@ -229,6 +229,38 @@ int ndt2d_relocalize_pairs_device(ndt2d_matcher *m, int level, const float *d_xy
                                   const double *d_centres, const ndt2d_window *win, int k, int64_t *d_best_idx,
                                   double *d_best_score, ndt2d_result *d_res);
 
+/* ---- pairs against submaps of posed scans (local submaps of keyframes for loop closure, SPEC 7.3) ----
+ * Scans packed as for ndt2d_align_pairs. Submap g is members e in [submap_offsets[g], submap_offsets[g+1])
+ * (submap_offsets[0] = 0, non-decreasing); member e is scan member_scans[e] at f64 pose member_poses[3e..3e+2]. Its target
+ * is that of ndt2d_set_target_scans of the member scans at those poses (SPEC 7.2); a scan may be a member of several
+ * submaps, at different poses, and a submap without members has an empty target. Pair p = (submap pairs[2p], source scan
+ * pairs[2p+1]):
+ *   ndt2d_align_submaps: res[p] equals ndt2d_set_target_scans(members) + ndt2d_align(source, init[3p..]) bit for bit;
+ *   ndt2d_relocalize_submaps: best_idx / best_score / res[p*k..] equal ndt2d_set_target_scans(members) +
+ *   ndt2d_relocalize(level, source, the window's hypotheses around centres[3p..], k), as for ndt2d_relocalize_pairs.
+ * With the members expressed relative to an anchor keyframe, the result is the source's pose in the anchor's frame.
+ * Submaps a pair names are limited to 43 690 points in all (10 922 with overlapping grids). Refused with NDT2D_EINVAL:
+ * bad submap offsets, a member, source or submap index out of range, a non-finite member pose (host forms), an oversized
+ * submap. A submap whose auto-fitted lattice exceeds 2^31 cells is reported after the call; its pairs end NO_OVERLAP.
+ * The handle's own target is not touched. Device forms: scans, member poses, initial poses / centres and outputs on the
+ * device; offsets (also given on the host), submap offsets, member scans, pairs and the window on the host, since the
+ * target list and the chunking are host work. Asynchronous on the handle's stream. */
+int ndt2d_align_submaps(ndt2d_matcher *m, const float *xy, const int64_t *offsets, int nscans, const int64_t *submap_offsets,
+                        int nsubmaps, const int32_t *member_scans, const double *member_poses, const int32_t *pairs, int npairs,
+                        const double *init, ndt2d_result *res);
+int ndt2d_align_submaps_device(ndt2d_matcher *m, const float *d_xy, const int64_t *d_offsets, const int64_t *offsets, int nscans,
+                               const int64_t *submap_offsets, int nsubmaps, const int32_t *member_scans, const double *d_member_poses,
+                               const int32_t *pairs, int npairs, const double *d_init, ndt2d_result *d_res);
+int ndt2d_relocalize_submaps(ndt2d_matcher *m, int level, const float *xy, const int64_t *offsets, int nscans,
+                             const int64_t *submap_offsets, int nsubmaps, const int32_t *member_scans, const double *member_poses,
+                             const int32_t *pairs, int npairs, const double *centres, const ndt2d_window *win, int k,
+                             int64_t *best_idx, double *best_score, ndt2d_result *res);
+int ndt2d_relocalize_submaps_device(ndt2d_matcher *m, int level, const float *d_xy, const int64_t *d_offsets,
+                                    const int64_t *offsets, int nscans, const int64_t *submap_offsets, int nsubmaps,
+                                    const int32_t *member_scans, const double *d_member_poses, const int32_t *pairs, int npairs,
+                                    const double *d_centres, const ndt2d_window *win, int k, int64_t *d_best_idx,
+                                    double *d_best_score, ndt2d_result *d_res);
+
 /* ---- windowed search of a batch of scans against the handle's target (relocalisation in a known map, SPEC 6.2) ----
  * Scans packed as for ndt2d_align_batch. Scan b with centre centres[3b..]: best_idx[b*k..], best_score[b*k..] and
  * res[b*k..] equal, bit for bit, ndt2d_relocalize(level, scan b, the window's hypotheses around the centre, k) on this

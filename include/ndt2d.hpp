@@ -30,6 +30,13 @@ struct Pose2d {
     double x = 0, y = 0, theta = 0;
 };
 
+// A submap of posed scans (SPEC 7.3): member i is scan scans[i] of a packed batch at poses[i], e.g. a keyframe and its graph
+// neighbours at their current estimates, relative to an anchor keyframe
+struct Submap {
+    std::vector<std::int32_t> scans;
+    std::vector<Pose2d> poses;
+};
+
 using Result = ndt2d_result;   // pose[3], score, grad[3], hessian[9] (row-major), iterations, status, count
 using Params = ndt2d_params;
 
@@ -198,6 +205,46 @@ class Matcher {
         return out;
     }
 
+    // pairs against submaps of posed scans (SPEC 7.3): pair p = (submap pairs[p].first, source scan pairs[p].second); submap g
+    // is the scans submaps[g].scans of the packed batch at submaps[g].poses. alignSubmaps equals setTargetScans(members) +
+    // align(source, init[p]) per pair; relocalizeSubmaps equals setTargetScans(members) + relocalize(source, window
+    // hypotheses around centres[p], k, level), returned as relocalizePairs returns them.
+    std::vector<Result> alignSubmaps(const std::vector<Point2f> &points, const std::vector<std::int64_t> &offsets,
+                                     const std::vector<Submap> &submaps, const std::vector<std::pair<std::int32_t, std::int32_t>> &pairs,
+                                     const std::vector<Pose2d> &init)
+    {
+        if (pairs.size() != init.size()) throw std::invalid_argument("alignSubmaps: one initial pose per pair");
+        checkPacked(points, offsets, "alignSubmaps");
+        PackedSubmaps s(submaps);
+        std::vector<Result> out(pairs.size());
+        ck(ndt2d_align_submaps(h_, reinterpret_cast<const float *>(points.data()), offsets.data(), static_cast<int>(offsets.size() - 1),
+                               s.offsets.data(), static_cast<int>(submaps.size()), s.scans.data(), s.poses.data(),
+                               reinterpret_cast<const std::int32_t *>(pairs.data()), static_cast<int>(pairs.size()),
+                               reinterpret_cast<const double *>(init.data()), out.data()));
+        return out;
+    }
+    std::vector<Result> relocalizeSubmaps(const std::vector<Point2f> &points, const std::vector<std::int64_t> &offsets,
+                                          const std::vector<Submap> &submaps, const std::vector<std::pair<std::int32_t, std::int32_t>> &pairs,
+                                          const std::vector<Pose2d> &centres, const ndt2d_window &window, int k, int level = 0,
+                                          std::vector<std::int64_t> *indices = nullptr, std::vector<double> *scores = nullptr)
+    {
+        if (pairs.size() != centres.size()) throw std::invalid_argument("relocalizeSubmaps: one centre per pair");
+        checkPacked(points, offsets, "relocalizeSubmaps");
+        if (k < 1) throw std::invalid_argument("relocalizeSubmaps: k >= 1");
+        PackedSubmaps s(submaps);
+        const size_t n = pairs.size() * static_cast<size_t>(k);
+        std::vector<Result> out(n);
+        std::vector<std::int64_t> idx(n, -1);
+        std::vector<double> val(n, 0.0);
+        ck(ndt2d_relocalize_submaps(h_, level, reinterpret_cast<const float *>(points.data()), offsets.data(),
+                                    static_cast<int>(offsets.size() - 1), s.offsets.data(), static_cast<int>(submaps.size()), s.scans.data(),
+                                    s.poses.data(), reinterpret_cast<const std::int32_t *>(pairs.data()), static_cast<int>(pairs.size()),
+                                    reinterpret_cast<const double *>(centres.data()), &window, k, idx.data(), val.data(), out.data()));
+        if (indices) *indices = std::move(idx);
+        if (scores) *scores = std::move(val);
+        return out;
+    }
+
     // windowed relocalisation of a batch of scans in this handle's map: for scan b, the window's hypotheses around centres[b]
     // are swept on `level` and the k best refined; equals relocalize(scan b, window hypotheses, k, level) per scan.
     // Returns nscans * k records, scan-major; indices / scores (optional) receive the k sweep indices and scores per scan
@@ -327,6 +374,27 @@ class Matcher {
         const int nb = static_cast<int>(poses.size());
         ck(add ? ndt2d_add_target_scans(h_, xy, offsets.data(), nb, p) : ndt2d_set_target_scans(h_, xy, offsets.data(), nb, p));
     }
+    static void checkPacked(const std::vector<Point2f> &points, const std::vector<std::int64_t> &offsets, const char *name)
+    {
+        if (offsets.empty()) throw std::invalid_argument(std::string(name) + ": offsets must have nscans + 1 entries");
+        if (offsets.front() < 0 || static_cast<size_t>(offsets.back()) > points.size())
+            throw std::invalid_argument(std::string(name) + ": offsets overrun points");
+    }
+    // the C ABI's three submap arrays
+    struct PackedSubmaps {
+        std::vector<std::int64_t> offsets{0};
+        std::vector<std::int32_t> scans;
+        std::vector<double> poses;
+        explicit PackedSubmaps(const std::vector<Submap> &submaps)
+        {
+            for (const Submap &s : submaps) {
+                if (s.scans.size() != s.poses.size()) throw std::invalid_argument("Submap: one pose per member scan");
+                scans.insert(scans.end(), s.scans.begin(), s.scans.end());
+                for (const Pose2d &p : s.poses) poses.insert(poses.end(), {p.x, p.y, p.theta});
+                offsets.push_back(static_cast<std::int64_t>(scans.size()));
+            }
+        }
+    };
     void targetRanges(const std::vector<float> &ranges, int nbeams, double angle_min, double angle_inc, float range_min,
                       float range_max, const std::vector<Pose2d> &poses, bool add)
     {
